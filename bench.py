@@ -19,6 +19,10 @@ joint source modes, centroidal momentum matrix / centre of mass alone / convecti
 with its error, BASELINE configs 1 and 2, and the end-to-end step with the packed mass matrix (`e2e_packed`) and with the dense matrix kept
 in one host buffer from step to step (`e2e_dense_kept`).
 
+`--dump-outputs DIR` writes what the last timed step returned -- mass_matrix.npy (entry-major [nv*nv][S]), qdd.npy (forward
+dynamics, [nv][S]) and tau.npy (inverse dynamics, [nv][S]), all fp64 -- for a fixed, seeded sample of S <= 2048 of the states.
+The states are generated on the device from fixed seeds, so two builds run with the same arguments see the same inputs.
+
 `--impl reference`: Mecano itself is Java and no JVM exists on these boxes (SURVEY.md 8c), so the reference arm
 times the reference-faithful C restatement (oracle/, "port") multithreaded on all host cores.
 """
@@ -37,6 +41,8 @@ sys.path.insert(0, ROOT)
 
 HUMANOID_SEED = 20251017
 STATE_SEED = 1234
+DUMP_SEED = 4321
+DUMP_STATES = 2048  # states in the --dump-outputs sample over all ranks: ~24 MB for H37, the dense mass matrix being most of it
 GRAVITY = (0.0, 0.0, -9.81)
 FP64_NOMINAL_TFLOPS = 37.2  # 148 SMs x 64 DFMA/clk x 2 flop x 1.965 GHz (SURVEY.md section 6); the measured DFMA-chain figure is ~93 % of it
 METRIC = "RNEA+ABA+CRBA states/sec (37-DoF humanoid, fp64)"
@@ -57,7 +63,14 @@ def parse_args():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-cpu", action="store_true")
     p.add_argument("--no-extras", action="store_true", help="skip the kernels timed outside the step (ncu launch lists of the step alone)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed, for a fixed sample of the states, "
+                                                         "as DIR/<name>.npy (fp64)")
+    args = p.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        p.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        p.error("--dump-outputs writes the outputs of the GPU step; the reference arm times other states")
+    return args
 
 
 def workload_name(neck, n):
@@ -339,6 +352,26 @@ def emit(line):
         os.write(_JSON_FD, data)
 
 
+def dump_outputs(path, outputs, n, world, rank):
+    """--dump-outputs: the same DUMP_STATES / world states (columns, drawn with DUMP_SEED) of every output on every rank,
+    concatenated rank after rank along the state axis; rank 0 writes path/<name>.npy.  The inputs are seeded, so two builds
+    run with the same arguments can be compared output for output."""
+    import torch
+    import torch.distributed as dist
+
+    k = max(1, min(n, DUMP_STATES // world))
+    idx = torch.from_numpy(np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False)))
+    for name, out in outputs.items():
+        part = out.index_select(1, idx.to(out.device))
+        if world > 1:
+            parts = [torch.empty_like(part) for _ in range(world)]
+            dist.all_gather(parts, part)
+            part = torch.cat(parts, dim=1)
+        if rank == 0:
+            os.makedirs(path, exist_ok=True)
+            np.save(os.path.join(path, name + ".npy"), part.cpu().numpy())
+
+
 def main():
     args = parse_args()
     claim_stdout()
@@ -425,6 +458,8 @@ def main():
     t_stop.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:  # before the extras below reuse the output buffers
+        dump_outputs(args.dump_outputs, {"mass_matrix": M, "qdd": qdd_out, "tau": tau}, n, world, rank)
 
     ms_total = t_start.elapsed_time(t_stop)
     ms_step = sharding.max_over_ranks(ms_total / args.steps, dev)
