@@ -95,6 +95,15 @@ extern "C" {
 #define MECANO_B200_ALGO_RNEA 0
 #define MECANO_B200_ALGO_ABA 1
 #define MECANO_B200_ALGO_CRBA 2
+#define MECANO_B200_ALGO_REGRESSOR 4 /* mecano_b200_kernel_info_get of mecano_b200_joint_torque_regressor (3: the Coriolis kernel) */
+
+/* Column order of a body's ten inertial parameters in the joint-torque regressor (mecano_b200_joint_torque_regressor): the
+ * column of the mass, the first of the three first moments m c (x, y, z) and the first of the six moments of inertia about the
+ * origin (xx, xy, xz, yy, yz, zz).  This order is this project's definition; the kernel, the bindings and the tests read it
+ * from here. */
+#define MECANO_B200_REGRESSOR_M 0
+#define MECANO_B200_REGRESSOR_MC 1
+#define MECANO_B200_REGRESSOR_I 4
 
 typedef struct mecano_b200_handle mecano_b200_handle;
 
@@ -281,6 +290,27 @@ int mecano_b200_coriolis(mecano_b200_handle *h, int64_t n_states, int64_t ld, co
                          double *coriolis_matrix, void *stream);
 
 /*
+ * Joint-torque regressor (Mecano's JointTorqueRegressorCalculator): the matrix Y(q, qd, qdd) with tau = Y pi for ANY inertial
+ * parameters pi of the bodies -- what system identification stacks over a log of states to fit masses, centres of mass and
+ * inertias.  For a tree of n_bodies bodies (the root body, which is fixed, has no columns) and n_dofs DoFs:
+ *   Y            [n_dofs * 10 n_bodies][ld]  entry (i, c) of state s at [(i * 10 n_bodies + c) * ld + s], every entry written
+ *                                            (including the structural zeros: rows of joints off the path from the root to the
+ *                                            column's body).  Row i = Mecano DoF row.  Column block w (ten columns) belongs to
+ *                                            the body whose external-wrench rows are [6 w, 6 w + 6), w = wrench_index[b], the
+ *                                            convention of fext / body_acc / joint_wrench.
+ * The parameters of body w, in the column order of the MECANO_B200_REGRESSOR_* table: m, m cx, m cy, m cz, Ixx, Ixy, Ixz, Iyy,
+ * Iyz, Izz, with c the centre of mass and I the moment of inertia about the origin, both expressed in the body's bodyFixedFrame
+ * (the CoM frame of the tree description: com_rot, com_pos), the frame in which Mecano holds a body's SpatialInertia.  The
+ * model's own parameters are therefore pi_w = [m, 0, 0, 0, J_xx, J_xy, J_xz, J_yy, J_yz, J_zz].  tau = Y pi is inverse dynamics
+ * with the handle's gravity and without external wrenches.
+ * Always runs the generic thread-per-state kernel, in fp64 (a handle set to fp32 refuses with MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY);
+ * the wrench_index ranks must be below n_bodies (MECANO_B200_ERR_SHAPE otherwise).  Y is large: 10 n_bodies n_dofs doubles per
+ * state (94,720 bytes for a 32-body, 37-DoF humanoid).
+ */
+int mecano_b200_joint_torque_regressor(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd, const double *qdd,
+                                       double *Y, void *stream);
+
+/*
  * Host-pointer entry points (what a JNI / Panama binding calls with DMatrixRMaj.data): inputs are
  * staged host -> device in chunks, the kernels run, results are copied back; the call returns when
  * the outputs are complete.  Pinned (page-locked) host memory makes the copies asynchronous and
@@ -339,6 +369,8 @@ int mecano_b200_multi_step_host(mecano_b200_multi *m, int64_t n_states, int64_t 
                                 const double *tau_in, const double *fext, double *tau_out, double *qdd_out, double *mass_matrix, uint32_t layout);
 int mecano_b200_coriolis_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd, double *mass_matrix,
                               double *coriolis_matrix);
+int mecano_b200_joint_torque_regressor_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd,
+                                            const double *qdd, double *Y);
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, double *mass_matrix, double *cmm,
                                      double *com, int frame);
 int mecano_b200_centroidal_convective_term_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd,

@@ -3,6 +3,7 @@
     InverseDynamicsCalculator                 M/algorithms/InverseDynamicsCalculator.java:201-251, 291-306, 343-403, 469-472, 496-501, 567-570
     ForwardDynamicsCalculator                 M/algorithms/ForwardDynamicsCalculator.java:128-196, 313-319, 508-520, 556-567
     CompositeRigidBodyMassMatrixCalculator    M/algorithms/CompositeRigidBodyMassMatrixCalculator.java:182-233, 286-291, 344-348
+    JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, see the class)
 
 Same names, argument meaning and error behaviour as the reference; the batching changes are that the joint state
 is passed explicitly as [rows, N] matrices (Mecano reads it from the joint objects) and that results come back as
@@ -553,6 +554,70 @@ class CompositeRigidBodyMassMatrixCalculator(_BatchedCalculator):
             return torch.empty((rows, ld), dtype=torch.float64).pin_memory().numpy()[:, :n]
         except Exception:
             return np.empty((rows, ld), dtype=np.float64)[:, :n]
+
+
+class JointTorqueRegressorCalculator(_BatchedCalculator):
+    """Mecano's JointTorqueRegressorCalculator for N states: the inertial-parameter regressor Y(q, qd, qdd) of inverse dynamics,
+    tau = Y pi for any inertial parameters pi of the bodies (with gravity, without external wrenches).  What system
+    identification stacks over a log of states to fit masses, centres of mass and inertias.
+
+    Y is [nDoFs * 10 nBodies, N], entry (i, c) of state s at [i * 10 nBodies + c, s]: row i = DoF row, column block w (ten
+    columns) = the successor of joint w (JointMatrixIndexProvider order), parameters m, m cx, m cy, m cz, Ixx, Ixy, Ixz, Iyy,
+    Iyz, Izz in the order of the _capi.REGRESSOR_* table, c and I (about the origin) in the body's CoM frame.  On systems with
+    fixed or ignored joints every body of the tree has its own block (the expanded tables, see _BatchedCalculator._expanded):
+    nBodies counts them all, and the rows are the system's own nDoFs.  One device only."""
+    _ALGO = _capi.ALGO_REGRESSOR
+
+    def __init__(self, input, device=0):
+        super().__init__(input, device)
+        self._Y = None
+
+    def _tables(self):
+        """(engine, expanded system or None) that serve this calculator."""
+        if isinstance(self._device, (list, tuple)):
+            raise NotImplementedError("the joint-torque regressor runs on one device")
+        if self._input.hasWeldedBodies():
+            return self._expanded()
+        return self._engine, None
+
+    def compute(self, q, qd, qdd):
+        """compute(q, qd, qdd) for N states; returns getJointTorqueRegressorMatrix() ([nDoFs * 10 nBodies, N])."""
+        nv, nq = self._input.getNumberOfDoFs(), self._input.getConfigurationMatrixSize()
+        n = q.shape[1] if q.ndim == 2 else -1
+        self._check("q", q, nq, n)
+        self._check("qd", qd, nv, n)
+        self._check("qdd", qdd, nv, n)
+        eng, x = self._tables()
+        cols = 10 * eng.nb
+        if x is None:
+            Y = self._empty_like(q, nv * cols, n)
+            eng.joint_torque_regressor(q, qd, qdd, Y)
+        else:
+            # the held joints' configuration / DoF rows follow the system's own: the leading nv rows of Y are the caller's
+            q2 = self._extended(q, x.n_extra_cfg, x.q_extra)
+            qd2, qdd2 = self._extended(qd, x.n_extra_dof), self._extended(qdd, x.n_extra_dof)
+            Y2 = self._empty_like(q2, (nv + x.n_extra_dof) * cols, n, match_ld=False)
+            eng.joint_torque_regressor(q2, qd2, qdd2, Y2)
+            Y = Y2[:nv * cols]
+        self._Y = Y
+        return Y
+
+    def getJointTorqueRegressorMatrix(self):
+        return self._Y
+
+    def getInertialParameterVector(self):
+        """[10 nBodies]: the model's own parameters in the column order of Y, pi_w = [m, 0, 0, 0, J_xx, J_xy, J_xz, J_yy, J_yz, J_zz]
+        (CoM frame: first moment zero, J about the CoM).  Y @ pi = the joint efforts of InverseDynamicsCalculator.compute."""
+        eng, x = self._tables()
+        d = (self._input if x is None else x).tables().contents
+        nb = d.n_bodies
+        pi = np.zeros(10 * nb)
+        for b in range(nb):
+            w = d.wrench_index[b] if d.wrench_index else b
+            pi[10 * w + _capi.REGRESSOR_M] = d.mass[b]
+            for k, e in enumerate((0, 1, 2, 4, 5, 8)):
+                pi[10 * w + _capi.REGRESSOR_I + k] = d.inertia[9 * b + e]
+        return pi
 
 
 class MultiBodyDynamicsStep:

@@ -29,6 +29,7 @@ struct mecano_b200_handle
    mb::FlatTree tree;
    double *d_consts = nullptr;
    uint16_t *d_zero = nullptr; // CRBA: structurally zero entries
+   uint32_t *d_yzero = nullptr; // joint-torque regressor: structurally zero rows (FlatTree::regressor_zero_rows)
    MbProgram *d_prog = nullptr; // [3] device copies of the traversal programs (warp-per-state kernels)
    std::vector<std::pair<int, int>> nonzero_runs; // CRBA: (first entry, count) runs of mass-matrix entries that are not structurally zero
    unsigned *d_counters = nullptr; // work counters of the persistent launches (kernels.cu: launch_thread_kernel): a ring of MB_COUNTERS,
@@ -43,14 +44,14 @@ struct mecano_b200_handle
    double gravity[3] = {0.0, 0.0, 0.0}; // Mecano calculators start with zero gravity until setGravitationalAcceleration
    mb::LaunchPlan plan[MB_NUM_ALGOS];
    bool fp32 = false; // mecano_b200_set_precision
-   int grid_limit[MB_NUM_ALGOS] = {0, 0, 0, 0}; // mecano_b200_set_grid_limit: cap on the persistent grids (0 = whole device)
+   int grid_limit[MB_NUM_ALGOS] = {0, 0, 0, 0, 0}; // mecano_b200_set_grid_limit: cap on the persistent grids (0 = whole device)
    int variant = MECANO_B200_VARIANT_AUTO;
    int max_children = 1, max_ndof = 1, sm_count = 148;
    int n_accel_source = 0;           // joints in ACCELERATION_SOURCE mode (mecano_b200_set_joint_source_modes)
    std::vector<std::pair<int, int>> effort_dof_runs; // (first DoF row, count) runs of DoF rows whose joints are EFFORT_SOURCE
    bool warp_ok = false;             // the body-parallel variant serves this tree (one-DoF / SixDoF joints; <= 32 bodies: a warp per state, else a team of warps)
    bool has_3dof = false;            // the tree has spherical / planar joints (generic thread-per-state kernels only)
-   int64_t warp_below[MB_NUM_ALGOS] = {0, 0, 0, 0}; // AUTO: batches smaller than this run warp-per-state
+   int64_t warp_below[MB_NUM_ALGOS] = {0, 0, 0, 0, 0}; // AUTO: batches smaller than this run warp-per-state
    std::string error;
    // host pipeline (lazy)
    cudaStream_t streams[MB_MAX_SLOTS] = {};
@@ -160,7 +161,7 @@ int run(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q,
    // states on; a thread per state needs tens of thousands but then has 10-30x the throughput)
    // calls with by-product buffers (mecano_b200_rnea_full) always run the generic thread-per-state kernel
    // (so does the packed mass-matrix layout: its row numbering follows the thread-per-state traversal)
-   const bool byprod = body_acc || joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || algo == MB_CORIOLIS || h->fp32 || packed;
+   const bool byprod = body_acc || joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || algo == MB_CORIOLIS || algo == MB_REGRESSOR || h->fp32 || packed;
    const int64_t vn = opt.variant_n > 0 ? opt.variant_n : n;
    const bool use_warp = !byprod && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && vn < h->warp_below[algo]));
    if (use_warp)
@@ -223,6 +224,11 @@ int run(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q,
    a.ws_ld = 0;
    a.zero_entries = h->d_zero;
    a.n_zero = (algo == MB_CRBA && (flags & (MECANO_B200_CRBA_ZEROS_PRESENT | MECANO_B200_CRBA_PACKED))) ? 0 : (int32_t)h->tree.zero_entries.size();
+   if (algo == MB_REGRESSOR)
+   {
+      a.zero_entries = reinterpret_cast<const uint16_t *>(h->d_yzero); // (kernel_args.h: the regressor's uint32 zero rows)
+      a.n_zero = (int32_t)h->tree.regressor_zero_rows.size();
+   }
    a.n = n; a.ld = ld;
    a.ld_qd = a.ld_x = ld;
    if (algo == MB_RNEA && (flags & (MECANO_B200_RNEA_NO_CORIOLIS | MECANO_B200_RNEA_NO_ACCELERATIONS)))
@@ -653,6 +659,7 @@ int mecano_b200_create(const mecano_b200_tree_desc *desc, int device, mecano_b20
       if (h->d_consts) cudaFree(h->d_consts);
       if (h->d_counters) cudaFree(h->d_counters);
       if (h->d_zero) cudaFree(h->d_zero);
+      if (h->d_yzero) cudaFree(h->d_yzero);
       if (h->d_prog) cudaFree(h->d_prog);
       delete h;
       return fail(nullptr, (int)ce, m);
@@ -684,13 +691,19 @@ int mecano_b200_create(const mecano_b200_tree_desc *desc, int device, mecano_b20
       if ((e = cudaMalloc(&h->d_zero, zb)) != cudaSuccess) return bail(e, "cudaMalloc(zero entries)");
       if ((e = cudaMemcpy(h->d_zero, h->tree.zero_entries.data(), zb, cudaMemcpyHostToDevice)) != cudaSuccess) return bail(e, "cudaMemcpy(zero entries)");
    }
+   if (!h->tree.regressor_zero_rows.empty())
+   {
+      const size_t zb = h->tree.regressor_zero_rows.size() * sizeof(uint32_t);
+      if ((e = cudaMalloc(&h->d_yzero, zb)) != cudaSuccess) return bail(e, "cudaMalloc(regressor zero rows)");
+      if ((e = cudaMemcpy(h->d_yzero, h->tree.regressor_zero_rows.data(), zb, cudaMemcpyHostToDevice)) != cudaSuccess) return bail(e, "cudaMemcpy(regressor zero rows)");
+   }
    for (int algo = 0; algo < MB_NUM_ALGOS; algo++)
    {
       bool fits = false;
       if ((e = mb::plan_thread_kernel(algo, h->tree.prog[algo], false, h->plan[algo], &fits)) != cudaSuccess) return bail(e, "kernel planning");
-      if (!fits && algo == MB_CORIOLIS)
+      if (!fits && (algo == MB_CORIOLIS || algo == MB_REGRESSOR))
       {
-         h->plan[algo].block = 0; // the by-product kernel alone does not fit: mecano_b200_coriolis reports it, everything else works
+         h->plan[algo].block = 0; // a by-product kernel alone does not fit: its entry point reports it, everything else works
          continue;
       }
       if (!fits)
@@ -698,6 +711,7 @@ int mecano_b200_create(const mecano_b200_tree_desc *desc, int device, mecano_b20
          cudaFree(h->d_consts);
          if (h->d_counters) cudaFree(h->d_counters);
          if (h->d_zero) cudaFree(h->d_zero);
+         if (h->d_yzero) cudaFree(h->d_yzero);
          delete h;
          return fail(nullptr, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the compiled per-state work areas (branch nesting / depth too large)");
       }
@@ -752,6 +766,7 @@ void mecano_b200_destroy(mecano_b200_handle *h)
    if (h->d_consts) cudaFree(h->d_consts);
    if (h->d_counters) cudaFree(h->d_counters);
    if (h->d_zero) cudaFree(h->d_zero);
+   if (h->d_yzero) cudaFree(h->d_yzero);
    if (h->d_prog) cudaFree(h->d_prog);
    for (int i = 0; i < 1 + MB_MAX_SLOTS; i++)
       if (h->d_ws[i]) cudaFree(h->d_ws[i]);
@@ -1057,6 +1072,65 @@ int mecano_b200_coriolis_host(mecano_b200_handle *h, int64_t n, int64_t ld, cons
    return rc;
 }
 
+// the regressor's refusals shared by its two entry points (after check_batch)
+int regressor_check(mecano_b200_handle *h)
+{
+   if (h->fp32)
+      return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the joint-torque regressor is computed in fp64 only (mecano_b200_set_precision)");
+   const MbProgram &P = h->tree.prog[MB_REGRESSOR];
+   for (int i = 0; i < P.nb; i++)
+      if (P.body[i].ext_index >= P.nb)
+         return fail(h, MECANO_B200_ERR_SHAPE, "joint-torque regressor: wrench_index ranks must be below n_bodies (one ten-column block per body)");
+   if (h->plan[MB_REGRESSOR].block == 0)
+      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the joint-torque regressor kernel (branch nesting / depth too large)");
+   return MECANO_B200_OK;
+}
+
+int mecano_b200_joint_torque_regressor(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, double *Y,
+                                       void *stream)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc) return rc;
+   if ((rc = regressor_check(h))) return rc;
+   if (n == 0) return MECANO_B200_OK;
+   if (!q || !qd || !qdd || !Y) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   MB_ON_DEVICE(h);
+   return run(h, MB_REGRESSOR, n, ld, q, qd, qdd, nullptr, Y, 0u, (cudaStream_t)stream);
+}
+
+int mecano_b200_joint_torque_regressor_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, double *Y)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc) return rc;
+   if ((rc = regressor_check(h))) return rc;
+   if (n == 0) return MECANO_B200_OK;
+   if (!q || !qd || !qdd || !Y) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   std::lock_guard<std::mutex> lk(h->mu);
+   MB_ON_DEVICE(h);
+   const size_t nq = h->tree.nq, nv = h->tree.nv, ny = nv * 10 * (size_t)h->tree.nb, rows = nq + 2 * nv + ny;
+   // chunks of at most 1 GiB of staging (94.7 KB of Y per state for a 32-body humanoid: 11 k states)
+   const size_t chunk = (size_t)std::min<int64_t>(n, (int64_t)std::max<size_t>(32, std::min<size_t>(16384, ((size_t)1 << 30) / (rows * sizeof(double)))));
+   double *d = nullptr;
+   MB_CUDA(h, cudaMalloc(&d, rows * chunk * sizeof(double)));
+   double *dq = d, *dqd = dq + nq * chunk, *dqdd = dqd + nv * chunk, *dY = dqdd + nv * chunk;
+   cudaError_t e = cudaSuccess;
+   for (int64_t s0 = 0; s0 < n && rc == 0 && e == cudaSuccess; s0 += (int64_t)chunk)
+   {
+      const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, n - s0);
+      e = copy_rows(dq, chunk, q + s0, (size_t)ld, w, nq, cudaMemcpyHostToDevice, nullptr);
+      if (e == cudaSuccess) e = copy_rows(dqd, chunk, qd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, nullptr);
+      if (e == cudaSuccess) e = copy_rows(dqdd, chunk, qdd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, nullptr);
+      if (e != cudaSuccess) break;
+      rc = mecano_b200_joint_torque_regressor(h, (int64_t)w, (int64_t)chunk, dq, dqd, dqdd, dY, nullptr);
+      if (rc) break;
+      e = copy_rows(Y + s0, (size_t)ld, dY, chunk, w, ny, cudaMemcpyDeviceToHost, nullptr);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(nullptr);
+   }
+   cudaFree(d);
+   if (e != cudaSuccess) return cuda_fail(h, e, "mecano_b200_joint_torque_regressor_host");
+   return rc;
+}
+
 // host-pointer variants of the two centroidal calls: plain staging through temporary device buffers, chunk by chunk
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame)
 {
@@ -1265,7 +1339,7 @@ int mecano_b200_step_host(mecano_b200_handle *h, int64_t n, int64_t ld, const do
 int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_states, mecano_b200_kernel_info *info)
 {
    if (!h || !info || algo < 0 || algo >= MB_NUM_ALGOS) return MECANO_B200_ERR_INVALID_ARGUMENT;
-   const bool warp = algo != MB_CORIOLIS && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && n_states > 0 && n_states < h->warp_below[algo]));
+   const bool warp = algo != MB_CORIOLIS && algo != MB_REGRESSOR && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && n_states > 0 && n_states < h->warp_below[algo]));
    if (warp)
    {
       std::memset(info, 0, sizeof *info);
@@ -1318,7 +1392,9 @@ int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_state
    info->stack_doubles = P.stack_doubles;
    info->max_depth = P.max_depth;
    const double nq = P.nq, nv = P.nv;
-   info->bytes_per_state = algo == MB_CRBA ? 8.0 * (nq + nv * nv) : (algo == MB_CORIOLIS ? 8.0 * (nq + nv + 2.0 * nv * nv) : 8.0 * (nq + 3.0 * nv)); // SURVEY.md 8(d)
+   info->bytes_per_state = algo == MB_CRBA ? 8.0 * (nq + nv * nv)
+                           : (algo == MB_CORIOLIS ? 8.0 * (nq + nv + 2.0 * nv * nv)
+                                                  : (algo == MB_REGRESSOR ? 8.0 * (nq + 2.0 * nv + 10.0 * P.nb * nv) : 8.0 * (nq + 3.0 * nv))); // SURVEY.md 8(d)
    return MECANO_B200_OK;
 }
 

@@ -89,7 +89,7 @@ int slot_size(int algo, int jtype)
       case MB_RNEA: return 6 + jp;       // accumulated wrench + joint parameters
       case MB_ABA: return 6 + jp + nd;   // twist + joint parameters + joint velocity
       case MB_CORIOLIS: return 6 + jp;   // twist + joint parameters
-      default: return jp;                // CRBA: joint parameters only
+      default: return jp;                // CRBA, regressor: joint parameters only
    }
 }
 
@@ -97,7 +97,8 @@ int aux_size(int algo)
 {
    switch (algo)
    {
-      case MB_RNEA: return 12; // twist + spatial acceleration of a branching body
+      case MB_RNEA:
+      case MB_REGRESSOR: return 12; // twist + spatial acceleration of a branching body
       case MB_ABA: return 27;  // articulated inertia (6 + 9 + 6) + bias wrench (6); reused for (v, a) in pass three
       case MB_CORIOLIS: return 46; // composite inertia (10) + composite factorized inertia (4 x 9)
       default: return 10;      // composite inertia (6 + 3 + 1)
@@ -116,7 +117,7 @@ int slot2_size(int algo, int jtype, bool root_parent)
          return jtype == MB_SIXDOF ? (root_parent ? 3 : 9) : 4;
       case MB_CORIOLIS: // twist (3) + sin/cos (1); SixDoF: twist (3) + transform (6)
          return jtype == MB_SIXDOF ? 9 : 4;
-      default: // CRBA: sin/cos (1); SixDoF: transform (6)
+      default: // CRBA, regressor: sin/cos (1); SixDoF: transform (6)
          return jtype == MB_SIXDOF ? 6 : 1;
    }
 }
@@ -664,6 +665,22 @@ int flatten_tree(const mecano_b200_tree_desc *d, FlatTree &out, std::string &err
                err = "internal error: packed mass-matrix column table";
                return MECANO_B200_ERR_INVALID_ARGUMENT;
             }
+         }
+   }
+   // ---- structural zeros of the joint-torque regressor: in the block of body i, the DoF rows of the joints that are not on the
+   //      path from the root to i (flatten.h); only for wrench_index ranks that fit the 10 nb columns (api.cu refuses the others)
+   {
+      const MbProgram &P = out.prog[MB_REGRESSOR];
+      bool cols_ok = true;
+      for (int i = 0; i < nb; i++)
+         cols_ok = cols_ok && P.body[i].ext_index < nb;
+      for (int i = 0; i < nb && cols_ok; i++)
+         for (int j = 0; j < nb; j++)
+         {
+            if (j <= i && i < subtree_end[j])
+               continue; // j is i or an ancestor of i
+            for (int r = 0; r < P.body[j].ndof; r++)
+               out.regressor_zero_rows.push_back((uint32_t)((P.body[j].dof_off + r) * 10 * nb + 10 * P.body[i].ext_index));
          }
    }
    return MECANO_B200_OK;

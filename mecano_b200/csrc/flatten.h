@@ -24,7 +24,10 @@ struct FlatTree
    // packed mass-matrix layout (MECANO_B200_CRBA_PACKED): packed row p holds M[packed_row[p]][packed_col[p]] (= the mirrored
    // entry); one row per unique entry that is not structurally zero, column by column, path from the root first
    std::vector<int32_t> packed_row, packed_col;
-   MbProgram prog[MB_NUM_ALGOS];    // MB_RNEA, MB_ABA, MB_CRBA, MB_CORIOLIS
+   // joint-torque regressor (MB_REGRESSOR): the structurally zero rows of each body's block, as the entry of the row's first
+   // column (row * 10 nb + 10 w); a row's ten columns are zero together.  Empty if a wrench_index rank is >= nb.
+   std::vector<uint32_t> regressor_zero_rows;
+   MbProgram prog[MB_NUM_ALGOS];    // MB_RNEA, MB_ABA, MB_CRBA, MB_CORIOLIS, MB_REGRESSOR
 };
 
 // Returns MECANO_B200_OK or a negative error code; `err` receives the message.

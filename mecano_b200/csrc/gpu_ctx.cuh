@@ -360,6 +360,27 @@ template <int BLOCK, int TM, int ROWS, bool M3 = false> struct GpuCtx2
    __device__ __forceinline__ void pf_commit() const { asm volatile("cp.async.commit_group;" ::: "memory"); }
    template <int N> __device__ __forceinline__ void pf_wait() const { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
    __device__ __forceinline__ double pf_ld(int stage, int j) const { return mb_lds1(rb + (unsigned)((stage * ROWS + ((j == 2 && ROWS < 3) ? 0 : j)) * (BLOCK * 8))); }
+   // joint-torque regressor (MB_REGRESSOR): entry e = row * 10 nb + col of Y at mbase + e * ld8, streamed past L2 like the mass matrix
+   const uint32_t *yzrows; // structurally zero rows: entry of the row's first column
+   int nyz;
+   __device__ __forceinline__ void st_Y(int e, double v) const
+   {
+      if (!kMayClamp || active)
+         mb_stg_cs(mb_row(mbase, (unsigned)e, ld8), v);
+   }
+   __device__ __forceinline__ int y_zero_parts(int nops) const { return (nyz + nops - 1) / nops; }
+   __device__ __forceinline__ void y_zero_fill_part(int k, int parts) const
+   {
+      const int k1 = min(nyz, (k + 1) * parts);
+#pragma unroll 1
+      for (int i = k * parts; i < k1; i++)
+      {
+         const int e = (int)__ldg(yzrows + i);
+#pragma unroll
+         for (int j = 0; j < 10; j++)
+            st_Y(e + j, 0.0);
+      }
+   }
 };
 
 // columns of tensor memory one warp owns when BLOCK / 32 warps share the four lane quarters

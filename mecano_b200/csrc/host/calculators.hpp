@@ -3,6 +3,7 @@
 //   InverseDynamicsCalculator                 M/algorithms/InverseDynamicsCalculator.java:201-251, 291-306, 343-403, 469-472, 496-501, 567-570
 //   ForwardDynamicsCalculator                 M/algorithms/ForwardDynamicsCalculator.java:128-196, 313-319, 508-520, 556-567
 //   CompositeRigidBodyMassMatrixCalculator    M/algorithms/CompositeRigidBodyMassMatrixCalculator.java:182-233, 286-291, 344-348
+//   JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, below)
 //
 // Same names, argument meaning and error behaviour (exceptions) as the reference, with two batching changes:
 //   * compute(...) takes the joint state explicitly as nRows x N row-major matrices (what a Java
@@ -303,5 +304,48 @@ class CompositeRigidBodyMassMatrixCalculator : public BatchedCalculatorBase
  private:
    CentroidalMomentumFrame frame_ = CentroidalMomentumFrame::World;
    bool coriolisEnabled_ = false;
+};
+
+// JointTorqueRegressorCalculator: the inertial-parameter regressor Y(q, qd, qdd) of inverse dynamics, tau = Y pi for any inertial
+// parameters pi (mecano_b200_joint_torque_regressor: layout, column order MECANO_B200_REGRESSOR_*, frames).  Systems whose fixed /
+// ignored joints are welded into other bodies are refused by the C ABI here (a welded body has no block of its own); the Python
+// calculator runs them on the expanded tables.
+class JointTorqueRegressorCalculator : public BatchedCalculatorBase
+{
+ public:
+   explicit JointTorqueRegressorCalculator(const MultiBodySystem &input, int device = 0) : BatchedCalculatorBase(input, device) {}
+   int64_t getNumberOfParameters() const { return 10 * (int64_t)tables_.parent.size(); }
+   // compute(q, qd, qdd) + getJointTorqueRegressorMatrix(), for N states: (nDoFs * 10 nBodies) x N, entry-major
+   void compute(const MatrixView &q, const MatrixView &qd, const MatrixView &qdd, const MatrixView &regressorOut, Memory where = Memory::Device)
+   {
+      const int64_t n = q.cols, nv = input_.getNumberOfDoFs(), nq = input_.getConfigurationMatrixSize();
+      checkShape(q, nq, n, "q");
+      checkShape(qd, nv, n, "qd");
+      checkShape(qdd, nv, n, "qdd");
+      checkShape(regressorOut, nv * getNumberOfParameters(), n, "jointTorqueRegressor");
+      if (qd.ld != q.ld || qdd.ld != q.ld || regressorOut.ld != q.ld)
+         throw MatrixDimensionException("all matrices of one call must share the same leading dimension");
+      if (where == Memory::Device)
+         check(mecano_b200_joint_torque_regressor(handle_, n, q.ld, q.data, qd.data, qdd.data, regressorOut.data, stream_));
+      else
+         check(mecano_b200_joint_torque_regressor_host(handle_, n, q.ld, q.data, qd.data, qdd.data, regressorOut.data));
+   }
+   // the model's own parameters in the column order of Y: [m, 0, 0, 0, J_xx, J_xy, J_xz, J_yy, J_yz, J_zz] per body (CoM frame)
+   std::vector<double> getInertialParameterVector() const
+   {
+      const size_t nb = tables_.parent.size();
+      std::vector<double> pi(10 * nb, 0.0);
+      const int sym[6] = {0, 1, 2, 4, 5, 8};
+      for (size_t b = 0; b < nb; b++)
+      {
+         const size_t w = tables_.wrench_index.empty() ? b : (size_t)tables_.wrench_index[b];
+         if (w >= nb)
+            throw std::runtime_error("getInertialParameterVector: the system has welded bodies (fixed / ignored joints)");
+         pi[10 * w + MECANO_B200_REGRESSOR_M] = tables_.mass[b];
+         for (int k = 0; k < 6; k++)
+            pi[10 * w + MECANO_B200_REGRESSOR_I + k] = tables_.inertia[9 * b + sym[k]];
+      }
+      return pi;
+   }
 };
 } // namespace mecano

@@ -77,6 +77,11 @@ namespace mb
 #else
 #define MB_INST_12 MB_SKIP
 #endif
+#if MB_INST == 14
+#define MB_INST_14 MB_EMIT
+#else
+#define MB_INST_14 MB_SKIP
+#endif
 MB_KERNEL_GROUPS(MB_X)
 
 #if MB_INST == 13

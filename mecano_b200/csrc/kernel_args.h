@@ -24,7 +24,9 @@ struct KernelArgs
    double *ws;                      // ABA: pass-two records [rec][ws_ld], one column per resident thread of the persistent grid
    long long ws_ld;
    const uint16_t *zero_entries;    // CRBA: structurally zero mass-matrix entries (multiple of 8, 16-byte aligned)
-   int32_t n_zero;
+   int32_t n_zero;                  // MB_REGRESSOR: `out` is the joint-torque regressor Y, [(row * 10 nb + col) * ld + s]; zero_entries
+                                    // then holds n_zero uint32 entries, the first column of each structurally zero row of Y
+                                    // (FlatTree::regressor_zero_rows; a row's ten columns are zero together)
    long long n, ld;
    long long ld_qd, ld_x; // row strides of qd and x (normally ld; 0 when the launcher substitutes one row of zeros)
    double grav[3];

@@ -39,6 +39,7 @@ KernelFn pick(int algo, bool fext, int layout, int cfg, bool m3)
       return m3 ? (fext ? pick_cfg<MB_ABA, true, 0, true>(cfg) : pick_cfg<MB_ABA, false, 0, true>(cfg))
                 : (fext ? pick_cfg<MB_ABA, true, 0, false>(cfg) : pick_cfg<MB_ABA, false, 0, false>(cfg));
    if (algo == MB_CORIOLIS) return pick_cfg<MB_CORIOLIS, false, 0, true>(cfg);
+   if (algo == MB_REGRESSOR) return pick_cfg<MB_REGRESSOR, false, 0, true>(cfg);
    // CRBA: the "FEXT" instantiation is the one with by-products (centroidal momentum matrix, centre of mass), entry-major only
    if (fext && layout == 0) return pick_cfg<MB_CRBA, true, 0, true>(cfg);
    return layout == 1 ? pick_cfg<MB_CRBA, false, 1, true>(cfg) : (layout == 2 ? pick_cfg<MB_CRBA, false, 2, true>(cfg) : pick_cfg<MB_CRBA, false, 0, true>(cfg));
@@ -46,8 +47,7 @@ KernelFn pick(int algo, bool fext, int layout, int cfg, bool m3)
 
 int class_of(int algo, const MbProgram &P)
 {
-   const int aux0 = algo == MB_RNEA ? kRnaAux0 : (algo == MB_ABA ? kAbaAux0 : (algo == MB_CRBA ? kCrbAux0 : kCorAux0));
-   const int aux1 = algo == MB_RNEA ? kRnaAux1 : (algo == MB_ABA ? kAbaAux1 : (algo == MB_CRBA ? kCrbAux1 : kCorAux1));
+   const int aux0 = aux_of(algo, 0), aux1 = aux_of(algo, 1);
    const int rec0 = algo == MB_ABA ? kAbaRec0 : 0, rec1 = algo == MB_ABA ? kAbaRec1 : 0;
    if (P.aux_doubles <= aux0 && P.rec_doubles <= rec0) return 0;
    if (P.aux_doubles <= aux1 && P.rec_doubles <= rec1) return 1;
@@ -70,7 +70,7 @@ int forced_cfg(int algo)
 {
    const char *e = getenv("MECANO_B200_CFG");
    if (!e) return -1;
-   const char *key = algo == MB_RNEA ? "rnea=" : (algo == MB_ABA ? "aba=" : (algo == MB_CRBA ? "crba=" : "cor="));
+   const char *key = algo == MB_RNEA ? "rnea=" : (algo == MB_ABA ? "aba=" : (algo == MB_CRBA ? "crba=" : (algo == MB_REGRESSOR ? "reg=" : "cor=")));
    const char *p = strstr(e, key);
    return p ? atoi(p + strlen(key)) : -1;
 }
@@ -132,9 +132,7 @@ cudaError_t plan_thread_kernel(int algo, const MbProgram &P, bool fext, LaunchPl
          nblk = 1; // cannot happen (smem_bytes), but a TMEM block must be alone on its SM
       // register spills cost more than the extra warps bring: a configuration whose kernel spills beyond its declared
       // work area only competes if nothing else fits
-      const int auxn = algo == MB_RNEA ? (kCfg[cfg].cls ? kRnaAux1 : kRnaAux0)
-                                       : (algo == MB_ABA ? (kCfg[cfg].cls ? kAbaAux1 : kAbaAux0)
-                                                         : (algo == MB_CRBA ? (kCfg[cfg].cls ? kCrbAux1 : kCrbAux0) : (kCfg[cfg].cls ? kCorAux1 : kCorAux0)));
+      const int auxn = aux_of(algo, kCfg[cfg].cls);
       // (the Coriolis kernel keeps two 46-double accumulators and three force columns live: a few hundred bytes of spills are its
       // normal state at 255 registers)
       const bool spills = (long)fa.localSizeBytes > 8l * auxn + (algo == MB_CORIOLIS ? 512 : 128);
@@ -145,8 +143,9 @@ cudaError_t plan_thread_kernel(int algo, const MbProgram &P, bool fext, LaunchPl
       // prefer more resident states; on ties the first configuration in the table wins -- except for the two store-bound
       // mass-matrix kernels, where more, smaller blocks win: hardware block scheduling evens out their store bursts (Coriolis,
       // H37: 2 x 128 threads 5.89 ms, 1 x 256 6.54 ms, profiles/r02h_cor_sweep.jsonl; CRBA, 4 x 128 against 2 x 256 threads:
-      // 7 / 15 / 25 / 32 / 51 bodies -2.9 / -8.4 / -0.8 / -1.4 / -4.3 %, profiles/r03g_crba_block_sweep.jsonl)
-      const bool small_blocks = algo == MB_CORIOLIS || algo == MB_CRBA;
+      // 7 / 15 / 25 / 32 / 51 bodies -2.9 / -8.4 / -0.8 / -1.4 / -4.3 %, profiles/r03g_crba_block_sweep.jsonl); the
+      // regressor, store-bound the same way, follows them
+      const bool small_blocks = algo == MB_CORIOLIS || algo == MB_CRBA || algo == MB_REGRESSOR;
       if (nblk > 0 && (score > best_threads || (small_blocks && score == best_threads && b < plan.block)))
       {
          best_threads = score;
@@ -214,7 +213,7 @@ cudaError_t launch_thread_kernel(int algo, const MbProgram &P, const KernelArgs 
    static const bool draw = [] { const char *e = getenv("MECANO_B200_DRAW"); return !e || atoi(e) != 0; }();
    // the warps of a persistent grid draw their states from a counter that the kernel itself re-arms (gpu_ctx.cuh: thread_block_run)
    // (RNEA / ABA only: the mass-matrix kernels are launched one block per tile, and their stores carry no guard for clamped lanes)
-   if (!(persistent && draw) || algo == MB_CRBA || algo == MB_CORIOLIS)
+   if (!(persistent && draw) || smem_stack_only(algo))
       b.work_counter = nullptr;
    fn<<<grid, plan.block, plan.smem, stream>>>(P, b);
    return cudaGetLastError();

@@ -5,6 +5,7 @@
 #include "f32_ctx.cuh"
 #include "gpu_ctx.cuh"
 #include "kernels.h"
+#include "regressor.cuh"
 
 namespace mb
 {
@@ -25,6 +26,12 @@ __device__ __forceinline__ void thread_kernel_body(const MbProgram &P, const Ker
          aba_state<double, Ctx, FEXT>(P, c2, a.grav);
       else if constexpr (ALGO == MB_CRBA)
          crba_state<double, Ctx, FEXT, LAYOUT == 2>(P, c2);
+      else if constexpr (ALGO == MB_REGRESSOR)
+      {
+         c2.yzrows = reinterpret_cast<const uint32_t *>(a.zero_entries);
+         c2.nyz = a.n_zero;
+         regressor_state<double, Ctx>(P, c2, a.grav);
+      }
       else
          coriolis_state<double, Ctx>(P, c2);
    });
@@ -63,6 +70,7 @@ constexpr int kRnaAux0 = 12 * 4, kRnaAux1 = 12 * 16;
 constexpr int kAbaAux0 = 27 * 4, kAbaAux1 = 27 * 16;
 constexpr int kCrbAux0 = 10 * 4, kCrbAux1 = 10 * 16;
 constexpr int kCorAux0 = 46 * 4, kCorAux1 = 46 * 16;
+constexpr int kRegAux0 = 12 * 4, kRegAux1 = 12 * 16;
 constexpr int kAbaRec0 = MB_ABA_REC * 33, kAbaRec1 = MB_ABA_REC * 128;
 // launch configurations: threads per block, work-area class, stack slots (double2) held in tensor memory
 struct Cfg
@@ -76,19 +84,30 @@ constexpr Cfg kCfg[kNumCfg] = {{512, 0, 32}, {384, 0, 42}, {320, 0, 42}, {256, 0
 
 typedef void (*KernelFn)(const MbProgram, const KernelArgs);
 
+// work area (doubles) of an algorithm's class 0 / 1
+__host__ __device__ constexpr int aux_of(int algo, int cls)
+{
+   return algo == MB_RNEA ? (cls ? kRnaAux1 : kRnaAux0)
+                          : (algo == MB_ABA ? (cls ? kAbaAux1 : kAbaAux0)
+                                            : (algo == MB_CRBA ? (cls ? kCrbAux1 : kCrbAux0)
+                                                               : (algo == MB_REGRESSOR ? (cls ? kRegAux1 : kRegAux0) : (cls ? kCorAux1 : kCorAux0))));
+}
+// the kernels whose stack lives in shared memory only (no wide area): their TMEM configurations alias the shared-memory kernels
+__host__ __device__ constexpr bool smem_stack_only(int algo) { return algo == MB_CRBA || algo == MB_CORIOLIS || algo == MB_REGRESSOR; }
+
 template <int ALGO, bool FEXT, int SM, bool M3> KernelFn pick_cfg(int cfg)
 {
-   constexpr int a0 = ALGO == MB_RNEA ? kRnaAux0 : (ALGO == MB_ABA ? kAbaAux0 : (ALGO == MB_CRBA ? kCrbAux0 : kCorAux0));
-   constexpr int a1 = ALGO == MB_RNEA ? kRnaAux1 : (ALGO == MB_ABA ? kAbaAux1 : (ALGO == MB_CRBA ? kCrbAux1 : kCorAux1));
+   constexpr int a0 = aux_of(ALGO, 0);
+   constexpr int a1 = aux_of(ALGO, 1);
    constexpr int r0 = ALGO == MB_ABA ? kAbaRec0 : 0, r1 = ALGO == MB_ABA ? kAbaRec1 : 0;
    switch (cfg)
    {
       // CRBA has no wide stack area: its TMEM configurations are never planned (mb_tm_fits) and alias the shared-memory kernels
-#define MB_CFG_CASE(i) case i: return thread_kernel<ALGO, FEXT, SM, kCfg[i].block, kCfg[i].cls ? a1 : a0, kCfg[i].cls ? r1 : r0, (ALGO == MB_CRBA || ALGO == MB_CORIOLIS) ? 0 : kCfg[i].tm, M3>;
+#define MB_CFG_CASE(i) case i: return thread_kernel<ALGO, FEXT, SM, kCfg[i].block, kCfg[i].cls ? a1 : a0, kCfg[i].cls ? r1 : r0, smem_stack_only(ALGO) ? 0 : kCfg[i].tm, M3>;
       MB_CFG_CASE(0) MB_CFG_CASE(1) MB_CFG_CASE(2) MB_CFG_CASE(3) MB_CFG_CASE(4) MB_CFG_CASE(5) MB_CFG_CASE(6)
       MB_CFG_CASE(7) MB_CFG_CASE(8) MB_CFG_CASE(9) MB_CFG_CASE(10) MB_CFG_CASE(11) MB_CFG_CASE(12) MB_CFG_CASE(14)
 #undef MB_CFG_CASE
-      default: return thread_kernel<ALGO, FEXT, SM, kCfg[13].block, a1, r1, (ALGO == MB_CRBA || ALGO == MB_CORIOLIS) ? 0 : kCfg[13].tm, M3>;
+      default: return thread_kernel<ALGO, FEXT, SM, kCfg[13].block, a1, r1, smem_stack_only(ALGO) ? 0 : kCfg[13].tm, M3>;
    }
 }
 
@@ -96,13 +115,13 @@ template <int ALGO, bool FEXT, int SM, bool M3> KernelFn pick_cfg(int cfg)
 constexpr int kF32Cfg[3] = {0, 1, 8}; // RNEA 512 threads + TMEM, ABA 384 threads + TMEM, CRBA 128 threads
 KernelFn pick_f32(int algo);
 
-// the instantiation groups: X(group, ALGO, FEXT, LAYOUT, M3).  The two store-bound matrix kernels (CRBA, Coriolis) exist only
+// the instantiation groups: X(group, ALGO, FEXT, LAYOUT, M3).  The store-bound matrix kernels (CRBA, Coriolis, regressor) exist only
 // with the three-DoF joints compiled in (one unit-momentum column loop per multi-DoF joint either way); RNEA and ABA come in
 // both forms (multidof.cuh: mb_sub_of)
 #define MB_KERNEL_GROUPS(X)                                                                                             \
    X(0, MB_RNEA, false, 0, false) X(1, MB_RNEA, true, 0, false) X(2, MB_ABA, false, 0, false) X(3, MB_ABA, true, 0, false)  \
    X(4, MB_CRBA, false, 0, true) X(5, MB_CRBA, false, 1, true) X(6, MB_CRBA, false, 2, true) X(7, MB_CRBA, true, 0, true)   \
    X(8, MB_CORIOLIS, false, 0, true) X(9, MB_RNEA, false, 0, true) X(10, MB_RNEA, true, 0, true)                            \
-   X(11, MB_ABA, false, 0, true) X(12, MB_ABA, true, 0, true)
-#define MB_NUM_KERNEL_GROUPS 13 // + group 13: the fp32 variant
+   X(11, MB_ABA, false, 0, true) X(12, MB_ABA, true, 0, true) X(14, MB_REGRESSOR, false, 0, true)
+#define MB_NUM_KERNEL_GROUPS 14 // + group 13: the fp32 variant
 } // namespace mb

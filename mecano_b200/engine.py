@@ -211,6 +211,22 @@ class Engine:
         else:
             check(lib.mecano_b200_coriolis(self._h, n, ld, pq, pqd, pm, pc, self._stream()), self._h)
 
+    def joint_torque_regressor(self, q, qd, qdd, Y):
+        """Y [nv * 10 nb, n] entry-major (mecano_b200_joint_torque_regressor); torch CUDA tensors or numpy arrays (host path)."""
+        n = q.shape[1]
+        host = isinstance(q, np.ndarray)
+        f = _host_ptr_ld if host else self._dp
+        pq, l0 = f(q, self.nq, n)
+        pqd, l1 = f(qd, self.nv, n)
+        pqdd, l2 = f(qdd, self.nv, n)
+        py, l3 = f(Y, self.nv * 10 * self.nb, n)
+        ld = _same_ld([l0, l1, l2, l3])
+        if host:
+            check(lib.mecano_b200_joint_torque_regressor_host(self._h, n, ld, pq, pqd, pqdd, py), self._h)
+        else:
+            check(lib.mecano_b200_joint_torque_regressor(self._h, n, ld, pq, pqd, pqdd, py, self._stream()), self._h)
+        return Y
+
     def crba_centroidal(self, q, M, cmm, com, frame=_capi.FRAME_WORLD):
         """M [nv*nv, n] entry-major, cmm [6*nv, n], com [4, n]; torch CUDA tensors or numpy arrays (host path)."""
         n = q.shape[1]
@@ -467,6 +483,7 @@ class MultiDeviceEngine:
         raise NotImplementedError("this entry point is served per device: build the calculator on one device")
 
     aba_sources_host = coriolis = crba_centroidal = centroidal_convective_term = center_of_mass = integrate_host = set_joint_source_modes = _single_device_only
+    joint_torque_regressor = _single_device_only
 
 
 def measure_fp64_peak(device=0):
