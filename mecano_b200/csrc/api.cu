@@ -7,6 +7,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <mutex>
 #include <string>
 #include <utility>
@@ -246,7 +247,9 @@ int run(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q,
             h->zero_row_doubles = 0;
          }
          MB_CUDA(h, cudaMalloc(&h->d_zero_row, (size_t)n * sizeof(double)));
-         MB_CUDA(h, cudaMemset(h->d_zero_row, 0, (size_t)n * sizeof(double)));
+         // zeroed before any stream reads it: the host pipeline's slots launch on other streams
+         MB_CUDA(h, cudaMemsetAsync(h->d_zero_row, 0, (size_t)n * sizeof(double), stream));
+         MB_CUDA(h, cudaStreamSynchronize(stream));
          h->zero_row_doubles = (size_t)n;
       }
       if (flags & MECANO_B200_RNEA_NO_CORIOLIS) { a.qd = h->d_zero_row; a.ld_qd = 0; }
@@ -292,16 +295,15 @@ int run(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q,
 // ForwardDynamicsCalculator.compute(tau, qdd_in) with per-joint source modes (ForwardDynamicsCalculator.java:508-520): passes one to
 // three in the ABA kernel; pass four (:1315-1363, the efforts of the ACCELERATION_SOURCE joints from the joint wrenches) is the upward
 // sweep of inverse dynamics on the accelerations just computed, i.e. one RNEA launch, after which the rows of the EFFORT_SOURCE
-// joints are restored to the caller's input as getJointTauMatrix() returns them (:566-590).
+// joints are restored to the caller's input as getJointTauMatrix() returns them (:566-590).  opt: ws_slot and variant_n only.
 int run_aba_sources(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *qdd_in,
-                    const double *fext, double *qdd, double *tau_out, cudaStream_t stream, int ws_slot)
+                    const double *fext, double *qdd, double *tau_out, cudaStream_t stream, RunOpts opt)
 {
    if (h->n_accel_source > 0 && !qdd_in)
       return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer (qdd_in) with joints in ACCELERATION_SOURCE mode");
-   RunOpts opt;
-   opt.ws_slot = ws_slot;
-   opt.x2 = qdd_in;
-   int rc = run(h, MB_ABA, n, ld, q, qd, tau, fext, qdd, 0u, stream, opt);
+   RunOpts aba = opt;
+   aba.x2 = qdd_in;
+   int rc = run(h, MB_ABA, n, ld, q, qd, tau, fext, qdd, 0u, stream, aba);
    if (rc || !tau_out)
       return rc;
    const size_t row = (size_t)ld * sizeof(double);
@@ -313,7 +315,7 @@ int run_aba_sources(mecano_b200_handle *h, int64_t n, int64_t ld, const double *
    }
    if (tau_out == tau)
       return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "tau_out must not alias tau when joints are in ACCELERATION_SOURCE mode");
-   rc = run(h, MB_RNEA, n, ld, q, qd, qdd, fext, tau_out, 0u, stream);
+   rc = run(h, MB_RNEA, n, ld, q, qd, qdd, fext, tau_out, 0u, stream, opt);
    if (rc) return rc;
    for (const auto &r : h->effort_dof_runs)
       MB_CUDA(h, cudaMemcpy2DAsync(tau_out + (size_t)r.first * ld, row, tau + (size_t)r.first * ld, row, (size_t)n * sizeof(double), (size_t)r.second,
@@ -366,86 +368,86 @@ cudaError_t copy_rows(double *dst, size_t dpitch, const double *src, size_t spit
 }
 
 // ------------------------------------------------------------------------------------------------ host-pointer pipeline
-// One host-pointer call on one handle ("lane"): pointers already offset to the lane's first state.  MB_STEP = the fused call
-// of the three calculators (mecano_b200_step_host).
-constexpr int MB_STEP = 100;
+// One host-pointer call on one handle ("lane"), declared as host matrices (entry-major, leading dimension ld) and the steps that
+// run on every chunk of states.  The pipeline stages each chunk in one slot: the inputs are uploaded, then each step is launched
+// and its outputs are copied back.  Pointers are already offset to the lane's first state.
+enum CopyBack
+{
+   COPY_ROWS,        // entry-major rows
+   COPY_STATES,      // state-major: `rows` contiguous doubles per state
+   COPY_NONZERO_RUNS // entry-major, the rows of h->nonzero_runs only (CRBA ZEROS_PRESENT: the host matrix already holds the zeros)
+};
+struct HostIn
+{
+   const double *host; // NULL: absent (no device rows)
+   size_t rows;
+};
+struct HostOut
+{
+   double *host; // NULL: device-only scratch
+   size_t rows;  // 0: absent
+   CopyBack how = COPY_ROWS;
+   int in = -1; // >= 0: written in place into the device rows of that input
+};
+// what a step's launch sees: the chunk's device rows (leading dimension ld = the chunk; NULL for an absent matrix) of every input
+// and of the step's outputs, the chunk width w and the slot's stream and options (ws_slot, variant_n)
+struct Chunk
+{
+   mecano_b200_handle *h;
+   std::vector<double *> in, out;
+   int64_t w = 0, ld = 0;
+   cudaStream_t stream = nullptr;
+   RunOpts opt;
+};
+struct HostStep
+{
+   std::function<int(const Chunk &)> launch;
+   std::vector<HostOut> out;
+};
 struct HostJob
 {
-   int algo = MB_RNEA;
    int64_t n = 0, ld = 0;
-   int64_t variant_n = 0;                               // size of the whole call (all lanes)
-   const double *q = nullptr, *qd = nullptr, *x = nullptr, *fext = nullptr, *x2 = nullptr; // x: qdd (RNEA) / tau (ABA); MB_STEP: qdd_in
-   const double *tau_in = nullptr;                       // MB_STEP: efforts for forward dynamics
-   double *out = nullptr;                                // tau (RNEA) / qdd (ABA) / mass matrix (CRBA); MB_STEP: tau_out
-   double *body_acc = nullptr, *joint_wrench = nullptr, *tau_out = nullptr; // by-products (RNEA), efforts of pass four (ABA with source modes)
-   double *qdd_out = nullptr, *M = nullptr;              // MB_STEP
-   uint32_t flags = 0;                                   // RNEA flags / CRBA layout (MB_STEP: layout)
+   std::vector<HostIn> in;
+   std::vector<HostStep> steps;
+   int64_t variant_n = 0; // size of the whole call (all lanes)
+   // staging per slot (r06ze: 229 ms per dense 2^20-state step against 239 ms with 128 MB, 231 ms with 512 MB)
+   double budget_mb = 256.0;
    // pipeline state
-   size_t chunk = 0, in_rows = 0, out_rows = 0, m_rows = 0;
+   size_t chunk = 0;
    int64_t s0 = 0;
    int slot = 0;
 };
 
-size_t mass_matrix_rows(const mecano_b200_handle *h, uint32_t layout)
-{
-   return (layout & MECANO_B200_CRBA_PACKED) ? h->tree.packed_row.size() : (size_t)h->tree.nv * (size_t)h->tree.nv;
-}
-
-// argument checks, chunk size, staging buffers.  Two slots per handle, each with its own stream: H2D of chunk k+1 overlaps the
-// kernels and the D2H of chunk k.
+// chunk size and staging buffers (arguments are checked by the entry points).  n_slots slots per handle, each with its own stream:
+// H2D of chunk k+1 overlaps the kernels and the D2H of chunk k.
 int host_begin(mecano_b200_handle *h, HostJob &j)
 {
-   int rc = check_batch(h, j.n, j.ld);
-   if (rc) return rc;
    if (j.n == 0) return MECANO_B200_OK;
-   const size_t nq = h->tree.nq, nv = h->tree.nv, nb = h->tree.nb;
-   if (j.algo == MB_STEP)
-   {
-      const bool rnea = j.x || j.out, aba = j.tau_in || j.qdd_out;
-      if (!j.q || ((rnea || aba) && !j.qd) || (rnea && (!j.x || !j.out)) || (aba && (!j.tau_in || !j.qdd_out)) || (!rnea && !aba && !j.M))
-         return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-      if (aba && h->n_accel_source > 0)
-         return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "joints in ACCELERATION_SOURCE mode need their accelerations: call mecano_b200_aba_sources_host");
-      // (state-major: as below, the kernel rewrites the structural zeros in the staging buffer every time)
-      if (j.flags & MECANO_B200_CRBA_STATE_MAJOR)
-         j.flags &= ~MECANO_B200_CRBA_ZEROS_PRESENT;
-      j.m_rows = j.M ? mass_matrix_rows(h, j.flags) : 0;
-      j.in_rows = nq + (rnea || aba ? nv : 0) + (rnea ? nv : 0) + (aba ? nv : 0) + (j.fext ? 6 * nb : 0);
-      j.out_rows = (rnea ? nv : 0) + (aba ? nv : 0) + j.m_rows;
-   }
-   else
-   {
-      if (!j.q || !j.out || (j.algo != MB_CRBA && (!j.qd || !j.x)))
-         return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-      // state-major: the whole per-state block is copied back from the staging buffer, which other calls on this handle reuse, so
-      // the kernel must write the structural zeros there every time (the transfer saving of ZEROS_PRESENT is entry-major only)
-      if (j.algo == MB_CRBA && (j.flags & MECANO_B200_CRBA_STATE_MAJOR))
-         j.flags &= ~MECANO_B200_CRBA_ZEROS_PRESENT;
-      j.m_rows = j.algo == MB_CRBA ? mass_matrix_rows(h, j.flags) : 0;
-      j.in_rows = j.algo == MB_CRBA ? nq : nq + 2 * nv + (j.fext ? 6 * nb : 0) + (j.x2 ? nv : 0);
-      j.out_rows = j.algo == MB_CRBA ? j.m_rows : nv + (j.body_acc ? 6 * nb : 0) + (j.joint_wrench ? 6 * nb : 0) + (j.tau_out ? nv : 0);
-   }
-   if ((j.flags & MECANO_B200_CRBA_PACKED) && (j.flags & (MECANO_B200_CRBA_STATE_MAJOR | MECANO_B200_CRBA_ZEROS_PRESENT)) && (j.algo == MB_CRBA || j.algo == MB_STEP))
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the packed mass-matrix layout does not combine with STATE_MAJOR / ZEROS_PRESENT");
-   // chunk: ~256 MB of rows per slot (MECANO_B200_HOST_CHUNK_MB; r06ze: 229 ms per dense 2^20-state step against 239 ms with 128 MB, 231 ms with
-   // 512 MB), at least 4096 states, multiple of 256
-   static const double chunk_mb = [] { const char *e = getenv("MECANO_B200_HOST_CHUNK_MB"); const double v = e ? atof(e) : 0.0; return v >= 1.0 ? v : 256.0; }();
-   size_t chunk = (size_t)(chunk_mb * 1024 * 1024 / 8 / (double)(j.in_rows + j.out_rows));
-   chunk = std::max<size_t>(4096, chunk & ~(size_t)255);
+   size_t rows = 0; // device rows per state of one slot
+   for (const HostIn &i : j.in)
+      rows += i.host ? i.rows : 0;
+   for (const HostStep &s : j.steps)
+      for (const HostOut &o : s.out)
+         rows += o.in < 0 ? o.rows : 0;
+   // chunk: the job's budget of rows per slot (MECANO_B200_HOST_CHUNK_MB overrides every job's), multiple of 256, at least 256 states
+   // (no more: a wide job -- the regressor, a dense mass matrix of nv > 90 -- would otherwise make every slot far larger than the budget)
+   static const double env_mb = [] { const char *e = getenv("MECANO_B200_HOST_CHUNK_MB"); const double v = e ? atof(e) : 0.0; return v >= 1.0 ? v : 0.0; }();
+   size_t chunk = (size_t)((env_mb > 0.0 ? env_mb : j.budget_mb) * 1024 * 1024 / 8 / (double)rows);
+   chunk = std::max<size_t>(256, chunk & ~(size_t)255);
    chunk = std::min<size_t>(chunk, ((size_t)j.n + 255) & ~(size_t)255);
    j.chunk = chunk;
    j.s0 = 0;
    j.slot = 0;
    MB_ON_DEVICE(h);
-   return ensure_pipeline(h, (j.in_rows + j.out_rows) * chunk);
+   return ensure_pipeline(h, rows * chunk);
 }
 
-// issues the next chunk of the job (H2D, kernels, D2H on the slot's stream); asynchronous with pinned host memory
+// issues the next chunk of the job (H2D, then each step's kernels and D2H, on the slot's stream); asynchronous with pinned host memory
 int host_issue_chunk(mecano_b200_handle *h, HostJob &j)
 {
    if (j.s0 >= j.n) return MECANO_B200_OK;
    MB_ON_DEVICE(h);
-   const size_t nq = h->tree.nq, nv = h->tree.nv, nb = h->tree.nb, chunk = j.chunk, ld = (size_t)j.ld;
+   const size_t chunk = j.chunk, ld = (size_t)j.ld;
    const int64_t s0 = j.s0;
    const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, j.n - s0);
    const int slot = j.slot;
@@ -454,94 +456,42 @@ int host_issue_chunk(mecano_b200_handle *h, HostJob &j)
    j.slot = (slot + 1) % h->n_slots;
    // a slot is reused every n_slots chunks: stream order already serialises it
    double *p = h->stage[slot];
-   auto take = [&](size_t rows) { double *r = p; p += rows * chunk; return r; };
-   auto h2d = [&](double *dst, const double *src, size_t rows) { return copy_rows(dst, chunk, src + s0, ld, w, rows, cudaMemcpyHostToDevice, st); };
-   auto d2h = [&](double *dst, const double *src, size_t rows) { return copy_rows(dst + s0, ld, src, chunk, w, rows, cudaMemcpyDeviceToHost, st); };
-   int rc = MECANO_B200_OK;
-   RunOpts opt;
-   opt.ws_slot = 1 + slot;
-   opt.variant_n = j.variant_n > 0 ? j.variant_n : j.n;
-   if (j.algo == MB_STEP)
+   Chunk c{h, {}, {}, (int64_t)w, (int64_t)chunk, st};
+   c.opt.ws_slot = 1 + slot;
+   c.opt.variant_n = j.variant_n > 0 ? j.variant_n : j.n;
+   for (const HostIn &i : j.in)
    {
-      const bool rnea = j.x != nullptr, aba = j.tau_in != nullptr;
-      double *dq = take(nq), *dqd = (rnea || aba) ? take(nv) : nullptr, *dqdd = rnea ? take(nv) : nullptr, *dtin = aba ? take(nv) : nullptr;
-      double *df = j.fext ? take(6 * nb) : nullptr;
-      double *dtau = rnea ? take(nv) : nullptr, *dqo = aba ? take(nv) : nullptr, *dM = j.M ? take(j.m_rows) : nullptr;
-      MB_CUDA(h, h2d(dq, j.q, nq));
-      if (dqd) MB_CUDA(h, h2d(dqd, j.qd, nv));
-      if (dqdd) MB_CUDA(h, h2d(dqdd, j.x, nv));
-      if (dtin) MB_CUDA(h, h2d(dtin, j.tau_in, nv));
-      if (df) MB_CUDA(h, h2d(df, j.fext, 6 * nb));
-      if (rnea)
+      c.in.push_back(i.host ? p : nullptr);
+      if (!i.host) continue;
+      MB_CUDA(h, copy_rows(p, chunk, i.host + s0, ld, w, i.rows, cudaMemcpyHostToDevice, st));
+      p += i.rows * chunk;
+   }
+   for (const HostStep &s : j.steps)
+   {
+      c.out.clear();
+      for (const HostOut &o : s.out)
       {
-         rc = run(h, MB_RNEA, (int64_t)w, (int64_t)chunk, dq, dqd, dqdd, df, dtau, 0u, st, opt);
-         if (rc) return rc;
-         MB_CUDA(h, d2h(j.out, dtau, nv));
+         c.out.push_back(o.in >= 0 ? c.in[(size_t)o.in] : (o.rows ? p : nullptr));
+         if (o.in < 0) p += o.rows * chunk;
       }
-      if (aba)
+      const int rc = s.launch(c);
+      if (rc) return rc;
+      for (size_t k = 0; k < s.out.size(); k++)
       {
-         rc = run(h, MB_ABA, (int64_t)w, (int64_t)chunk, dq, dqd, dtin, df, dqo, 0u, st, opt);
-         if (rc) return rc;
-         MB_CUDA(h, d2h(j.qdd_out, dqo, nv));
-      }
-      if (j.M)
-      {
-         rc = run(h, MB_CRBA, (int64_t)w, (int64_t)chunk, dq, nullptr, nullptr, nullptr, dM, j.flags, st, opt);
-         if (rc) return rc;
-         if (j.flags & MECANO_B200_CRBA_STATE_MAJOR)
-            MB_CUDA(h, cudaMemcpyAsync(j.M + (size_t)s0 * nv * nv, dM, w * nv * nv * sizeof(double), cudaMemcpyDeviceToHost, st));
-         else if (j.flags & MECANO_B200_CRBA_ZEROS_PRESENT)
+         const HostOut &o = s.out[k];
+         const double *d = c.out[k];
+         if (!o.host || !o.rows) continue;
+         if (o.how == COPY_STATES)
+            MB_CUDA(h, cudaMemcpyAsync(o.host + (size_t)s0 * o.rows, d, w * o.rows * sizeof(double), cudaMemcpyDeviceToHost, st));
+         else if (o.how == COPY_NONZERO_RUNS)
          {
-            // entry-major: a structurally zero entry is a whole row of the host matrix, which already holds zeros (and which the
-            // kernel did not write in the staging buffer)
             for (const auto &run : h->nonzero_runs)
-               MB_CUDA(h, copy_rows(j.M + (size_t)run.first * ld + s0, ld, dM + (size_t)run.first * chunk, chunk, w, (size_t)run.second, cudaMemcpyDeviceToHost, st));
+               MB_CUDA(h, copy_rows(o.host + (size_t)run.first * ld + s0, ld, d + (size_t)run.first * chunk, chunk, w, (size_t)run.second, cudaMemcpyDeviceToHost, st));
          }
          else
-            MB_CUDA(h, d2h(j.M, dM, j.m_rows));
+            MB_CUDA(h, copy_rows(o.host + s0, ld, d, chunk, w, o.rows, cudaMemcpyDeviceToHost, st));
       }
-      return MECANO_B200_OK;
    }
-   const int algo = j.algo;
-   const bool state_major = algo == MB_CRBA && (j.flags & MECANO_B200_CRBA_STATE_MAJOR);
-   const bool sources = algo == MB_ABA && (j.x2 || j.tau_out); // mecano_b200_aba_sources_host
-   double *dq = take(nq), *dqd = nullptr, *dx = nullptr, *df = nullptr, *dx2 = nullptr;
-   MB_CUDA(h, h2d(dq, j.q, nq));
-   if (algo != MB_CRBA)
-   {
-      dqd = take(nv);
-      dx = take(nv);
-      MB_CUDA(h, h2d(dqd, j.qd, nv));
-      MB_CUDA(h, h2d(dx, j.x, nv));
-      if (j.fext) { df = take(6 * nb); MB_CUDA(h, h2d(df, j.fext, 6 * nb)); }
-      if (j.x2) { dx2 = take(nv); MB_CUDA(h, h2d(dx2, j.x2, nv)); }
-   }
-   double *dout = take(algo == MB_CRBA ? j.m_rows : nv);
-   double *dacc = j.body_acc ? take(6 * nb) : nullptr;
-   double *dwr = j.joint_wrench ? take(6 * nb) : nullptr;
-   double *dtau = j.tau_out ? take(nv) : nullptr;
-   if (sources)
-      rc = run_aba_sources(h, (int64_t)w, (int64_t)chunk, dq, dqd, dx, dx2, df, dout, dtau, st, 1 + slot);
-   else
-   {
-      opt.body_acc = dacc;
-      opt.joint_wrench = dwr;
-      rc = run(h, algo, (int64_t)w, (int64_t)chunk, dq, dqd, dx, df, dout, j.flags, st, opt);
-   }
-   if (rc) return rc;
-   if (dtau) MB_CUDA(h, d2h(j.tau_out, dtau, nv));
-   if (dacc) MB_CUDA(h, d2h(j.body_acc, dacc, 6 * nb));
-   if (dwr) MB_CUDA(h, d2h(j.joint_wrench, dwr, 6 * nb));
-   if (state_major)
-      MB_CUDA(h, cudaMemcpyAsync(j.out + (size_t)s0 * nv * nv, dout, w * nv * nv * sizeof(double), cudaMemcpyDeviceToHost, st));
-   else if (algo == MB_CRBA && (j.flags & MECANO_B200_CRBA_ZEROS_PRESENT))
-   {
-      // entry-major: a structurally zero entry is a whole row of the host matrix, which already holds zeros
-      for (const auto &run : h->nonzero_runs)
-         MB_CUDA(h, copy_rows(j.out + (size_t)run.first * ld + s0, ld, dout + (size_t)run.first * chunk, chunk, w, (size_t)run.second, cudaMemcpyDeviceToHost, st));
-   }
-   else
-      MB_CUDA(h, d2h(j.out, dout, algo == MB_CRBA ? j.m_rows : nv));
    return MECANO_B200_OK;
 }
 
@@ -592,25 +542,147 @@ int run_host_lanes(const std::vector<mecano_b200_handle *> &lanes, std::vector<H
    return rc;
 }
 
-int run_host(mecano_b200_handle *h, HostJob &job)
+int run_host(mecano_b200_handle *h, const HostJob &job)
 {
-   if (!h) return MECANO_B200_ERR_INVALID_ARGUMENT;
    std::vector<mecano_b200_handle *> lanes(1, h);
    std::vector<HostJob> jobs(1, job);
    int failed = 0;
    return run_host_lanes(lanes, jobs, &failed);
 }
 
-int run_host(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q, const double *qd, const double *x, const double *fext,
-             double *out, uint32_t flags, double *body_acc = nullptr, double *joint_wrench = nullptr, const double *x2 = nullptr,
-             double *tau_out = nullptr)
+// The jobs of the RNEA / ABA / CRBA host calls, single- and multi-device: argument checks (an empty batch gives an empty job), then
+// the job.
+int rnea_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext, double *tau,
+             double *body_acc, double *joint_wrench, uint32_t flags, HostJob &j)
 {
-   HostJob j;
-   j.algo = algo; j.n = n; j.ld = ld;
-   j.q = q; j.qd = qd; j.x = x; j.fext = fext; j.x2 = x2;
-   j.out = out; j.body_acc = body_acc; j.joint_wrench = joint_wrench; j.tau_out = tau_out;
-   j.flags = flags;
-   return run_host(h, j);
+   int rc = check_batch(h, n, ld);
+   if (rc || n == 0) return rc;
+   if (!q || !qd || !qdd || !tau) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   const size_t nq = h->tree.nq, nv = h->tree.nv, nw = 6 * (size_t)h->tree.nb;
+   j = HostJob{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}, {fext, nw}}};
+   j.steps.push_back({[flags](const Chunk &c) {
+      RunOpts opt = c.opt;
+      opt.body_acc = c.out[1];
+      opt.joint_wrench = c.out[2];
+      return run(c.h, MB_RNEA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[0], flags, c.stream, opt);
+   }, {{tau, nv}, {body_acc, body_acc ? nw : 0}, {joint_wrench, joint_wrench ? nw : 0}}});
+   return MECANO_B200_OK;
+}
+
+// qdd_in / tau_out given: mecano_b200_aba_sources_host
+int aba_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *qdd_in,
+            const double *fext, double *qdd, double *tau_out, uint32_t flags, HostJob &j)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc || n == 0) return rc;
+   if (!q || !qd || !tau || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   const bool sources = qdd_in || tau_out;
+   j = HostJob{n, ld, {{q, nq}, {qd, nv}, {tau, nv}, {fext, 6 * (size_t)h->tree.nb}, {qdd_in, nv}}};
+   j.steps.push_back({[flags, sources](const Chunk &c) {
+      if (sources) return run_aba_sources(c.h, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[4], c.in[3], c.out[0], c.out[1], c.stream, c.opt);
+      return run(c.h, MB_ABA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[0], flags, c.stream, c.opt);
+   }, {{qdd, nv}, {tau_out, tau_out ? nv : 0}}});
+   return MECANO_B200_OK;
+}
+
+// mecano_b200_step_host: inputs q, qd, qdd_in, tau_in, fext; steps RNEA -> tau_out, ABA -> qdd_out, CRBA -> M, each one present
+// when its buffers are (M alone: mecano_b200_crba_host)
+int step_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd_in, const double *tau_in,
+             const double *fext, double *tau_out, double *qdd_out, double *M, uint32_t layout, HostJob &j)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc || n == 0) return rc;
+   const bool rnea = qdd_in || tau_out, aba = tau_in || qdd_out;
+   if (!q || ((rnea || aba) && !qd) || (rnea && (!qdd_in || !tau_out)) || (aba && (!tau_in || !qdd_out)) || (!rnea && !aba && !M))
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (aba && h->n_accel_source > 0)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "joints in ACCELERATION_SOURCE mode need their accelerations: call mecano_b200_aba_sources_host");
+   if ((layout & MECANO_B200_CRBA_PACKED) && (layout & (MECANO_B200_CRBA_STATE_MAJOR | MECANO_B200_CRBA_ZEROS_PRESENT)))
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the packed mass-matrix layout does not combine with STATE_MAJOR / ZEROS_PRESENT");
+   // state-major: the whole per-state block is copied back from the staging buffer, which other calls on this handle reuse, so
+   // the kernel must write the structural zeros there every time (the transfer saving of ZEROS_PRESENT is entry-major only)
+   if (layout & MECANO_B200_CRBA_STATE_MAJOR)
+      layout &= ~MECANO_B200_CRBA_ZEROS_PRESENT;
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   j = HostJob{n, ld, {{q, nq}, {rnea || aba ? qd : nullptr, nv}, {qdd_in, nv}, {tau_in, nv}, {fext, 6 * (size_t)h->tree.nb}}};
+   if (rnea)
+      j.steps.push_back({[](const Chunk &c) { return run(c.h, MB_RNEA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[4], c.out[0], 0u, c.stream, c.opt); },
+                         {{tau_out, nv}}});
+   if (aba)
+      j.steps.push_back({[](const Chunk &c) { return run(c.h, MB_ABA, c.w, c.ld, c.in[0], c.in[1], c.in[3], c.in[4], c.out[0], 0u, c.stream, c.opt); },
+                         {{qdd_out, nv}}});
+   if (M)
+   {
+      const CopyBack how = (layout & MECANO_B200_CRBA_STATE_MAJOR) ? COPY_STATES : (layout & MECANO_B200_CRBA_ZEROS_PRESENT) ? COPY_NONZERO_RUNS : COPY_ROWS;
+      j.steps.push_back({[layout](const Chunk &c) { return run(c.h, MB_CRBA, c.w, c.ld, c.in[0], nullptr, nullptr, nullptr, c.out[0], layout, c.stream, c.opt); },
+                         {{M, (layout & MECANO_B200_CRBA_PACKED) ? h->tree.packed_row.size() : nv * nv, how}}});
+   }
+   return MECANO_B200_OK;
+}
+
+// The kernels of mecano_b200_crba_centroidal (M, cmm given) and of mecano_b200_center_of_mass (M = cmm = NULL) on checked arguments.
+// The latter is the by-product CRBA kernel launched without a matrix: it keeps the composite-inertia recursion and drops the unit
+// momenta, their ancestor walks and every matrix store (crba.cuh: com_only) -- the same arithmetic, hence the same bits, as the com
+// rows of the former.
+int enqueue_centroidal(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame,
+                       cudaStream_t st, RunOpts opt)
+{
+   // the kernel sums (mass * CoM, mass) over the children of the root body into the com rows
+   MB_CUDA(h, cudaMemset2DAsync(com, (size_t)ld * sizeof(double), 0, (size_t)n * sizeof(double), 4, st));
+   opt.cmm = cmm;
+   opt.com = com;
+   const int rc = run(h, MB_CRBA, n, ld, q, nullptr, nullptr, nullptr, M, MECANO_B200_CRBA_ENTRY_MAJOR, st, opt);
+   if (rc) return rc;
+   mb::CentroidalArgs ca;
+   ca.cols = cmm; ca.com = com; ca.n = n; ca.ld = ld; ca.ncols = cmm ? h->tree.nv : 0;
+   ca.normalize_com = 1;
+   ca.shift = frame == MECANO_B200_FRAME_CENTER_OF_MASS;
+   MB_CUDA(h, mb::launch_centroidal_finish(ca, st));
+   return MECANO_B200_OK;
+}
+
+// The kernels of mecano_b200_centroidal_convective_term on checked arguments; tau: nv rows for the joint efforts nobody reads.
+int enqueue_convective_term(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *com, double *out,
+                            double *tau, int frame, cudaStream_t st, RunOpts opt)
+{
+   // :811-839: the net wrench of every body under zero joint accelerations and no gravity, summed in the centroidal frame = the
+   // wrench at the root of inverse dynamics run that way
+   MB_CUDA(h, cudaMemset2DAsync(out, (size_t)ld * sizeof(double), 0, (size_t)n * sizeof(double), 6, st));
+   opt.root_wrench = out;
+   opt.zero_gravity = true;
+   const int rc = run(h, MB_RNEA, n, ld, q, qd, qd, nullptr, tau, MECANO_B200_RNEA_NO_ACCELERATIONS, st, opt);
+   if (rc) return rc;
+   if (frame == MECANO_B200_FRAME_CENTER_OF_MASS)
+   {
+      mb::CentroidalArgs ca;
+      ca.cols = out; ca.com = const_cast<double *>(com); ca.n = n; ca.ld = ld; ca.ncols = 1;
+      ca.normalize_com = 0;
+      ca.shift = 1;
+      MB_CUDA(h, mb::launch_centroidal_finish(ca, st));
+   }
+   return MECANO_B200_OK;
+}
+
+// The kernel of mecano_b200_integrate on checked arguments.
+int enqueue_integrate(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, double *q, double *qd, double *qdd, cudaStream_t st)
+{
+   mb::IntegrateJoints J;
+   const MbProgram &P = h->tree.prog[MB_RNEA];
+   J.nb = P.nb;
+   for (int i = 0; i < P.nb; i++)
+   {
+      J.cfg[i] = (uint16_t)P.body[i].cfg_off;
+      J.dof[i] = (uint16_t)P.body[i].dof_off;
+      J.type[i] = (uint8_t)P.body[i].jtype;
+      J.sub[i] = (uint8_t)P.body[i].sub;
+   }
+   mb::IntegrateArgs a;
+   a.q = q; a.qd = qd; a.qdd = qdd;
+   a.n = n; a.ld = ld;
+   a.dt = dt;
+   MB_CUDA(h, mb::launch_integrate_kernel(J, a, h->sm_count, st));
+   return MECANO_B200_OK;
 }
 } // namespace
 
@@ -920,7 +992,7 @@ int mecano_b200_aba_sources(mecano_b200_handle *h, int64_t n, int64_t ld, const 
    if (n == 0) return MECANO_B200_OK;
    if (!q || !qd || !tau || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
    MB_ON_DEVICE(h);
-   return run_aba_sources(h, n, ld, q, qd, tau, qdd_in, fext, qdd, tau_out, (cudaStream_t)stream, 0);
+   return run_aba_sources(h, n, ld, q, qd, tau, qdd_in, fext, qdd, tau_out, (cudaStream_t)stream, RunOpts());
 }
 
 int mecano_b200_aba_sources_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau,
@@ -928,7 +1000,9 @@ int mecano_b200_aba_sources_host(mecano_b200_handle *h, int64_t n, int64_t ld, c
 {
    if (h && h->n_accel_source > 0 && !qdd_in)
       return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer (qdd_in) with joints in ACCELERATION_SOURCE mode");
-   return run_host(h, MB_ABA, n, ld, q, qd, tau, fext, qdd, 0u, nullptr, nullptr, qdd_in, tau_out);
+   HostJob j;
+   const int rc = aba_job(h, n, ld, q, qd, tau, qdd_in, fext, qdd, tau_out, 0u, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_crba_centroidal(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame,
@@ -941,26 +1015,11 @@ int mecano_b200_crba_centroidal(mecano_b200_handle *h, int64_t n, int64_t ld, co
    if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
       return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
    MB_ON_DEVICE(h);
-   cudaStream_t st = (cudaStream_t)stream;
-   // the kernel sums (mass * CoM, mass) over the children of the root body into the com rows
-   MB_CUDA(h, cudaMemset2DAsync(com, (size_t)ld * sizeof(double), 0, (size_t)n * sizeof(double), 4, st));
-   RunOpts opt;
-   opt.cmm = cmm;
-   opt.com = com;
-   rc = run(h, MB_CRBA, n, ld, q, nullptr, nullptr, nullptr, M, MECANO_B200_CRBA_ENTRY_MAJOR, st, opt);
-   if (rc) return rc;
-   mb::CentroidalArgs ca;
-   ca.cols = cmm; ca.com = com; ca.n = n; ca.ld = ld; ca.ncols = h->tree.nv;
-   ca.normalize_com = 1;
-   ca.shift = frame == MECANO_B200_FRAME_CENTER_OF_MASS;
-   MB_CUDA(h, mb::launch_centroidal_finish(ca, st));
-   return MECANO_B200_OK;
+   return enqueue_centroidal(h, n, ld, q, M, cmm, com, frame, (cudaStream_t)stream, RunOpts());
 }
 
 // The centre of mass alone (CenterOfMassCalculator.getCenterOfMass() / getTotalMass(), CenterOfMassCalculator.java:70-124; what
-// CenterOfMassReferenceFrame.updateTransformToParent(), CenterOfMassReferenceFrame.java:45-50, asks for): the by-product CRBA kernel
-// launched without a matrix keeps the composite-inertia recursion and drops the unit momenta, their ancestor walks and every
-// matrix store (crba.cuh: com_only) -- the same arithmetic, hence the same bits, as the com rows of mecano_b200_crba_centroidal.
+// CenterOfMassReferenceFrame.updateTransformToParent(), CenterOfMassReferenceFrame.java:45-50, asks for).
 int mecano_b200_center_of_mass(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *com, void *stream)
 {
    int rc = check_batch(h, n, ld);
@@ -968,18 +1027,7 @@ int mecano_b200_center_of_mass(mecano_b200_handle *h, int64_t n, int64_t ld, con
    if (n == 0) return MECANO_B200_OK;
    if (!q || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
    MB_ON_DEVICE(h);
-   cudaStream_t st = (cudaStream_t)stream;
-   MB_CUDA(h, cudaMemset2DAsync(com, (size_t)ld * sizeof(double), 0, (size_t)n * sizeof(double), 4, st));
-   RunOpts opt;
-   opt.com = com;
-   rc = run(h, MB_CRBA, n, ld, q, nullptr, nullptr, nullptr, nullptr, MECANO_B200_CRBA_ENTRY_MAJOR, st, opt);
-   if (rc) return rc;
-   mb::CentroidalArgs ca;
-   ca.cols = nullptr; ca.com = com; ca.n = n; ca.ld = ld; ca.ncols = 0;
-   ca.normalize_com = 1;
-   ca.shift = 0;
-   MB_CUDA(h, mb::launch_centroidal_finish(ca, st));
-   return MECANO_B200_OK;
+   return enqueue_centroidal(h, n, ld, q, nullptr, nullptr, com, MECANO_B200_FRAME_WORLD, (cudaStream_t)stream, RunOpts());
 }
 
 int mecano_b200_centroidal_convective_term(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *com,
@@ -994,7 +1042,6 @@ int mecano_b200_centroidal_convective_term(mecano_b200_handle *h, int64_t n, int
    if (frame == MECANO_B200_FRAME_CENTER_OF_MASS && !com)
       return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the centre-of-mass frame needs the com rows of mecano_b200_crba_centroidal");
    MB_ON_DEVICE(h);
-   cudaStream_t st = (cudaStream_t)stream;
    const size_t need = (size_t)h->tree.nv * (size_t)ld;
    if (h->scratch_doubles < need)
    {
@@ -1008,23 +1055,7 @@ int mecano_b200_centroidal_convective_term(mecano_b200_handle *h, int64_t n, int
       MB_CUDA(h, cudaMalloc(&h->d_scratch, need * sizeof(double)));
       h->scratch_doubles = need;
    }
-   // :811-839: the net wrench of every body under zero joint accelerations and no gravity, summed in the centroidal frame = the
-   // wrench at the root of inverse dynamics run that way
-   MB_CUDA(h, cudaMemset2DAsync(out, (size_t)ld * sizeof(double), 0, (size_t)n * sizeof(double), 6, st));
-   RunOpts opt;
-   opt.root_wrench = out;
-   opt.zero_gravity = true;
-   rc = run(h, MB_RNEA, n, ld, q, qd, qd, nullptr, h->d_scratch, MECANO_B200_RNEA_NO_ACCELERATIONS, st, opt);
-   if (rc) return rc;
-   if (frame == MECANO_B200_FRAME_CENTER_OF_MASS)
-   {
-      mb::CentroidalArgs ca;
-      ca.cols = out; ca.com = const_cast<double *>(com); ca.n = n; ca.ld = ld; ca.ncols = 1;
-      ca.normalize_com = 0;
-      ca.shift = 1;
-      MB_CUDA(h, mb::launch_centroidal_finish(ca, st));
-   }
-   return MECANO_B200_OK;
+   return enqueue_convective_term(h, n, ld, q, qd, com, out, h->d_scratch, frame, (cudaStream_t)stream, RunOpts());
 }
 
 int mecano_b200_coriolis(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, double *M, double *C, void *stream)
@@ -1047,29 +1078,16 @@ int mecano_b200_coriolis_host(mecano_b200_handle *h, int64_t n, int64_t ld, cons
    if (rc) return rc;
    if (n == 0) return MECANO_B200_OK;
    if (!q || !qd || !M || !C) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   std::lock_guard<std::mutex> lk(h->mu);
-   MB_ON_DEVICE(h);
-   const size_t nq = h->tree.nq, nv = h->tree.nv, rows = nq + nv + 2 * nv * nv;
-   const size_t chunk = (size_t)std::min<int64_t>(n, 16384);
-   double *d = nullptr;
-   MB_CUDA(h, cudaMalloc(&d, rows * chunk * sizeof(double)));
-   double *dq = d, *dqd = dq + nq * chunk, *dM = dqd + nv * chunk, *dC = dM + nv * nv * chunk;
-   cudaError_t e = cudaSuccess;
-   for (int64_t s0 = 0; s0 < n && rc == 0 && e == cudaSuccess; s0 += (int64_t)chunk)
-   {
-      const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, n - s0);
-      e = copy_rows(dq, chunk, q + s0, (size_t)ld, w, nq, cudaMemcpyHostToDevice, nullptr);
-      if (e == cudaSuccess) e = copy_rows(dqd, chunk, qd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, nullptr);
-      if (e != cudaSuccess) break;
-      rc = mecano_b200_coriolis(h, (int64_t)w, (int64_t)chunk, dq, dqd, dM, dC, nullptr);
-      if (rc) break;
-      e = copy_rows(M + s0, (size_t)ld, dM, chunk, w, nv * nv, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = copy_rows(C + s0, (size_t)ld, dC, chunk, w, nv * nv, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(nullptr);
-   }
-   cudaFree(d);
-   if (e != cudaSuccess) return cuda_fail(h, e, "mecano_b200_coriolis_host");
-   return rc;
+   if (h->plan[MB_CORIOLIS].block == 0)
+      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the Coriolis-matrix kernel (branch nesting / depth too large)");
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   HostJob j{n, ld, {{q, nq}, {qd, nv}}};
+   j.steps.push_back({[](const Chunk &c) {
+      RunOpts opt = c.opt;
+      opt.cor = c.out[1];
+      return run(c.h, MB_CORIOLIS, c.w, c.ld, c.in[0], c.in[1], c.in[1], nullptr, c.out[0], 0u, c.stream, opt);
+   }, {{M, nv * nv}, {C, nv * nv}}});
+   return run_host(h, j);
 }
 
 // the regressor's refusals shared by its two entry points (after check_batch)
@@ -1105,62 +1123,26 @@ int mecano_b200_joint_torque_regressor_host(mecano_b200_handle *h, int64_t n, in
    if ((rc = regressor_check(h))) return rc;
    if (n == 0) return MECANO_B200_OK;
    if (!q || !qd || !qdd || !Y) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   std::lock_guard<std::mutex> lk(h->mu);
-   MB_ON_DEVICE(h);
-   const size_t nq = h->tree.nq, nv = h->tree.nv, ny = nv * 10 * (size_t)h->tree.nb, rows = nq + 2 * nv + ny;
-   // chunks of at most 1 GiB of staging (94.7 KB of Y per state for a 32-body humanoid: 11 k states)
-   const size_t chunk = (size_t)std::min<int64_t>(n, (int64_t)std::max<size_t>(32, std::min<size_t>(16384, ((size_t)1 << 30) / (rows * sizeof(double)))));
-   double *d = nullptr;
-   MB_CUDA(h, cudaMalloc(&d, rows * chunk * sizeof(double)));
-   double *dq = d, *dqd = dq + nq * chunk, *dqdd = dqd + nv * chunk, *dY = dqdd + nv * chunk;
-   cudaError_t e = cudaSuccess;
-   for (int64_t s0 = 0; s0 < n && rc == 0 && e == cudaSuccess; s0 += (int64_t)chunk)
-   {
-      const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, n - s0);
-      e = copy_rows(dq, chunk, q + s0, (size_t)ld, w, nq, cudaMemcpyHostToDevice, nullptr);
-      if (e == cudaSuccess) e = copy_rows(dqd, chunk, qd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, nullptr);
-      if (e == cudaSuccess) e = copy_rows(dqdd, chunk, qdd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, nullptr);
-      if (e != cudaSuccess) break;
-      rc = mecano_b200_joint_torque_regressor(h, (int64_t)w, (int64_t)chunk, dq, dqd, dqdd, dY, nullptr);
-      if (rc) break;
-      e = copy_rows(Y + s0, (size_t)ld, dY, chunk, w, ny, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(nullptr);
-   }
-   cudaFree(d);
-   if (e != cudaSuccess) return cuda_fail(h, e, "mecano_b200_joint_torque_regressor_host");
-   return rc;
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   HostJob j{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}}};
+   j.steps.push_back({[](const Chunk &c) { return run(c.h, MB_REGRESSOR, c.w, c.ld, c.in[0], c.in[1], c.in[2], nullptr, c.out[0], 0u, c.stream, c.opt); },
+                      {{Y, nv * 10 * (size_t)h->tree.nb}}});
+   return run_host(h, j);
 }
 
-// host-pointer variants of the two centroidal calls: plain staging through temporary device buffers, chunk by chunk
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame)
 {
    int rc = check_batch(h, n, ld);
    if (rc) return rc;
    if (n == 0) return MECANO_B200_OK;
    if (!q || !M || !cmm || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   std::lock_guard<std::mutex> lk(h->mu);
-   MB_ON_DEVICE(h);
-   const size_t nq = h->tree.nq, nv = h->tree.nv, rows = nq + nv * nv + 6 * nv + 4;
-   const size_t chunk = (size_t)std::min<int64_t>(n, 16384);
-   double *d = nullptr;
-   MB_CUDA(h, cudaMalloc(&d, rows * chunk * sizeof(double)));
-   double *dq = d, *dM = dq + nq * chunk, *dA = dM + nv * nv * chunk, *dc = dA + 6 * nv * chunk;
-   cudaError_t e = cudaSuccess;
-   for (int64_t s0 = 0; s0 < n && rc == 0 && e == cudaSuccess; s0 += (int64_t)chunk)
-   {
-      const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, n - s0);
-      e = copy_rows(dq, chunk, q + s0, (size_t)ld, w, nq, cudaMemcpyHostToDevice, nullptr);
-      if (e != cudaSuccess) break;
-      rc = mecano_b200_crba_centroidal(h, (int64_t)w, (int64_t)chunk, dq, dM, dA, dc, frame, nullptr);
-      if (rc) break;
-      e = copy_rows(M + s0, (size_t)ld, dM, chunk, w, nv * nv, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = copy_rows(cmm + s0, (size_t)ld, dA, chunk, w, 6 * nv, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = copy_rows(com + s0, (size_t)ld, dc, chunk, w, 4, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(nullptr);
-   }
-   cudaFree(d);
-   if (e != cudaSuccess) return cuda_fail(h, e, "mecano_b200_crba_centroidal_host");
-   return rc;
+   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
+   const size_t nv = h->tree.nv;
+   HostJob j{n, ld, {{q, (size_t)h->tree.nq}}};
+   j.steps.push_back({[frame](const Chunk &c) { return enqueue_centroidal(c.h, c.w, c.ld, c.in[0], c.out[0], c.out[1], c.out[2], frame, c.stream, c.opt); },
+                      {{M, nv * nv}, {cmm, 6 * nv}, {com, 4}}});
+   return run_host(h, j);
 }
 
 int mecano_b200_centroidal_convective_term_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *com,
@@ -1170,29 +1152,16 @@ int mecano_b200_centroidal_convective_term_host(mecano_b200_handle *h, int64_t n
    if (rc) return rc;
    if (n == 0) return MECANO_B200_OK;
    if (!q || !qd || !out) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   std::lock_guard<std::mutex> lk(h->mu);
-   MB_ON_DEVICE(h);
-   const size_t nq = h->tree.nq, nv = h->tree.nv, rows = nq + nv + 4 + 6;
-   const size_t chunk = (size_t)std::min<int64_t>(n, 262144);
-   double *d = nullptr;
-   MB_CUDA(h, cudaMalloc(&d, rows * chunk * sizeof(double)));
-   double *dq = d, *dqd = dq + nq * chunk, *dc = dqd + nv * chunk, *dout = dc + 4 * chunk;
-   cudaError_t e = cudaSuccess;
-   for (int64_t s0 = 0; s0 < n && rc == 0 && e == cudaSuccess; s0 += (int64_t)chunk)
-   {
-      const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, n - s0);
-      e = copy_rows(dq, chunk, q + s0, (size_t)ld, w, nq, cudaMemcpyHostToDevice, nullptr);
-      if (e == cudaSuccess) e = copy_rows(dqd, chunk, qd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, nullptr);
-      if (e == cudaSuccess && com) e = copy_rows(dc, chunk, com + s0, (size_t)ld, w, 4, cudaMemcpyHostToDevice, nullptr);
-      if (e != cudaSuccess) break;
-      rc = mecano_b200_centroidal_convective_term(h, (int64_t)w, (int64_t)chunk, dq, dqd, com ? dc : nullptr, dout, frame, nullptr);
-      if (rc) break;
-      e = copy_rows(out + s0, (size_t)ld, dout, chunk, w, 6, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(nullptr);
-   }
-   cudaFree(d);
-   if (e != cudaSuccess) return cuda_fail(h, e, "mecano_b200_centroidal_convective_term_host");
-   return rc;
+   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
+   if (frame == MECANO_B200_FRAME_CENTER_OF_MASS && !com)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the centre-of-mass frame needs the com rows of mecano_b200_crba_centroidal");
+   const size_t nv = h->tree.nv;
+   HostJob j{n, ld, {{q, (size_t)h->tree.nq}, {qd, nv}, {com, 4}}};
+   // the joint efforts nobody reads live in the slot
+   j.steps.push_back({[frame](const Chunk &c) { return enqueue_convective_term(c.h, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.out[0], c.out[1], frame, c.stream, c.opt); },
+                      {{out, 6}, {nullptr, nv}}});
+   return run_host(h, j);
 }
 
 int mecano_b200_center_of_mass_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *com)
@@ -1201,27 +1170,10 @@ int mecano_b200_center_of_mass_host(mecano_b200_handle *h, int64_t n, int64_t ld
    if (rc) return rc;
    if (n == 0) return MECANO_B200_OK;
    if (!q || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   std::lock_guard<std::mutex> lk(h->mu);
-   MB_ON_DEVICE(h);
-   const size_t nq = h->tree.nq, rows = nq + 4;
-   const size_t chunk = (size_t)std::min<int64_t>(n, 262144);
-   double *d = nullptr;
-   MB_CUDA(h, cudaMalloc(&d, rows * chunk * sizeof(double)));
-   double *dq = d, *dc = dq + nq * chunk;
-   cudaError_t e = cudaSuccess;
-   for (int64_t s0 = 0; s0 < n && rc == 0 && e == cudaSuccess; s0 += (int64_t)chunk)
-   {
-      const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, n - s0);
-      e = copy_rows(dq, chunk, q + s0, (size_t)ld, w, nq, cudaMemcpyHostToDevice, nullptr);
-      if (e != cudaSuccess) break;
-      rc = mecano_b200_center_of_mass(h, (int64_t)w, (int64_t)chunk, dq, dc, nullptr);
-      if (rc) break;
-      e = copy_rows(com + s0, (size_t)ld, dc, chunk, w, 4, cudaMemcpyDeviceToHost, nullptr);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(nullptr);
-   }
-   cudaFree(d);
-   if (e != cudaSuccess) return cuda_fail(h, e, "mecano_b200_center_of_mass_host");
-   return rc;
+   HostJob j{n, ld, {{q, (size_t)h->tree.nq}}};
+   j.steps.push_back({[](const Chunk &c) { return enqueue_centroidal(c.h, c.w, c.ld, c.in[0], nullptr, nullptr, c.out[0], MECANO_B200_FRAME_WORLD, c.stream, c.opt); },
+                      {{com, 4}}});
+   return run_host(h, j);
 }
 
 int mecano_b200_crba(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, uint32_t layout, void *stream)
@@ -1237,19 +1189,23 @@ int mecano_b200_crba(mecano_b200_handle *h, int64_t n, int64_t ld, const double 
 int mecano_b200_rnea_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd,
                           const double *fext, double *tau, uint32_t flags)
 {
-   return run_host(h, MB_RNEA, n, ld, q, qd, qdd, fext, tau, flags);
+   return mecano_b200_rnea_full_host(h, n, ld, q, qd, qdd, fext, tau, nullptr, nullptr, flags);
 }
 
 int mecano_b200_rnea_full_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd,
                                const double *fext, double *tau, double *body_acc, double *joint_wrench, uint32_t flags)
 {
-   return run_host(h, MB_RNEA, n, ld, q, qd, qdd, fext, tau, flags, body_acc, joint_wrench);
+   HostJob j;
+   const int rc = rnea_job(h, n, ld, q, qd, qdd, fext, tau, body_acc, joint_wrench, flags, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_aba_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau,
                          const double *fext, double *qdd, uint32_t flags)
 {
-   return run_host(h, MB_ABA, n, ld, q, qd, tau, fext, qdd, flags);
+   HostJob j;
+   const int rc = aba_job(h, n, ld, q, qd, tau, nullptr, fext, qdd, nullptr, flags, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_integrate(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, double *q, double *qd, double *qdd, void *stream)
@@ -1260,22 +1216,7 @@ int mecano_b200_integrate(mecano_b200_handle *h, int64_t n, int64_t ld, double d
    if (!q || !qd || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
    if (!(dt == dt)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "dt is NaN");
    MB_ON_DEVICE(h);
-   mb::IntegrateJoints J;
-   const MbProgram &P = h->tree.prog[MB_RNEA];
-   J.nb = P.nb;
-   for (int i = 0; i < P.nb; i++)
-   {
-      J.cfg[i] = (uint16_t)P.body[i].cfg_off;
-      J.dof[i] = (uint16_t)P.body[i].dof_off;
-      J.type[i] = (uint8_t)P.body[i].jtype;
-      J.sub[i] = (uint8_t)P.body[i].sub;
-   }
-   mb::IntegrateArgs a;
-   a.q = q; a.qd = qd; a.qdd = qdd;
-   a.n = n; a.ld = ld;
-   a.dt = dt;
-   MB_CUDA(h, mb::launch_integrate_kernel(J, a, h->sm_count, (cudaStream_t)stream));
-   return MECANO_B200_OK;
+   return enqueue_integrate(h, n, ld, dt, q, qd, qdd, (cudaStream_t)stream);
 }
 
 int mecano_b200_integrate_host(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, double *q, double *qd, double *qdd)
@@ -1284,35 +1225,18 @@ int mecano_b200_integrate_host(mecano_b200_handle *h, int64_t n, int64_t ld, dou
    if (rc) return rc;
    if (n == 0) return MECANO_B200_OK;
    if (!q || !qd || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   std::lock_guard<std::mutex> lk(h->mu);
-   MB_ON_DEVICE(h);
-   const size_t nq = h->tree.nq, nv = h->tree.nv, rows = nq + 2 * nv;
-   size_t chunk = (size_t)(64.0 * 1024 * 1024 / 8 / (double)rows);
-   chunk = std::max<size_t>(4096, chunk & ~(size_t)255);
-   chunk = std::min<size_t>(chunk, ((size_t)n + 255) & ~(size_t)255);
-   rc = ensure_pipeline(h, rows * chunk);
-   if (rc) return rc;
-   int slot = 0;
-   for (int64_t s0 = 0; s0 < n; s0 += (int64_t)chunk, slot = (slot + 1) % h->n_slots)
-   {
-      const size_t w = (size_t)std::min<int64_t>((int64_t)chunk, n - s0);
-      cudaStream_t st = h->streams[slot];
-      double *dq = h->stage[slot], *dqd = dq + nq * chunk, *dx = dqd + nv * chunk;
-      MB_CUDA(h, copy_rows(dq, chunk, q + s0, (size_t)ld, w, nq, cudaMemcpyHostToDevice, st));
-      MB_CUDA(h, copy_rows(dqd, chunk, qd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, st));
-      MB_CUDA(h, copy_rows(dx, chunk, qdd + s0, (size_t)ld, w, nv, cudaMemcpyHostToDevice, st));
-      rc = mecano_b200_integrate(h, (int64_t)w, (int64_t)chunk, dt, dq, dqd, dx, st);
-      if (rc) return rc;
-      MB_CUDA(h, copy_rows(q + s0, (size_t)ld, dq, chunk, w, nq, cudaMemcpyDeviceToHost, st));
-      MB_CUDA(h, copy_rows(qd + s0, (size_t)ld, dqd, chunk, w, nv, cudaMemcpyDeviceToHost, st));
-      MB_CUDA(h, copy_rows(qdd + s0, (size_t)ld, dx, chunk, w, nv, cudaMemcpyDeviceToHost, st));
-   }
-   return host_finish(h);
+   if (!(dt == dt)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "dt is NaN");
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   HostJob j{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}}};
+   j.budget_mb = 64.0; // 2^20 H37 states on a B200 (1000 W), pinned: 22 ms per call against 24 ms with 256 MB per slot; pageable 148 against 153 ms
+   j.steps.push_back({[dt](const Chunk &c) { return enqueue_integrate(c.h, c.w, c.ld, dt, c.in[0], c.in[1], c.in[2], c.stream); },
+                      {{q, nq, COPY_ROWS, 0}, {qd, nv, COPY_ROWS, 1}, {qdd, nv, COPY_ROWS, 2}}});
+   return run_host(h, j);
 }
 
 int mecano_b200_crba_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, uint32_t layout)
 {
-   return run_host(h, MB_CRBA, n, ld, q, nullptr, nullptr, nullptr, M, layout);
+   return mecano_b200_step_host(h, n, ld, q, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, M, layout);
 }
 
 int mecano_b200_crba_packed_size(const mecano_b200_handle *h) { return h ? (int)h->tree.packed_row.size() : -1; }
@@ -1329,11 +1253,8 @@ int mecano_b200_step_host(mecano_b200_handle *h, int64_t n, int64_t ld, const do
                           const double *fext, double *tau_out, double *qdd_out, double *M, uint32_t layout)
 {
    HostJob j;
-   j.algo = MB_STEP; j.n = n; j.ld = ld;
-   j.q = q; j.qd = qd; j.x = qdd_in; j.tau_in = tau_in; j.fext = fext;
-   j.out = tau_out; j.qdd_out = qdd_out; j.M = M;
-   j.flags = layout;
-   return run_host(h, j);
+   const int rc = step_job(h, n, ld, q, qd, qdd_in, tau_in, fext, tau_out, qdd_out, M, layout, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_states, mecano_b200_kernel_info *info)
@@ -1501,39 +1422,37 @@ int multi_fail(mecano_b200_multi *m, int rc, int lane)
    return rc;
 }
 
-// one job per lane from a whole-batch job: pointers offset to the lane's first state (state-major mass matrices by whole states)
-int multi_run(mecano_b200_multi *m, const HostJob &whole)
+// One job per lane from the whole-batch job that `build` checks and declares on the first lane's handle: every pointer offset to the
+// lane's first state (state-major outputs by whole states).
+template <class Build>
+int multi_run(mecano_b200_multi *m, int64_t n, int64_t ld, const Build &build)
 {
    if (!m) return MECANO_B200_ERR_INVALID_ARGUMENT;
-   if (whole.n < 0 || whole.ld < whole.n)
+   if (n < 0 || ld < n)
    {
       m->error = "n_states must be >= 0 and ld >= n_states";
       return MECANO_B200_ERR_SHAPE;
    }
+   HostJob whole;
+   int rc = build(m->lanes[0], whole);
+   if (rc) return multi_fail(m, rc, 0);
    const int L = (int)m->lanes.size();
    std::vector<HostJob> jobs((size_t)L, whole);
    for (int i = 0; i < L; i++)
    {
       int64_t s0 = 0, cnt = 0;
-      multi_slice(whole.n, L, i, &s0, &cnt);
+      multi_slice(n, L, i, &s0, &cnt);
       HostJob &j = jobs[(size_t)i];
       j.n = cnt;
-      j.variant_n = whole.n;
-      auto off = [&](const double *p) { return p ? p + s0 : nullptr; };
-      auto offw = [&](double *p) { return p ? p + s0 : nullptr; };
-      j.q = off(whole.q); j.qd = off(whole.qd); j.x = off(whole.x); j.fext = off(whole.fext); j.x2 = off(whole.x2); j.tau_in = off(whole.tau_in);
-      j.body_acc = offw(whole.body_acc); j.joint_wrench = offw(whole.joint_wrench); j.tau_out = offw(whole.tau_out); j.qdd_out = offw(whole.qdd_out);
-      const size_t nv = (size_t)m->lanes[(size_t)i]->tree.nv;
-      const bool sm = (whole.flags & MECANO_B200_CRBA_STATE_MAJOR) != 0;
-      if (whole.algo == MB_CRBA)
-         j.out = whole.out ? (sm ? whole.out + (size_t)s0 * nv * nv : whole.out + s0) : nullptr;
-      else
-         j.out = offw(whole.out);
-      if (whole.algo == MB_STEP)
-         j.M = whole.M ? (sm ? whole.M + (size_t)s0 * nv * nv : whole.M + s0) : nullptr;
+      j.variant_n = n;
+      for (HostIn &in : j.in)
+         if (in.host) in.host += s0;
+      for (HostStep &st : j.steps)
+         for (HostOut &o : st.out)
+            if (o.host) o.host += o.how == COPY_STATES ? (size_t)s0 * o.rows : (size_t)s0;
    }
    int failed = 0;
-   const int rc = run_host_lanes(m->lanes, jobs, &failed);
+   rc = run_host_lanes(m->lanes, jobs, &failed);
    return multi_fail(m, rc, failed);
 }
 } // namespace
@@ -1590,35 +1509,26 @@ int mecano_b200_multi_set_gravity(mecano_b200_multi *m, double gx, double gy, do
 int mecano_b200_multi_rnea_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
                                 double *tau, uint32_t flags)
 {
-   HostJob j;
-   j.algo = MB_RNEA; j.n = n; j.ld = ld; j.q = q; j.qd = qd; j.x = qdd; j.fext = fext; j.out = tau; j.flags = flags;
-   return multi_run(m, j);
+   return multi_run(m, n, ld, [&](mecano_b200_handle *h, HostJob &j) { return rnea_job(h, n, ld, q, qd, qdd, fext, tau, nullptr, nullptr, flags, j); });
 }
 
 int mecano_b200_multi_aba_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
                                double *qdd, uint32_t flags)
 {
-   HostJob j;
-   j.algo = MB_ABA; j.n = n; j.ld = ld; j.q = q; j.qd = qd; j.x = tau; j.fext = fext; j.out = qdd; j.flags = flags;
-   return multi_run(m, j);
+   return multi_run(m, n, ld, [&](mecano_b200_handle *h, HostJob &j) { return aba_job(h, n, ld, q, qd, tau, nullptr, fext, qdd, nullptr, flags, j); });
 }
 
 int mecano_b200_multi_crba_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, double *M, uint32_t layout)
 {
-   HostJob j;
-   j.algo = MB_CRBA; j.n = n; j.ld = ld; j.q = q; j.out = M; j.flags = layout;
-   return multi_run(m, j);
+   return mecano_b200_multi_step_host(m, n, ld, q, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, M, layout);
 }
 
 int mecano_b200_multi_step_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd_in, const double *tau_in,
                                 const double *fext, double *tau_out, double *qdd_out, double *M, uint32_t layout)
 {
-   HostJob j;
-   j.algo = MB_STEP; j.n = n; j.ld = ld;
-   j.q = q; j.qd = qd; j.x = qdd_in; j.tau_in = tau_in; j.fext = fext;
-   j.out = tau_out; j.qdd_out = qdd_out; j.M = M;
-   j.flags = layout;
-   return multi_run(m, j);
+   return multi_run(m, n, ld, [&](mecano_b200_handle *h, HostJob &j) {
+      return step_job(h, n, ld, q, qd, qdd_in, tau_in, fext, tau_out, qdd_out, M, layout, j);
+   });
 }
 
 #pragma GCC visibility pop
