@@ -96,6 +96,7 @@ extern "C" {
 #define MECANO_B200_ALGO_ABA 1
 #define MECANO_B200_ALGO_CRBA 2
 #define MECANO_B200_ALGO_REGRESSOR 4 /* mecano_b200_kernel_info_get of mecano_b200_joint_torque_regressor (3: the Coriolis kernel) */
+#define MECANO_B200_ALGO_GRAVITY_GRADIENT 5 /* mecano_b200_kernel_info_get of mecano_b200_gravity_gradient */
 
 /* Column order of a body's ten inertial parameters in the joint-torque regressor (mecano_b200_joint_torque_regressor): the
  * column of the mass, the first of the three first moments m c (x, y, z) and the first of the six moments of inertia about the
@@ -311,6 +312,29 @@ int mecano_b200_joint_torque_regressor(mecano_b200_handle *h, int64_t n_states, 
                                        double *Y, void *stream);
 
 /*
+ * Gravity gradient (Mecano's MultiBodyGravityGradientCalculator): the joint efforts that gravity and the external wrenches cause,
+ * tau_g(q), and their configuration gradient G(q) = d tau_g / dq -- what gravity compensation with joint stiffness, the stability
+ * margin of a posture and the linearisation of the dynamics need.  For N states, with the handle's gravity:
+ *   tau       [n_dofs][ld]            the joint efforts of mecano_b200_rnea at the same q and fext with qd = 0 and qdd = 0
+ *   gradient  [n_dofs * n_dofs][ld]   entry (i, j) of G at [(i * n_dofs + j) * ld + s], entry-major like the mass matrix, every
+ *                                     entry written; the entries that couple joints of unrelated branches (the structural zeros of
+ *                                     the mass matrix) are 0.0.
+ * Entry (i, j) is d/d eps tau_i(q (+) eps e_j) at eps = 0, where q (+) eps e_j is what mecano_b200_integrate does to q with dt = eps,
+ * qd = e_j and qdd = 0: q + eps for a one-DoF joint; for SixDoF, spherical and planar joints a step along the body-frame velocity
+ * coordinate j, in frameAfterJoint.  The columns of a floating base are therefore perturbations in its own frame, the convention
+ * under which G is n_dofs x n_dofs.
+ * fext (nullable): the convention of mecano_b200_rnea (rows [6 w, 6 w + 6), w = wrench_index[b], in the body's CoM frame): the
+ * external wrenches are body-fixed and turn with their body.  With fext the wrench_index ranks must be below n_bodies
+ * (MECANO_B200_ERR_SHAPE otherwise).
+ * G is not symmetric in general; it is symmetric to round-off on trees of one-DoF joints without fext, where it is the Hessian of
+ * the potential energy.  The floating-base and external-wrench conventions of Mecano's own calculator are unpinned (its source is
+ * not at hand): the ones above are this project's definition.
+ * Always runs the generic thread-per-state kernel, in fp64 (a handle set to fp32 refuses with MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY).
+ */
+int mecano_b200_gravity_gradient(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *fext, double *tau,
+                                 double *gradient, void *stream);
+
+/*
  * Host-pointer entry points (what a JNI / Panama binding calls with DMatrixRMaj.data): inputs are
  * staged host -> device in chunks, the kernels run, results are copied back; the call returns when
  * the outputs are complete.  Pinned (page-locked) host memory makes the copies asynchronous and
@@ -371,6 +395,8 @@ int mecano_b200_coriolis_host(mecano_b200_handle *h, int64_t n_states, int64_t l
                               double *coriolis_matrix);
 int mecano_b200_joint_torque_regressor_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd,
                                             const double *qdd, double *Y);
+int mecano_b200_gravity_gradient_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *fext, double *tau,
+                                      double *gradient);
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, double *mass_matrix, double *cmm,
                                      double *com, int frame);
 int mecano_b200_centroidal_convective_term_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd,

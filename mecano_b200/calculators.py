@@ -4,6 +4,7 @@
     ForwardDynamicsCalculator                 M/algorithms/ForwardDynamicsCalculator.java:128-196, 313-319, 508-520, 556-567
     CompositeRigidBodyMassMatrixCalculator    M/algorithms/CompositeRigidBodyMassMatrixCalculator.java:182-233, 286-291, 344-348
     JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, see the class)
+    MultiBodyGravityGradientCalculator        gravity torques and their configuration gradient (project definition, see the class)
 
 Same names, argument meaning and error behaviour as the reference; the batching changes are that the joint state
 is passed explicitly as [rows, N] matrices (Mecano reads it from the joint objects) and that results come back as
@@ -618,6 +619,54 @@ class JointTorqueRegressorCalculator(_BatchedCalculator):
             for k, e in enumerate((0, 1, 2, 4, 5, 8)):
                 pi[10 * w + _capi.REGRESSOR_I + k] = d.inertia[9 * b + e]
         return pi
+
+
+class MultiBodyGravityGradientCalculator(_BatchedCalculator):
+    """Mecano's MultiBodyGravityGradientCalculator for N states: the joint efforts that gravity and the external wrenches cause,
+    tau_g(q), and their configuration gradient G(q) = d tau_g / dq (mecano_b200_gravity_gradient in include/mecano_b200.h: column j
+    is the derivative along the step the state integrator takes with qd = e_j, so a floating base's columns are perturbations in
+    its own frame; external wrenches are body-fixed).  G is not symmetric in general.
+
+    getTauMatrix() is [nDoFs, N]; getTauGradientMatrix() is [nDoFs * nDoFs, N], entry (i, j) of state s at [i * nDoFs + j, s].
+    Systems with fixed or ignored joints run on their welded tables (lumping does not change gravity torques), or, with external
+    wrenches, on the expanded tables (see _BatchedCalculator._expanded), of which the system's own rows and columns are returned.
+    One device only."""
+    _ALGO = _capi.ALGO_GRAVITY_GRADIENT
+
+    def __init__(self, input, device=0):
+        super().__init__(input, device)
+        self._tau = self._G = None
+
+    def compute(self, q):
+        """compute(q) for N states; returns getTauGradientMatrix() ([nDoFs * nDoFs, N])."""
+        if isinstance(self._device, (list, tuple)):
+            raise NotImplementedError("the gravity gradient runs on one device")
+        nv, nq = self._input.getNumberOfDoFs(), self._input.getConfigurationMatrixSize()
+        n = q.shape[1] if q.ndim == 2 else -1
+        self._check("q", q, nq, n)
+        if self._fext is not None:
+            self._check("externalWrenches", self._fext, 6 * self._input.getNumberOfJoints(), n)
+        if self._fext is not None and self._input.hasWeldedBodies():
+            eng, x = self._expanded()
+            q2 = self._extended(q, x.n_extra_cfg, x.q_extra)
+            nv2 = nv + x.n_extra_dof
+            tau2 = self._empty_like(q2, nv2, n, match_ld=False)
+            G2 = self._empty_like(q2, nv2 * nv2, n, match_ld=False)
+            eng.gravity_gradient(q2, tau2, G2, fext=self._extended(self._fext, 6 * x.n_extra_wrench_blocks))
+            # the held joints' DoFs follow the system's own in both the rows and the columns
+            self._tau = tau2[:nv]
+            self._G = G2.reshape(nv2, nv2, n)[:nv, :nv].reshape(nv * nv, n)
+            return self._G
+        self._tau = self._empty_like(q, nv, n)
+        self._G = self._empty_like(q, nv * nv, n)
+        self._engine.gravity_gradient(q, self._tau, self._G, fext=self._fext)
+        return self._G
+
+    def getTauMatrix(self):
+        return self._tau
+
+    def getTauGradientMatrix(self):
+        return self._G
 
 
 class MultiBodyDynamicsStep:

@@ -89,7 +89,7 @@ int slot_size(int algo, int jtype)
       case MB_RNEA: return 6 + jp;       // accumulated wrench + joint parameters
       case MB_ABA: return 6 + jp + nd;   // twist + joint parameters + joint velocity
       case MB_CORIOLIS: return 6 + jp;   // twist + joint parameters
-      default: return jp;                // CRBA, regressor: joint parameters only
+      default: return jp;                // CRBA, regressor, gravity gradient: joint parameters only
    }
 }
 
@@ -101,6 +101,7 @@ int aux_size(int algo)
       case MB_REGRESSOR: return 12; // twist + spatial acceleration of a branching body
       case MB_ABA: return 27;  // articulated inertia (6 + 9 + 6) + bias wrench (6); reused for (v, a) in pass three
       case MB_CORIOLIS: return 46; // composite inertia (10) + composite factorized inertia (4 x 9)
+      case MB_GRAVITY_GRADIENT: return 16; // composite inertia (10) + composite external wrench (6)
       default: return 10;      // composite inertia (6 + 3 + 1)
    }
 }
@@ -117,7 +118,7 @@ int slot2_size(int algo, int jtype, bool root_parent)
          return jtype == MB_SIXDOF ? (root_parent ? 3 : 9) : 4;
       case MB_CORIOLIS: // twist (3) + sin/cos (1); SixDoF: twist (3) + transform (6)
          return jtype == MB_SIXDOF ? 9 : 4;
-      default: // CRBA, regressor: sin/cos (1); SixDoF: transform (6)
+      default: // CRBA, regressor, gravity gradient: sin/cos (1); SixDoF: transform (6)
          return jtype == MB_SIXDOF ? 6 : 1;
    }
 }

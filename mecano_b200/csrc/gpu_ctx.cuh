@@ -300,11 +300,17 @@ template <int BLOCK, int TM, int ROWS, bool M3 = false> struct GpuCtx2
       if (!kMayClamp || active)
          mb_stg_cs(mb_row(mbase, (unsigned)e, mstride), v);
    }
-   char *corb; // Coriolis matrix (MB_CORIOLIS), entry-major
+   char *corb; // Coriolis matrix (MB_CORIOLIS), entry-major; joint efforts (MB_GRAVITY_GRADIENT)
    __device__ __forceinline__ void st_C(int e, double v) const
    {
       if (!kMayClamp || active)
          mb_stg_cs(mb_row(corb, (unsigned)e, ld8), v);
+   }
+   // gravity gradient (MB_GRAVITY_GRADIENT): the joint efforts tau_g, row r of `cor` (kernel_args.h); G goes through st_M
+   __device__ __forceinline__ void st_tau(int r, double v) const
+   {
+      if (!kMayClamp || active)
+         mb_stg(mb_row(corb, (unsigned)r, ld8), v);
    }
    __device__ __forceinline__ void zero_fill_mc_part(int k, int parts) const
    {

@@ -4,6 +4,7 @@
 //   ForwardDynamicsCalculator                 M/algorithms/ForwardDynamicsCalculator.java:128-196, 313-319, 508-520, 556-567
 //   CompositeRigidBodyMassMatrixCalculator    M/algorithms/CompositeRigidBodyMassMatrixCalculator.java:182-233, 286-291, 344-348
 //   JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, below)
+//   MultiBodyGravityGradientCalculator        gravity torques and their configuration gradient (project definition, below)
 //
 // Same names, argument meaning and error behaviour (exceptions) as the reference, with two batching changes:
 //   * compute(...) takes the joint state explicitly as nRows x N row-major matrices (what a Java
@@ -346,6 +347,31 @@ class JointTorqueRegressorCalculator : public BatchedCalculatorBase
             pi[10 * w + MECANO_B200_REGRESSOR_I + k] = tables_.inertia[9 * b + sym[k]];
       }
       return pi;
+   }
+};
+
+// MultiBodyGravityGradientCalculator: the joint efforts tau_g(q) that gravity and the external wrenches cause, and their configuration
+// gradient G = d tau_g / dq (mecano_b200_gravity_gradient: layout, floating-base and external-wrench conventions).  For systems
+// without welded bodies (fixed / ignored joints): with external wrenches the C ABI refuses their tables, whose wrench ranks count
+// the welded joints; the Python calculator runs them on the expanded tables.
+class MultiBodyGravityGradientCalculator : public BatchedCalculatorBase
+{
+ public:
+   explicit MultiBodyGravityGradientCalculator(const MultiBodySystem &input, int device = 0) : BatchedCalculatorBase(input, device) {}
+   // compute(q) + getTauMatrix() (nDoFs x N) + getTauGradientMatrix() ((nDoFs * nDoFs) x N, entry (i, j) at row i * nDoFs + j)
+   void compute(const MatrixView &q, const MatrixView &tauOut, const MatrixView &gradientOut, Memory where = Memory::Device)
+   {
+      const int64_t n = q.cols, nv = input_.getNumberOfDoFs(), nq = input_.getConfigurationMatrixSize();
+      checkShape(q, nq, n, "q");
+      checkShape(tauOut, nv, n, "tau");
+      checkShape(gradientOut, nv * nv, n, "tauGradient");
+      if (fext_.data) checkShape(fext_, 6 * (int64_t)tables_.parent.size(), n, "externalWrenches");
+      if (tauOut.ld != q.ld || gradientOut.ld != q.ld || (fext_.data && fext_.ld != q.ld))
+         throw MatrixDimensionException("all matrices of one call must share the same leading dimension");
+      if (where == Memory::Device)
+         check(mecano_b200_gravity_gradient(handle_, n, q.ld, q.data, fext_.data, tauOut.data, gradientOut.data, stream_));
+      else
+         check(mecano_b200_gravity_gradient_host(handle_, n, q.ld, q.data, fext_.data, tauOut.data, gradientOut.data));
    }
 };
 } // namespace mecano

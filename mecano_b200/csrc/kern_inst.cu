@@ -82,6 +82,11 @@ namespace mb
 #else
 #define MB_INST_14 MB_SKIP
 #endif
+#if MB_INST == 15
+#define MB_INST_15 MB_EMIT
+#else
+#define MB_INST_15 MB_SKIP
+#endif
 MB_KERNEL_GROUPS(MB_X)
 
 #if MB_INST == 13

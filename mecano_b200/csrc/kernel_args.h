@@ -18,6 +18,8 @@ struct KernelArgs
    double *cmm, *com;               // CRBA by-products (nullable): centroidal momentum matrix rows [r * nv + col], r = 0..5, in the root frame;
                                     // com rows 0..3 accumulate (mass * CoM, mass) over the root's children (zeroed before the launch)
    double *cor;                     // MB_CORIOLIS: the Coriolis matrix, entry-major like the mass matrix in `out`
+                                    // MB_GRAVITY_GRADIENT: the joint efforts tau_g [nv][ld]; `out` is then G, entry-major like the mass
+                                    // matrix, and zero_entries / n_zero are the mass matrix's (G has its structural zeros)
    double *root_wrench;             // RNEA by-product (nullable): rows 0..5 accumulate the wrench at the root in the root frame (zeroed before)
    int fp32;                        // optional fp32 variant (mecano_b200_set_precision): arithmetic in float, buffers stay fp64
    const double *consts;            // device copy of the per-body constant records

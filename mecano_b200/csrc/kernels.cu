@@ -40,6 +40,7 @@ KernelFn pick(int algo, bool fext, int layout, int cfg, bool m3)
                 : (fext ? pick_cfg<MB_ABA, true, 0, false>(cfg) : pick_cfg<MB_ABA, false, 0, false>(cfg));
    if (algo == MB_CORIOLIS) return pick_cfg<MB_CORIOLIS, false, 0, true>(cfg);
    if (algo == MB_REGRESSOR) return pick_cfg<MB_REGRESSOR, false, 0, true>(cfg);
+   if (algo == MB_GRAVITY_GRADIENT) return pick_cfg<MB_GRAVITY_GRADIENT, false, 0, true>(cfg); // (external wrenches: tested at run time)
    // CRBA: the "FEXT" instantiation is the one with by-products (centroidal momentum matrix, centre of mass), entry-major only
    if (fext && layout == 0) return pick_cfg<MB_CRBA, true, 0, true>(cfg);
    return layout == 1 ? pick_cfg<MB_CRBA, false, 1, true>(cfg) : (layout == 2 ? pick_cfg<MB_CRBA, false, 2, true>(cfg) : pick_cfg<MB_CRBA, false, 0, true>(cfg));
@@ -70,7 +71,7 @@ int forced_cfg(int algo)
 {
    const char *e = getenv("MECANO_B200_CFG");
    if (!e) return -1;
-   const char *key = algo == MB_RNEA ? "rnea=" : (algo == MB_ABA ? "aba=" : (algo == MB_CRBA ? "crba=" : (algo == MB_REGRESSOR ? "reg=" : "cor=")));
+   const char *key = algo == MB_RNEA ? "rnea=" : (algo == MB_ABA ? "aba=" : (algo == MB_CRBA ? "crba=" : (algo == MB_REGRESSOR ? "reg=" : (algo == MB_GRAVITY_GRADIENT ? "gg=" : "cor="))));
    const char *p = strstr(e, key);
    return p ? atoi(p + strlen(key)) : -1;
 }
@@ -144,8 +145,8 @@ cudaError_t plan_thread_kernel(int algo, const MbProgram &P, bool fext, LaunchPl
       // mass-matrix kernels, where more, smaller blocks win: hardware block scheduling evens out their store bursts (Coriolis,
       // H37: 2 x 128 threads 5.89 ms, 1 x 256 6.54 ms, profiles/r02h_cor_sweep.jsonl; CRBA, 4 x 128 against 2 x 256 threads:
       // 7 / 15 / 25 / 32 / 51 bodies -2.9 / -8.4 / -0.8 / -1.4 / -4.3 %, profiles/r03g_crba_block_sweep.jsonl); the
-      // regressor, store-bound the same way, follows them
-      const bool small_blocks = algo == MB_CORIOLIS || algo == MB_CRBA || algo == MB_REGRESSOR;
+      // regressor and the gravity gradient, store-bound the same way, follow them
+      const bool small_blocks = algo == MB_CORIOLIS || algo == MB_CRBA || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT;
       if (nblk > 0 && (score > best_threads || (small_blocks && score == best_threads && b < plan.block)))
       {
          best_threads = score;

@@ -227,6 +227,23 @@ class Engine:
             check(lib.mecano_b200_joint_torque_regressor(self._h, n, ld, pq, pqd, pqdd, py, self._stream()), self._h)
         return Y
 
+    def gravity_gradient(self, q, tau, G, fext=None):
+        """tau [nv, n], G [nv * nv, n] entry-major (mecano_b200_gravity_gradient), fext [6 * nb, n] or None; torch CUDA tensors or
+        numpy arrays (host path)."""
+        n = q.shape[1]
+        host = isinstance(q, np.ndarray)
+        f = _host_ptr_ld if host else self._dp
+        pq, l0 = f(q, self.nq, n)
+        pf, l1 = f(fext, 6 * self.nb, n)
+        pt, l2 = f(tau, self.nv, n)
+        pg, l3 = f(G, self.nv * self.nv, n)
+        ld = _same_ld([l0, l1, l2, l3])
+        if host:
+            check(lib.mecano_b200_gravity_gradient_host(self._h, n, ld, pq, pf, pt, pg), self._h)
+        else:
+            check(lib.mecano_b200_gravity_gradient(self._h, n, ld, pq, pf, pt, pg, self._stream()), self._h)
+        return G
+
     def crba_centroidal(self, q, M, cmm, com, frame=_capi.FRAME_WORLD):
         """M [nv*nv, n] entry-major, cmm [6*nv, n], com [4, n]; torch CUDA tensors or numpy arrays (host path)."""
         n = q.shape[1]
@@ -483,7 +500,7 @@ class MultiDeviceEngine:
         raise NotImplementedError("this entry point is served per device: build the calculator on one device")
 
     aba_sources_host = coriolis = crba_centroidal = centroidal_convective_term = center_of_mass = integrate_host = set_joint_source_modes = _single_device_only
-    joint_torque_regressor = _single_device_only
+    joint_torque_regressor = gravity_gradient = _single_device_only
 
 
 def measure_fp64_peak(device=0):
