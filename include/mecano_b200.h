@@ -97,6 +97,7 @@ extern "C" {
 #define MECANO_B200_ALGO_CRBA 2
 #define MECANO_B200_ALGO_REGRESSOR 4 /* mecano_b200_kernel_info_get of mecano_b200_joint_torque_regressor (3: the Coriolis kernel) */
 #define MECANO_B200_ALGO_GRAVITY_GRADIENT 5 /* mecano_b200_kernel_info_get of mecano_b200_gravity_gradient */
+#define MECANO_B200_ALGO_RNEA_DERIVATIVES 6 /* mecano_b200_kernel_info_get of mecano_b200_rnea_derivatives */
 
 /* Column order of a body's ten inertial parameters in the joint-torque regressor (mecano_b200_joint_torque_regressor): the
  * column of the mass, the first of the three first moments m c (x, y, z) and the first of the six moments of inertia about the
@@ -335,6 +336,28 @@ int mecano_b200_gravity_gradient(mecano_b200_handle *h, int64_t n_states, int64_
                                  double *gradient, void *stream);
 
 /*
+ * Inverse-dynamics derivatives: the joint efforts tau(q, qd, qdd) of RNEA and their first-order partials d tau / dq and d tau / dqd
+ * at a general state -- what MPC, iLQR / DDP and trajectory optimisation linearise along a trajectory.  The third partial,
+ * d tau / dqdd, is the mass matrix (mecano_b200_crba); the forward-dynamics partials follow as dqdd / dx = -M^-1 d tau / dx.
+ * For N states, with the handle's gravity:
+ *   tau       [n_dofs][ld]            the joint efforts of mecano_b200_rnea on the same q, qd, qdd and fext, with no flags
+ *   dtau_dq   [n_dofs * n_dofs][ld]   entry (i, j) at [(i * n_dofs + j) * ld + s], entry-major like the mass matrix
+ *   dtau_dqd  [n_dofs * n_dofs][ld]   the same layout
+ * Every entry of both matrices is written; the entries that couple joints of unrelated branches (the structural zeros of the mass
+ * matrix) are 0.0.  Column j of dtau_dq follows the convention of mecano_b200_gravity_gradient: the derivative along the step
+ * mecano_b200_integrate takes with dt = eps, qd = e_j and qdd = 0, so a floating base's columns are perturbations in its own frame;
+ * qd and qdd are held.  Column j of dtau_dqd is d tau / d qd_j with q and qdd held.
+ * fext (nullable): the convention of mecano_b200_rnea (rows [6 w, 6 w + 6), w = wrench_index[b], in the body's CoM frame): the
+ * external wrenches are body-fixed and turn with their body.  With fext the wrench_index ranks must be below n_bodies
+ * (MECANO_B200_ERR_SHAPE otherwise).
+ * At qd = qdd = 0, dtau_dq is the gradient of mecano_b200_gravity_gradient (to round-off) and dtau_dqd is zero.  Mecano has no
+ * counterpart of this call: the definition above is this project's.
+ * Always runs the generic thread-per-state kernel, in fp64 (a handle set to fp32 refuses with MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY).
+ */
+int mecano_b200_rnea_derivatives(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd, const double *qdd,
+                                 const double *fext, double *tau, double *dtau_dq, double *dtau_dqd, void *stream);
+
+/*
  * Host-pointer entry points (what a JNI / Panama binding calls with DMatrixRMaj.data): inputs are
  * staged host -> device in chunks, the kernels run, results are copied back; the call returns when
  * the outputs are complete.  Pinned (page-locked) host memory makes the copies asynchronous and
@@ -397,6 +420,8 @@ int mecano_b200_joint_torque_regressor_host(mecano_b200_handle *h, int64_t n_sta
                                             const double *qdd, double *Y);
 int mecano_b200_gravity_gradient_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *fext, double *tau,
                                       double *gradient);
+int mecano_b200_rnea_derivatives_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd, const double *qdd,
+                                      const double *fext, double *tau, double *dtau_dq, double *dtau_dqd);
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, double *mass_matrix, double *cmm,
                                      double *com, int frame);
 int mecano_b200_centroidal_convective_term_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd,

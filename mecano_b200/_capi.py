@@ -30,6 +30,7 @@ CRBA_PACKED = 4  # one row per unique, structurally non-zero entry (mecano_b200_
 ALGO_RNEA, ALGO_ABA, ALGO_CRBA = 0, 1, 2
 ALGO_REGRESSOR = 4
 ALGO_GRAVITY_GRADIENT = 5
+ALGO_RNEA_DERIVATIVES = 6
 # column order of a body's ten inertial parameters in the joint-torque regressor (MECANO_B200_REGRESSOR_*): mass, first of the
 # first moments m c (x y z), first of the moments of inertia about the origin (xx xy xz yy yz zz)
 REGRESSOR_M, REGRESSOR_MC, REGRESSOR_I = 0, 1, 4
@@ -77,6 +78,7 @@ EXPORTS = [
     "mecano_b200_multi_crba_host", "mecano_b200_multi_step_host",
     "mecano_b200_joint_torque_regressor", "mecano_b200_joint_torque_regressor_host",
     "mecano_b200_gravity_gradient", "mecano_b200_gravity_gradient_host",
+    "mecano_b200_rnea_derivatives", "mecano_b200_rnea_derivatives_host",
 ]
 
 lib.mecano_b200_create.argtypes = [ctypes.POINTER(TreeDesc), ctypes.c_int, ctypes.POINTER(c_vp)]
@@ -111,6 +113,8 @@ lib.mecano_b200_joint_torque_regressor.argtypes = [c_vp, c_i64, c_i64, c_vp, c_v
 lib.mecano_b200_joint_torque_regressor_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp]
 lib.mecano_b200_gravity_gradient.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp]
 lib.mecano_b200_gravity_gradient_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp]
+lib.mecano_b200_rnea_derivatives.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
+lib.mecano_b200_rnea_derivatives_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
 lib.mecano_b200_crba.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_u32, c_vp]
 lib.mecano_b200_rnea_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_u32]
 lib.mecano_b200_aba_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_u32]

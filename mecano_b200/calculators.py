@@ -5,6 +5,7 @@
     CompositeRigidBodyMassMatrixCalculator    M/algorithms/CompositeRigidBodyMassMatrixCalculator.java:182-233, 286-291, 344-348
     JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, see the class)
     MultiBodyGravityGradientCalculator        gravity torques and their configuration gradient (project definition, see the class)
+    InverseDynamicsDerivativesCalculator      d tau / dq and d tau / dqd of inverse dynamics (project definition, see the class)
 
 Same names, argument meaning and error behaviour as the reference; the batching changes are that the joint state
 is passed explicitly as [rows, N] matrices (Mecano reads it from the joint objects) and that results come back as
@@ -667,6 +668,64 @@ class MultiBodyGravityGradientCalculator(_BatchedCalculator):
 
     def getTauGradientMatrix(self):
         return self._G
+
+
+class InverseDynamicsDerivativesCalculator(_BatchedCalculator):
+    """The first-order partials of inverse dynamics for N states: tau(q, qd, qdd) of InverseDynamicsCalculator together with
+    d tau / dq and d tau / dqd (mecano_b200_rnea_derivatives in include/mecano_b200.h: column j of d tau / dq is the derivative along
+    the step the state integrator takes with qd = e_j, so a floating base's columns are perturbations in its own frame; external
+    wrenches are body-fixed).  d tau / dqdd is the mass matrix (CompositeRigidBodyMassMatrixCalculator).  Mecano has no counterpart:
+    the definition is this project's, the one of MultiBodyGravityGradientCalculator extended to a moving state.
+
+    getJointTauMatrix() is [nDoFs, N]; getTauConfigurationGradientMatrix() and getTauVelocityGradientMatrix() are [nDoFs * nDoFs, N],
+    entry (i, j) of state s at [i * nDoFs + j, s].  Systems with fixed or ignored joints run on their welded tables, or, with external
+    wrenches, on the expanded tables (see _BatchedCalculator._expanded), of which the system's own rows and columns are returned.
+    One device only."""
+    _ALGO = _capi.ALGO_RNEA_DERIVATIVES
+
+    def __init__(self, input, device=0):
+        super().__init__(input, device)
+        self._tau = self._dq = self._dqd = None
+
+    def compute(self, q, qd, qdd):
+        """compute(q, qd, qdd) for N states; returns getTauConfigurationGradientMatrix() ([nDoFs * nDoFs, N])."""
+        if isinstance(self._device, (list, tuple)):
+            raise NotImplementedError("the inverse-dynamics derivatives run on one device")
+        nv, nq = self._input.getNumberOfDoFs(), self._input.getConfigurationMatrixSize()
+        n = q.shape[1] if q.ndim == 2 else -1
+        self._check("q", q, nq, n)
+        self._check("qd", qd, nv, n)
+        self._check("qdd", qdd, nv, n)
+        if self._fext is not None:
+            self._check("externalWrenches", self._fext, 6 * self._input.getNumberOfJoints(), n)
+        if self._fext is not None and self._input.hasWeldedBodies():
+            eng, x = self._expanded()
+            q2 = self._extended(q, x.n_extra_cfg, x.q_extra)
+            qd2, qdd2 = self._extended(qd, x.n_extra_dof), self._extended(qdd, x.n_extra_dof)
+            nv2 = nv + x.n_extra_dof
+            tau2 = self._empty_like(q2, nv2, n, match_ld=False)
+            dq2 = self._empty_like(q2, nv2 * nv2, n, match_ld=False)
+            dqd2 = self._empty_like(q2, nv2 * nv2, n, match_ld=False)
+            eng.rnea_derivatives(q2, qd2, qdd2, tau2, dq2, dqd2, fext=self._extended(self._fext, 6 * x.n_extra_wrench_blocks))
+            # the held joints' DoFs follow the system's own in both the rows and the columns
+            self._tau = tau2[:nv]
+            self._dq = dq2.reshape(nv2, nv2, n)[:nv, :nv].reshape(nv * nv, n)
+            self._dqd = dqd2.reshape(nv2, nv2, n)[:nv, :nv].reshape(nv * nv, n)
+            return self._dq
+        self._tau = self._empty_like(q, nv, n)
+        self._dq = self._empty_like(q, nv * nv, n)
+        self._dqd = self._empty_like(q, nv * nv, n)
+        self._engine.rnea_derivatives(q, qd, qdd, self._tau, self._dq, self._dqd, fext=self._fext)
+        return self._dq
+
+    def getJointTauMatrix(self):
+        return self._tau
+
+    def getTauConfigurationGradientMatrix(self):
+        return self._dq
+
+    def getTauVelocityGradientMatrix(self):
+        return self._dqd
 
 
 class MultiBodyDynamicsStep:

@@ -45,14 +45,14 @@ struct mecano_b200_handle
    double gravity[3] = {0.0, 0.0, 0.0}; // Mecano calculators start with zero gravity until setGravitationalAcceleration
    mb::LaunchPlan plan[MB_NUM_ALGOS];
    bool fp32 = false; // mecano_b200_set_precision
-   int grid_limit[MB_NUM_ALGOS] = {0, 0, 0, 0, 0, 0}; // mecano_b200_set_grid_limit: cap on the persistent grids (0 = whole device)
+   int grid_limit[MB_NUM_ALGOS] = {0, 0, 0, 0, 0, 0, 0}; // mecano_b200_set_grid_limit: cap on the persistent grids (0 = whole device)
    int variant = MECANO_B200_VARIANT_AUTO;
    int max_children = 1, max_ndof = 1, sm_count = 148;
    int n_accel_source = 0;           // joints in ACCELERATION_SOURCE mode (mecano_b200_set_joint_source_modes)
    std::vector<std::pair<int, int>> effort_dof_runs; // (first DoF row, count) runs of DoF rows whose joints are EFFORT_SOURCE
    bool warp_ok = false;             // the body-parallel variant serves this tree (one-DoF / SixDoF joints; <= 32 bodies: a warp per state, else a team of warps)
    bool has_3dof = false;            // the tree has spherical / planar joints (generic thread-per-state kernels only)
-   int64_t warp_below[MB_NUM_ALGOS] = {0, 0, 0, 0, 0, 0}; // AUTO: batches smaller than this run warp-per-state
+   int64_t warp_below[MB_NUM_ALGOS] = {0, 0, 0, 0, 0, 0, 0}; // AUTO: batches smaller than this run warp-per-state
    std::string error;
    // host pipeline (lazy)
    cudaStream_t streams[MB_MAX_SLOTS] = {};
@@ -162,7 +162,7 @@ int run(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q,
    // states on; a thread per state needs tens of thousands but then has 10-30x the throughput)
    // calls with by-product buffers (mecano_b200_rnea_full) always run the generic thread-per-state kernel
    // (so does the packed mass-matrix layout: its row numbering follows the thread-per-state traversal)
-   const bool byprod = body_acc || joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || h->fp32 || packed;
+   const bool byprod = body_acc || joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES || h->fp32 || packed;
    const int64_t vn = opt.variant_n > 0 ? opt.variant_n : n;
    const bool use_warp = !byprod && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && vn < h->warp_below[algo]));
    if (use_warp)
@@ -773,7 +773,7 @@ int mecano_b200_create(const mecano_b200_tree_desc *desc, int device, mecano_b20
    {
       bool fits = false;
       if ((e = mb::plan_thread_kernel(algo, h->tree.prog[algo], false, h->plan[algo], &fits)) != cudaSuccess) return bail(e, "kernel planning");
-      if (!fits && (algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT))
+      if (!fits && (algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES))
       {
          h->plan[algo].block = 0; // a by-product kernel alone does not fit: its entry point reports it, everything else works
          continue;
@@ -1175,6 +1175,56 @@ int mecano_b200_gravity_gradient_host(mecano_b200_handle *h, int64_t n, int64_t 
    return run_host(h, j);
 }
 
+// the refusals of the inverse-dynamics derivatives, shared by their two entry points
+int rnea_derivatives_check(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
+                           const double *tau, const double *dq, const double *dqd)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc) return rc;
+   if (h->fp32)
+      return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the inverse-dynamics derivatives are computed in fp64 only (mecano_b200_set_precision)");
+   if (h->plan[MB_RNEA_DERIVATIVES].block == 0)
+      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the inverse-dynamics derivatives kernel (branch nesting / depth too large)");
+   if (n > 0 && (!q || !qd || !qdd || !tau || !dq || !dqd))
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (fext)
+   {
+      const MbProgram &P = h->tree.prog[MB_RNEA_DERIVATIVES];
+      for (int i = 0; i < P.nb; i++)
+         if (P.body[i].ext_index >= P.nb)
+            return fail(h, MECANO_B200_ERR_SHAPE, "inverse-dynamics derivatives: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
+   }
+   return MECANO_B200_OK;
+}
+
+int mecano_b200_rnea_derivatives(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
+                                 double *tau, double *dq, double *dqd, void *stream)
+{
+   const int rc = rnea_derivatives_check(h, n, ld, q, qd, qdd, fext, tau, dq, dqd);
+   if (rc || n == 0) return rc;
+   MB_ON_DEVICE(h);
+   RunOpts opt;
+   opt.cor = dqd;          // (kernel_args.h: d tau / dq travels in `out`, d tau / dqd in `cor`,
+   opt.root_wrench = tau;  //  the joint efforts in `root_wrench`)
+   return run(h, MB_RNEA_DERIVATIVES, n, ld, q, qd, qdd, fext, dq, 0u, (cudaStream_t)stream, opt);
+}
+
+int mecano_b200_rnea_derivatives_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd,
+                                      const double *fext, double *tau, double *dq, double *dqd)
+{
+   const int rc = rnea_derivatives_check(h, n, ld, q, qd, qdd, fext, tau, dq, dqd);
+   if (rc || n == 0) return rc;
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   HostJob j{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}, {fext, 6 * (size_t)h->tree.nb}}};
+   j.steps.push_back({[](const Chunk &c) {
+      RunOpts opt = c.opt;
+      opt.root_wrench = c.out[0];
+      opt.cor = c.out[2];
+      return run(c.h, MB_RNEA_DERIVATIVES, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[1], 0u, c.stream, opt);
+   }, {{tau, nv}, {dq, nv * nv}, {dqd, nv * nv}}});
+   return run_host(h, j);
+}
+
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame)
 {
    int rc = check_batch(h, n, ld);
@@ -1305,7 +1355,7 @@ int mecano_b200_step_host(mecano_b200_handle *h, int64_t n, int64_t ld, const do
 int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_states, mecano_b200_kernel_info *info)
 {
    if (!h || !info || algo < 0 || algo >= MB_NUM_ALGOS) return MECANO_B200_ERR_INVALID_ARGUMENT;
-   const bool warp = algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && n_states > 0 && n_states < h->warp_below[algo]));
+   const bool warp = algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && algo != MB_RNEA_DERIVATIVES && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && n_states > 0 && n_states < h->warp_below[algo]));
    if (warp)
    {
       std::memset(info, 0, sizeof *info);
@@ -1358,11 +1408,13 @@ int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_state
    info->stack_doubles = P.stack_doubles;
    info->max_depth = P.max_depth;
    const double nq = P.nq, nv = P.nv;
-   // (the gravity gradient: q in, tau and G out; a call with external wrenches reads 48 n_bodies bytes more)
+   // (the gravity gradient: q in, tau and G out; the inverse-dynamics derivatives: q, qd, qdd in, tau and two matrices out; a call with
+   // external wrenches reads 48 n_bodies bytes more)
    info->bytes_per_state = algo == MB_CRBA ? 8.0 * (nq + nv * nv)
+                           : (algo == MB_RNEA_DERIVATIVES ? 8.0 * (nq + 3.0 * nv + 2.0 * nv * nv)
                            : (algo == MB_GRAVITY_GRADIENT ? 8.0 * (nq + nv + nv * nv)
                            : (algo == MB_CORIOLIS ? 8.0 * (nq + nv + 2.0 * nv * nv)
-                                                  : (algo == MB_REGRESSOR ? 8.0 * (nq + 2.0 * nv + 10.0 * P.nb * nv) : 8.0 * (nq + 3.0 * nv)))); // SURVEY.md 8(d)
+                                                  : (algo == MB_REGRESSOR ? 8.0 * (nq + 2.0 * nv + 10.0 * P.nb * nv) : 8.0 * (nq + 3.0 * nv))))); // SURVEY.md 8(d)
    return MECANO_B200_OK;
 }
 

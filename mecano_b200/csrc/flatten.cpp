@@ -102,6 +102,7 @@ int aux_size(int algo)
       case MB_ABA: return 27;  // articulated inertia (6 + 9 + 6) + bias wrench (6); reused for (v, a) in pass three
       case MB_CORIOLIS: return 46; // composite inertia (10) + composite factorized inertia (4 x 9)
       case MB_GRAVITY_GRADIENT: return 16; // composite inertia (10) + composite external wrench (6)
+      case MB_RNEA_DERIVATIVES: return 58; // composite inertia (10), factorized inertia (4 x 9), momentum (6), RNEA force (6)
       default: return 10;      // composite inertia (6 + 3 + 1)
    }
 }
@@ -118,6 +119,9 @@ int slot2_size(int algo, int jtype, bool root_parent)
          return jtype == MB_SIXDOF ? (root_parent ? 3 : 9) : 4;
       case MB_CORIOLIS: // twist (3) + sin/cos (1); SixDoF: twist (3) + transform (6)
          return jtype == MB_SIXDOF ? 9 : 4;
+      case MB_RNEA_DERIVATIVES: // twist (3) + sin/cos (1); SixDoF: twist, the parent's twist and acceleration (9) + transform (6) unless
+                                // attached to the root body (the body's acceleration: a per-depth area behind the branch save area)
+         return jtype == MB_SIXDOF ? (root_parent ? 9 : 15) : 4;
       default: // CRBA, regressor, gravity gradient: sin/cos (1); SixDoF: transform (6)
          return jtype == MB_SIXDOF ? 6 : 1;
    }
@@ -572,6 +576,8 @@ int flatten_tree(const mecano_b200_tree_desc *d, FlatTree &out, std::string &err
          }
       }
       P.rec_doubles = algo == MB_ABA ? MB_ABA_REC * (nb + rec_extra) : 0;
+      if (algo == MB_RNEA_DERIVATIVES)
+         P.aux_doubles += 6 * (P.max_depth + 1); // the spatial acceleration of the open body at each depth (rnea_derivatives.cuh)
 
       // ops: iterative DFS emitting DESCEND on entry and ASCEND on exit
       int nops = 0;

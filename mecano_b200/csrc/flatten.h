@@ -27,7 +27,7 @@ struct FlatTree
    // joint-torque regressor (MB_REGRESSOR): the structurally zero rows of each body's block, as the entry of the row's first
    // column (row * 10 nb + 10 w); a row's ten columns are zero together.  Empty if a wrench_index rank is >= nb.
    std::vector<uint32_t> regressor_zero_rows;
-   MbProgram prog[MB_NUM_ALGOS];    // MB_RNEA, MB_ABA, MB_CRBA, MB_CORIOLIS, MB_REGRESSOR, MB_GRAVITY_GRADIENT
+   MbProgram prog[MB_NUM_ALGOS];    // MB_RNEA, MB_ABA, MB_CRBA, MB_CORIOLIS, MB_REGRESSOR, MB_GRAVITY_GRADIENT, MB_RNEA_DERIVATIVES
 };
 
 // Returns MECANO_B200_OK or a negative error code; `err` receives the message.

@@ -300,7 +300,7 @@ template <int BLOCK, int TM, int ROWS, bool M3 = false> struct GpuCtx2
       if (!kMayClamp || active)
          mb_stg_cs(mb_row(mbase, (unsigned)e, mstride), v);
    }
-   char *corb; // Coriolis matrix (MB_CORIOLIS), entry-major; joint efforts (MB_GRAVITY_GRADIENT)
+   char *corb; // Coriolis matrix (MB_CORIOLIS), entry-major; joint efforts (MB_GRAVITY_GRADIENT); d tau / dqd (MB_RNEA_DERIVATIVES)
    __device__ __forceinline__ void st_C(int e, double v) const
    {
       if (!kMayClamp || active)
@@ -311,6 +311,13 @@ template <int BLOCK, int TM, int ROWS, bool M3 = false> struct GpuCtx2
    {
       if (!kMayClamp || active)
          mb_stg(mb_row(corb, (unsigned)r, ld8), v);
+   }
+   // inverse-dynamics derivatives (MB_RNEA_DERIVATIVES): the joint efforts tau, row r of `root_wrench` (kernel_args.h); d tau / dq goes
+   // through st_M, d tau / dqd through st_C
+   __device__ __forceinline__ void st_jtau(int r, double v) const
+   {
+      if (!kMayClamp || active)
+         mb_stg(mb_row(rwb, (unsigned)r, ld8), v);
    }
    __device__ __forceinline__ void zero_fill_mc_part(int k, int parts) const
    {

@@ -5,6 +5,7 @@
 //   CompositeRigidBodyMassMatrixCalculator    M/algorithms/CompositeRigidBodyMassMatrixCalculator.java:182-233, 286-291, 344-348
 //   JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, below)
 //   MultiBodyGravityGradientCalculator        gravity torques and their configuration gradient (project definition, below)
+//   InverseDynamicsDerivativesCalculator      d tau / dq and d tau / dqd of inverse dynamics (project definition, below)
 //
 // Same names, argument meaning and error behaviour (exceptions) as the reference, with two batching changes:
 //   * compute(...) takes the joint state explicitly as nRows x N row-major matrices (what a Java
@@ -372,6 +373,35 @@ class MultiBodyGravityGradientCalculator : public BatchedCalculatorBase
          check(mecano_b200_gravity_gradient(handle_, n, q.ld, q.data, fext_.data, tauOut.data, gradientOut.data, stream_));
       else
          check(mecano_b200_gravity_gradient_host(handle_, n, q.ld, q.data, fext_.data, tauOut.data, gradientOut.data));
+   }
+};
+
+// InverseDynamicsDerivativesCalculator: the joint efforts tau(q, qd, qdd) and their partials d tau / dq, d tau / dqd
+// (mecano_b200_rnea_derivatives: layout, floating-base and external-wrench conventions).  For systems without welded bodies (fixed /
+// ignored joints) with external wrenches, as MultiBodyGravityGradientCalculator.
+class InverseDynamicsDerivativesCalculator : public BatchedCalculatorBase
+{
+ public:
+   explicit InverseDynamicsDerivativesCalculator(const MultiBodySystem &input, int device = 0) : BatchedCalculatorBase(input, device) {}
+   // compute(q, qd, qdd) + getJointTauMatrix() (nDoFs x N) + getTauConfigurationGradientMatrix() / getTauVelocityGradientMatrix()
+   // ((nDoFs * nDoFs) x N each, entry (i, j) at row i * nDoFs + j)
+   void compute(const MatrixView &q, const MatrixView &qd, const MatrixView &qdd, const MatrixView &tauOut, const MatrixView &dqOut,
+                const MatrixView &dqdOut, Memory where = Memory::Device)
+   {
+      const int64_t n = q.cols, nv = input_.getNumberOfDoFs(), nq = input_.getConfigurationMatrixSize();
+      checkShape(q, nq, n, "q");
+      checkShape(qd, nv, n, "qd");
+      checkShape(qdd, nv, n, "qdd");
+      checkShape(tauOut, nv, n, "tau");
+      checkShape(dqOut, nv * nv, n, "tauConfigurationGradient");
+      checkShape(dqdOut, nv * nv, n, "tauVelocityGradient");
+      if (fext_.data) checkShape(fext_, 6 * (int64_t)tables_.parent.size(), n, "externalWrenches");
+      if (qd.ld != q.ld || qdd.ld != q.ld || tauOut.ld != q.ld || dqOut.ld != q.ld || dqdOut.ld != q.ld || (fext_.data && fext_.ld != q.ld))
+         throw MatrixDimensionException("all matrices of one call must share the same leading dimension");
+      if (where == Memory::Device)
+         check(mecano_b200_rnea_derivatives(handle_, n, q.ld, q.data, qd.data, qdd.data, fext_.data, tauOut.data, dqOut.data, dqdOut.data, stream_));
+      else
+         check(mecano_b200_rnea_derivatives_host(handle_, n, q.ld, q.data, qd.data, qdd.data, fext_.data, tauOut.data, dqOut.data, dqdOut.data));
    }
 };
 } // namespace mecano

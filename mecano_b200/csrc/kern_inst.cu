@@ -87,6 +87,11 @@ namespace mb
 #else
 #define MB_INST_15 MB_SKIP
 #endif
+#if MB_INST == 16
+#define MB_INST_16 MB_EMIT
+#else
+#define MB_INST_16 MB_SKIP
+#endif
 MB_KERNEL_GROUPS(MB_X)
 
 #if MB_INST == 13

@@ -20,7 +20,10 @@ struct KernelArgs
    double *cor;                     // MB_CORIOLIS: the Coriolis matrix, entry-major like the mass matrix in `out`
                                     // MB_GRAVITY_GRADIENT: the joint efforts tau_g [nv][ld]; `out` is then G, entry-major like the mass
                                     // matrix, and zero_entries / n_zero are the mass matrix's (G has its structural zeros)
+                                    // MB_RNEA_DERIVATIVES: d tau / dqd, entry-major; `out` is then d tau / dq, zero_entries / n_zero the
+                                    // mass matrix's (both matrices have its structural zeros) and `root_wrench` the joint efforts
    double *root_wrench;             // RNEA by-product (nullable): rows 0..5 accumulate the wrench at the root in the root frame (zeroed before)
+                                    // MB_RNEA_DERIVATIVES: the joint efforts tau [nv][ld]
    int fp32;                        // optional fp32 variant (mecano_b200_set_precision): arithmetic in float, buffers stay fp64
    const double *consts;            // device copy of the per-body constant records
    double *ws;                      // ABA: pass-two records [rec][ws_ld], one column per resident thread of the persistent grid

@@ -41,6 +41,7 @@ KernelFn pick(int algo, bool fext, int layout, int cfg, bool m3)
    if (algo == MB_CORIOLIS) return pick_cfg<MB_CORIOLIS, false, 0, true>(cfg);
    if (algo == MB_REGRESSOR) return pick_cfg<MB_REGRESSOR, false, 0, true>(cfg);
    if (algo == MB_GRAVITY_GRADIENT) return pick_cfg<MB_GRAVITY_GRADIENT, false, 0, true>(cfg); // (external wrenches: tested at run time)
+   if (algo == MB_RNEA_DERIVATIVES) return pick_cfg<MB_RNEA_DERIVATIVES, false, 0, true>(cfg); // (likewise)
    // CRBA: the "FEXT" instantiation is the one with by-products (centroidal momentum matrix, centre of mass), entry-major only
    if (fext && layout == 0) return pick_cfg<MB_CRBA, true, 0, true>(cfg);
    return layout == 1 ? pick_cfg<MB_CRBA, false, 1, true>(cfg) : (layout == 2 ? pick_cfg<MB_CRBA, false, 2, true>(cfg) : pick_cfg<MB_CRBA, false, 0, true>(cfg));
@@ -71,7 +72,7 @@ int forced_cfg(int algo)
 {
    const char *e = getenv("MECANO_B200_CFG");
    if (!e) return -1;
-   const char *key = algo == MB_RNEA ? "rnea=" : (algo == MB_ABA ? "aba=" : (algo == MB_CRBA ? "crba=" : (algo == MB_REGRESSOR ? "reg=" : (algo == MB_GRAVITY_GRADIENT ? "gg=" : "cor="))));
+   const char *key = algo == MB_RNEA ? "rnea=" : (algo == MB_ABA ? "aba=" : (algo == MB_CRBA ? "crba=" : (algo == MB_REGRESSOR ? "reg=" : (algo == MB_GRAVITY_GRADIENT ? "gg=" : (algo == MB_RNEA_DERIVATIVES ? "rd=" : "cor=")))));
    const char *p = strstr(e, key);
    return p ? atoi(p + strlen(key)) : -1;
 }
@@ -135,8 +136,9 @@ cudaError_t plan_thread_kernel(int algo, const MbProgram &P, bool fext, LaunchPl
       // work area only competes if nothing else fits
       const int auxn = aux_of(algo, kCfg[cfg].cls);
       // (the Coriolis kernel keeps two 46-double accumulators and three force columns live: a few hundred bytes of spills are its
-      // normal state at 255 registers)
-      const bool spills = (long)fa.localSizeBytes > 8l * auxn + (algo == MB_CORIOLIS ? 512 : 128);
+      // normal state at 255 registers; so are some 670 bytes for the inverse-dynamics derivatives, four accumulators of 58 doubles
+      // and four force columns)
+      const bool spills = (long)fa.localSizeBytes > 8l * auxn + (algo == MB_CORIOLIS ? 512 : (algo == MB_RNEA_DERIVATIVES ? 768 : 128));
       // warps that do not split evenly over the four sub-partitions lose more than they bring (ABA 320 threads: 3.44 ms,
       // 256 threads: 2.23 ms; profiles/r01i_cfg_sweep.jsonl): such block sizes only compete if nothing else fits
       const bool uneven = ((nblk * b) % 128) != 0 && nblk * b > 128;
@@ -145,8 +147,8 @@ cudaError_t plan_thread_kernel(int algo, const MbProgram &P, bool fext, LaunchPl
       // mass-matrix kernels, where more, smaller blocks win: hardware block scheduling evens out their store bursts (Coriolis,
       // H37: 2 x 128 threads 5.89 ms, 1 x 256 6.54 ms, profiles/r02h_cor_sweep.jsonl; CRBA, 4 x 128 against 2 x 256 threads:
       // 7 / 15 / 25 / 32 / 51 bodies -2.9 / -8.4 / -0.8 / -1.4 / -4.3 %, profiles/r03g_crba_block_sweep.jsonl); the
-      // regressor and the gravity gradient, store-bound the same way, follow them
-      const bool small_blocks = algo == MB_CORIOLIS || algo == MB_CRBA || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT;
+      // regressor, the gravity gradient and the inverse-dynamics derivatives, store-bound the same way, follow them
+      const bool small_blocks = algo == MB_CORIOLIS || algo == MB_CRBA || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES;
       if (nblk > 0 && (score > best_threads || (small_blocks && score == best_threads && b < plan.block)))
       {
          best_threads = score;

@@ -244,9 +244,10 @@ static inline int mb_sub_ndof(int sub) { return sub == MB_SUB_SIX ? 6 : 3; }
 #define MB_ABA_RING_ROWS (1 + MB_ABA_REC / 2) // pass-three ring, double2 rows per stage: (-, qd) + the record
 
 // MB_CORIOLIS: mass matrix + Coriolis matrix (coriolis.cuh); MB_REGRESSOR: joint-torque regressor (regressor.cuh);
-// MB_GRAVITY_GRADIENT: gravity torques and their configuration gradient (gravity_gradient.cuh)
-enum MbAlgo { MB_RNEA = 0, MB_ABA = 1, MB_CRBA = 2, MB_CORIOLIS = 3, MB_REGRESSOR = 4, MB_GRAVITY_GRADIENT = 5 };
-#define MB_NUM_ALGOS 6
+// MB_GRAVITY_GRADIENT: gravity torques and their configuration gradient (gravity_gradient.cuh); MB_RNEA_DERIVATIVES: joint efforts
+// and their derivatives in q and qd (rnea_derivatives.cuh)
+enum MbAlgo { MB_RNEA = 0, MB_ABA = 1, MB_CRBA = 2, MB_CORIOLIS = 3, MB_REGRESSOR = 4, MB_GRAVITY_GRADIENT = 5, MB_RNEA_DERIVATIVES = 6 };
+#define MB_NUM_ALGOS 7
 
 // Shared-memory stack slots (double2 per state) of a thread-per-state block.  With a tensor-memory stack (tm > 0 slots,
 // RNEA / ABA) the wide area lives in TMEM and only the narrow one in shared memory.  ABA overlays its pass-three ring
@@ -257,7 +258,7 @@ __host__ __device__
 static inline int mb_smem_stack_slots(int algo, const MbProgram &P, int tm)
 {
    int s = P.stack2;
-   if (tm > 0 && algo != MB_CRBA && algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT)
+   if (tm > 0 && algo != MB_CRBA && algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && algo != MB_RNEA_DERIVATIVES)
       s = P.nstack2 + (P.wstack2 > tm ? P.wstack2 - tm : 0); // wide slots beyond the TMEM share spill over behind the narrow area
    if (algo == MB_ABA && s < 4 * MB_ABA_RING_ROWS)
       s = 4 * MB_ABA_RING_ROWS; // the pass-three ring (4 stages) is overlaid on the stack area
@@ -272,5 +273,5 @@ __host__ __device__
 #endif
 static inline bool mb_tm_fits(int algo, const MbProgram &P, int tm, int block)
 {
-   return tm == 0 || (algo != MB_CRBA && algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && (P.wstack2 <= tm || block == MB_PARTIAL_TM_BLOCK));
+   return tm == 0 || (algo != MB_CRBA && algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && algo != MB_RNEA_DERIVATIVES && (P.wstack2 <= tm || block == MB_PARTIAL_TM_BLOCK));
 }

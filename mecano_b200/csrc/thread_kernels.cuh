@@ -7,6 +7,7 @@
 #include "kernels.h"
 #include "gravity_gradient.cuh"
 #include "regressor.cuh"
+#include "rnea_derivatives.cuh"
 
 namespace mb
 {
@@ -35,6 +36,8 @@ __device__ __forceinline__ void thread_kernel_body(const MbProgram &P, const Ker
       }
       else if constexpr (ALGO == MB_GRAVITY_GRADIENT)
          gravity_gradient_state<double, Ctx>(P, c2, a.grav);
+      else if constexpr (ALGO == MB_RNEA_DERIVATIVES)
+         rnea_derivatives_state<double, Ctx>(P, c2, a.grav);
       else
          coriolis_state<double, Ctx>(P, c2);
    });
@@ -75,6 +78,7 @@ constexpr int kCrbAux0 = 10 * 4, kCrbAux1 = 10 * 16;
 constexpr int kCorAux0 = 46 * 4, kCorAux1 = 46 * 16;
 constexpr int kRegAux0 = 12 * 4, kRegAux1 = 12 * 16;
 constexpr int kGgAux0 = 16 * 4, kGgAux1 = 16 * 16;
+constexpr int kRdAux0 = 58 * 4, kRdAux1 = 58 * 16;
 constexpr int kAbaRec0 = MB_ABA_REC * 33, kAbaRec1 = MB_ABA_REC * 128;
 // launch configurations: threads per block, work-area class, stack slots (double2) held in tensor memory
 struct Cfg
@@ -96,10 +100,11 @@ __host__ __device__ constexpr int aux_of(int algo, int cls)
                                             : (algo == MB_CRBA ? (cls ? kCrbAux1 : kCrbAux0)
                                                                : (algo == MB_REGRESSOR ? (cls ? kRegAux1 : kRegAux0)
                                                                                        : (algo == MB_GRAVITY_GRADIENT ? (cls ? kGgAux1 : kGgAux0)
-                                                                                                                      : (cls ? kCorAux1 : kCorAux0)))));
+                                                                                                                      : (algo == MB_RNEA_DERIVATIVES ? (cls ? kRdAux1 : kRdAux0)
+                                                                                                                                                     : (cls ? kCorAux1 : kCorAux0))))));
 }
 // the kernels whose stack lives in shared memory only (no wide area): their TMEM configurations alias the shared-memory kernels
-__host__ __device__ constexpr bool smem_stack_only(int algo) { return algo == MB_CRBA || algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT; }
+__host__ __device__ constexpr bool smem_stack_only(int algo) { return algo == MB_CRBA || algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES; }
 
 template <int ALGO, bool FEXT, int SM, bool M3> KernelFn pick_cfg(int cfg)
 {
@@ -122,7 +127,7 @@ constexpr int kF32Cfg[3] = {0, 1, 8}; // RNEA 512 threads + TMEM, ABA 384 thread
 KernelFn pick_f32(int algo);
 
 // the instantiation groups: X(group, ALGO, FEXT, LAYOUT, M3).  The store-bound matrix kernels (CRBA, Coriolis, regressor, gravity
-// gradient: external wrenches tested at run time) exist only
+// gradient and inverse-dynamics derivatives: external wrenches tested at run time) exist only
 // with the three-DoF joints compiled in (one unit-momentum column loop per multi-DoF joint either way); RNEA and ABA come in
 // both forms (multidof.cuh: mb_sub_of)
 #define MB_KERNEL_GROUPS(X)                                                                                             \
@@ -130,6 +135,6 @@ KernelFn pick_f32(int algo);
    X(4, MB_CRBA, false, 0, true) X(5, MB_CRBA, false, 1, true) X(6, MB_CRBA, false, 2, true) X(7, MB_CRBA, true, 0, true)   \
    X(8, MB_CORIOLIS, false, 0, true) X(9, MB_RNEA, false, 0, true) X(10, MB_RNEA, true, 0, true)                            \
    X(11, MB_ABA, false, 0, true) X(12, MB_ABA, true, 0, true) X(14, MB_REGRESSOR, false, 0, true)                           \
-   X(15, MB_GRAVITY_GRADIENT, false, 0, true)
-#define MB_NUM_KERNEL_GROUPS 15 // + group 13: the fp32 variant
+   X(15, MB_GRAVITY_GRADIENT, false, 0, true) X(16, MB_RNEA_DERIVATIVES, false, 0, true)
+#define MB_NUM_KERNEL_GROUPS 16 // + group 13: the fp32 variant
 } // namespace mb

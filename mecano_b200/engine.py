@@ -244,6 +244,26 @@ class Engine:
             check(lib.mecano_b200_gravity_gradient(self._h, n, ld, pq, pf, pt, pg, self._stream()), self._h)
         return G
 
+    def rnea_derivatives(self, q, qd, qdd, tau, dq, dqd, fext=None):
+        """tau [nv, n], dq and dqd [nv * nv, n] entry-major (mecano_b200_rnea_derivatives), fext [6 * nb, n] or None; torch CUDA
+        tensors or numpy arrays (host path)."""
+        n = q.shape[1]
+        host = isinstance(q, np.ndarray)
+        f = _host_ptr_ld if host else self._dp
+        pq, l0 = f(q, self.nq, n)
+        pv, l1 = f(qd, self.nv, n)
+        pa, l2 = f(qdd, self.nv, n)
+        pf, l3 = f(fext, 6 * self.nb, n)
+        pt, l4 = f(tau, self.nv, n)
+        pdq, l5 = f(dq, self.nv * self.nv, n)
+        pdv, l6 = f(dqd, self.nv * self.nv, n)
+        ld = _same_ld([l0, l1, l2, l3, l4, l5, l6])
+        if host:
+            check(lib.mecano_b200_rnea_derivatives_host(self._h, n, ld, pq, pv, pa, pf, pt, pdq, pdv), self._h)
+        else:
+            check(lib.mecano_b200_rnea_derivatives(self._h, n, ld, pq, pv, pa, pf, pt, pdq, pdv, self._stream()), self._h)
+        return dq
+
     def crba_centroidal(self, q, M, cmm, com, frame=_capi.FRAME_WORLD):
         """M [nv*nv, n] entry-major, cmm [6*nv, n], com [4, n]; torch CUDA tensors or numpy arrays (host path)."""
         n = q.shape[1]
@@ -500,7 +520,7 @@ class MultiDeviceEngine:
         raise NotImplementedError("this entry point is served per device: build the calculator on one device")
 
     aba_sources_host = coriolis = crba_centroidal = centroidal_convective_term = center_of_mass = integrate_host = set_joint_source_modes = _single_device_only
-    joint_torque_regressor = gravity_gradient = _single_device_only
+    joint_torque_regressor = gravity_gradient = rnea_derivatives = _single_device_only
 
 
 def measure_fp64_peak(device=0):
