@@ -45,14 +45,14 @@ struct mecano_b200_handle
    double gravity[3] = {0.0, 0.0, 0.0}; // Mecano calculators start with zero gravity until setGravitationalAcceleration
    mb::LaunchPlan plan[MB_NUM_ALGOS];
    bool fp32 = false; // mecano_b200_set_precision
-   int grid_limit[MB_NUM_ALGOS] = {0, 0, 0, 0, 0, 0, 0}; // mecano_b200_set_grid_limit: cap on the persistent grids (0 = whole device)
+   int grid_limit[MB_NUM_ALGOS] = {}; // mecano_b200_set_grid_limit: cap on the persistent grids (0 = whole device)
    int variant = MECANO_B200_VARIANT_AUTO;
    int max_children = 1, max_ndof = 1, sm_count = 148;
    int n_accel_source = 0;           // joints in ACCELERATION_SOURCE mode (mecano_b200_set_joint_source_modes)
    std::vector<std::pair<int, int>> effort_dof_runs; // (first DoF row, count) runs of DoF rows whose joints are EFFORT_SOURCE
    bool warp_ok = false;             // the body-parallel variant serves this tree (one-DoF / SixDoF joints; <= 32 bodies: a warp per state, else a team of warps)
    bool has_3dof = false;            // the tree has spherical / planar joints (generic thread-per-state kernels only)
-   int64_t warp_below[MB_NUM_ALGOS] = {0, 0, 0, 0, 0, 0, 0}; // AUTO: batches smaller than this run warp-per-state
+   int64_t warp_below[MB_NUM_ALGOS] = {}; // AUTO: batches smaller than this run warp-per-state
    std::string error;
    // host pipeline (lazy)
    cudaStream_t streams[MB_MAX_SLOTS] = {};
@@ -113,6 +113,13 @@ struct DeviceGuard
    DeviceGuard device_guard_((h)->device);                                         \
    if (device_guard_.err != cudaSuccess) return cuda_fail(h, device_guard_.err, "cudaSetDevice")
 
+// mecano_b200_kernel_info::bytes_per_state: what one state reads and writes (MbAlgoInfo::io_*)
+double bytes_per_state(int algo, double nq, double nv, double nb)
+{
+   const MbAlgoInfo d = mb_algo(algo);
+   return 8.0 * (d.io_nq * nq + d.io_nv * nv + d.io_nv2 * nv * nv + d.io_nbnv * nb * nv);
+}
+
 int check_batch(mecano_b200_handle *h, int64_t n, int64_t ld)
 {
    if (!h) return MECANO_B200_ERR_INVALID_ARGUMENT;
@@ -153,7 +160,7 @@ int run(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q,
    if (h->fp32)
    {
       // the optional fp32 variant: plain calls on the thread-per-state kernels only, never a silent fp64 substitute
-      if (algo > MB_CRBA || packed || fext || opt.body_acc || opt.joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || flags != 0)
+      if (mb_algo(algo).thread_only || packed || fext || opt.body_acc || opt.joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || flags != 0)
          return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the fp32 variant covers plain RNEA / ABA / CRBA calls only (no external wrenches, flags, by-products)");
       if (!h->plan[algo].fp32_ok || h->has_3dof)
          return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the fp32 variant is compiled for the launch configuration of humanoid-sized trees of one-DoF and SixDoF joints only");
@@ -162,7 +169,7 @@ int run(mecano_b200_handle *h, int algo, int64_t n, int64_t ld, const double *q,
    // states on; a thread per state needs tens of thousands but then has 10-30x the throughput)
    // calls with by-product buffers (mecano_b200_rnea_full) always run the generic thread-per-state kernel
    // (so does the packed mass-matrix layout: its row numbering follows the thread-per-state traversal)
-   const bool byprod = body_acc || joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES || h->fp32 || packed;
+   const bool byprod = body_acc || joint_wrench || x2 || opt.cmm || opt.com || opt.root_wrench || mb_algo(algo).thread_only || h->fp32 || packed;
    const int64_t vn = opt.variant_n > 0 ? opt.variant_n : n;
    const bool use_warp = !byprod && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && vn < h->warp_below[algo]));
    if (use_warp)
@@ -773,7 +780,7 @@ int mecano_b200_create(const mecano_b200_tree_desc *desc, int device, mecano_b20
    {
       bool fits = false;
       if ((e = mb::plan_thread_kernel(algo, h->tree.prog[algo], false, h->plan[algo], &fits)) != cudaSuccess) return bail(e, "kernel planning");
-      if (!fits && (algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES))
+      if (!fits && mb_algo(algo).thread_only)
       {
          h->plan[algo].block = 0; // a by-product kernel alone does not fit: its entry point reports it, everything else works
          continue;
@@ -1355,7 +1362,7 @@ int mecano_b200_step_host(mecano_b200_handle *h, int64_t n, int64_t ld, const do
 int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_states, mecano_b200_kernel_info *info)
 {
    if (!h || !info || algo < 0 || algo >= MB_NUM_ALGOS) return MECANO_B200_ERR_INVALID_ARGUMENT;
-   const bool warp = algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && algo != MB_RNEA_DERIVATIVES && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && n_states > 0 && n_states < h->warp_below[algo]));
+   const bool warp = !mb_algo(algo).thread_only && (h->variant == MECANO_B200_VARIANT_WARP || (h->variant == MECANO_B200_VARIANT_AUTO && h->warp_ok && n_states > 0 && n_states < h->warp_below[algo]));
    if (warp)
    {
       std::memset(info, 0, sizeof *info);
@@ -1371,8 +1378,7 @@ int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_state
       info->static_smem_bytes = (int32_t)fa.sharedSizeBytes;
       info->sm_count = h->sm_count;
       info->max_depth = h->tree.prog[algo].max_depth;
-      const double nq = h->tree.nq, nv = h->tree.nv;
-      info->bytes_per_state = algo == MB_CRBA ? 8.0 * (nq + nv * nv) : 8.0 * (nq + 3.0 * nv);
+      info->bytes_per_state = bytes_per_state(algo, h->tree.nq, h->tree.nv, h->tree.prog[algo].nb);
       return MECANO_B200_OK;
    }
    const mb::LaunchPlan &p = h->plan[algo];
@@ -1407,14 +1413,7 @@ int mecano_b200_kernel_info_get(mecano_b200_handle *h, int algo, int64_t n_state
    cudaDeviceGetAttribute(&info->sm_count, cudaDevAttrMultiProcessorCount, h->device);
    info->stack_doubles = P.stack_doubles;
    info->max_depth = P.max_depth;
-   const double nq = P.nq, nv = P.nv;
-   // (the gravity gradient: q in, tau and G out; the inverse-dynamics derivatives: q, qd, qdd in, tau and two matrices out; a call with
-   // external wrenches reads 48 n_bodies bytes more)
-   info->bytes_per_state = algo == MB_CRBA ? 8.0 * (nq + nv * nv)
-                           : (algo == MB_RNEA_DERIVATIVES ? 8.0 * (nq + 3.0 * nv + 2.0 * nv * nv)
-                           : (algo == MB_GRAVITY_GRADIENT ? 8.0 * (nq + nv + nv * nv)
-                           : (algo == MB_CORIOLIS ? 8.0 * (nq + nv + 2.0 * nv * nv)
-                                                  : (algo == MB_REGRESSOR ? 8.0 * (nq + 2.0 * nv + 10.0 * P.nb * nv) : 8.0 * (nq + 3.0 * nv))))); // SURVEY.md 8(d)
+   info->bytes_per_state = bytes_per_state(algo, P.nq, P.nv, P.nb);
    return MECANO_B200_OK;
 }
 

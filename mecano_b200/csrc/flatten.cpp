@@ -93,21 +93,6 @@ int slot_size(int algo, int jtype)
    }
 }
 
-int aux_size(int algo)
-{
-   switch (algo)
-   {
-      case MB_RNEA:
-      case MB_REGRESSOR: return 12; // twist + spatial acceleration of a branching body
-      case MB_ABA: return 27;  // articulated inertia (6 + 9 + 6) + bias wrench (6); reused for (v, a) in pass three
-      case MB_CORIOLIS: return 46; // composite inertia (10) + composite factorized inertia (4 x 9)
-      case MB_GRAVITY_GRADIENT: return 16; // composite inertia (10) + composite external wrench (6)
-      case MB_RNEA_DERIVATIVES: return 58; // composite inertia (10), factorized inertia (4 x 9), momentum (6), RNEA force (6)
-      default: return 10;      // composite inertia (6 + 3 + 1)
-   }
-}
-
-
 // v2 stack slots, in double2 units (rnea.cuh / aba.cuh / crba.cuh)
 int slot2_size(int algo, int jtype, bool root_parent)
 {
@@ -178,7 +163,7 @@ void build_op2(int algo, MbProgram &P, const std::vector<int> &nchild)
       {
          const MbBody &Bp = P.body[B.parent];
          s = slot2[B.parent] + slot2_size(algo, Bp.jtype, Bp.parent < 0);
-         if (algo == MB_RNEA || algo == MB_ABA)
+         if (mb_algo(algo).wide_stack)
          {
             wslot[i] = wslot[B.parent] + 3;
             nslot[i] = nslot[B.parent] + slot2_size(algo, Bp.jtype, Bp.parent < 0) - 3;
@@ -189,7 +174,7 @@ void build_op2(int algo, MbProgram &P, const std::vector<int> &nchild)
       if (nchild[i] > 0 || B.jtype == MB_SIXDOF)
       {
          P.stack2 = std::max(P.stack2, s + slot2_size(algo, B.jtype, B.parent < 0));
-         if (algo == MB_RNEA || algo == MB_ABA)
+         if (mb_algo(algo).wide_stack)
          {
             P.wstack2 = std::max(P.wstack2, wslot[i] + 3);
             P.nstack2 = std::max(P.nstack2, nslot[i] + slot2_size(algo, B.jtype, B.parent < 0) - 3);
@@ -564,10 +549,10 @@ int flatten_tree(const mecano_b200_tree_desc *d, FlatTree &out, std::string &err
          int paux = 0;
          for (int a = parent_i[i]; a >= 0; a = parent_i[a])
             if (nchild[a] >= 2)
-               paux += aux_size(algo);
+               paux += mb_algo(algo).aux;
          B.aux = nchild[i] >= 2 ? paux : -1;
          if (nchild[i] >= 2)
-            P.aux_doubles = std::max(P.aux_doubles, paux + aux_size(algo));
+            P.aux_doubles = std::max(P.aux_doubles, paux + mb_algo(algo).aux);
          B.rec = -1;
          if (B.jtype == MB_SIXDOF && B.sub != MB_SUB_SIX)
          {

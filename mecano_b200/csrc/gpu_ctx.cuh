@@ -30,8 +30,8 @@ __device__ __forceinline__ unsigned mb_smem_u32()
 // thread's stack live in TMEM instead: a warp owns the 32 lanes of its lane quarter (warp % 4) and a private range of
 // columns, a double2 is four 32-bit columns, lane = thread: tcgen05.st/ld.32x32b.x4 (STTM/LDTM, scoreboarded like any
 // load).  Slots >= TM stay in shared memory.  scripts/microbench/tmem_stack.cu measures the round trip.
-// ROWS: rows of the prefetch ring per stage -- RNEA (q, qd, qdd), ABA (q | tau, qd: an op never needs q and tau together), CRBA (q)
-__host__ __device__ constexpr int ring_rows(int algo) { return algo == MB_RNEA ? 3 : (algo == MB_ABA ? 2 : 1); }
+// ROWS: rows of the prefetch ring per stage (program.h: MbAlgoInfo)
+__host__ __device__ constexpr int ring_rows(int algo) { return mb_algo(algo).ring_rows; }
 
 // handle of a constant record in shared memory (Ctx::cst): 32-bit shared address of the record
 struct SmemCst
@@ -407,7 +407,7 @@ template <int ALGO, bool STATE_MAJOR, int BLOCK, int AUXN, int TM, bool M3 = fal
 __device__ __forceinline__ void thread_block_run(const KernelArgs &a, const int ncst, const int smem_slots, const int nstack2, Body body)
 {
    static_assert(TM * 4 <= tm_warp_cols(BLOCK), "TMEM stack slots exceed the columns of one warp");
-   static_assert(TM == 0 || ALGO != MB_CRBA, "CRBA keeps its (narrow-only) stack in shared memory");
+   static_assert(TM == 0 || mb_algo(ALGO).wide_stack, "a kernel without a wide stack area keeps its stack in shared memory");
    __shared__ unsigned tm_base_s;
    if (TM > 0)
    {

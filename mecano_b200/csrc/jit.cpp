@@ -256,8 +256,7 @@ int spec_compile_only(const std::string &src, size_t *cubin_bytes, std::string &
 size_t spec_smem_bytes(int algo, const MbProgram &P, int block, int tm)
 {
    const int smem_slots = mb_smem_stack_slots(algo, P, tm);
-   const int rows = algo == MB_RNEA ? 3 : (algo == MB_ABA ? 2 : 1); // gpu_ctx.cuh: ring_rows()
-   size_t bytes = sizeof(double) * ((2 * (size_t)smem_slots + rows * MB_PF_STAGES) * block);
+   size_t bytes = sizeof(double) * ((2 * (size_t)smem_slots + mb_algo(algo).ring_rows * MB_PF_STAGES) * block);
    // a block with a TMEM stack allocates all 512 columns: keep it alone on its SM (a second block would spin in tcgen05.alloc)
    if (tm > 0)
       bytes = std::max<size_t>(bytes, 120 * 1024);

@@ -97,9 +97,9 @@ MB_KERNEL_GROUPS(MB_X)
 #if MB_INST == 13
 KernelFn pick_f32(int algo)
 {
-   if (algo == MB_RNEA) return thread_kernel_f32<MB_RNEA, kCfg[kF32Cfg[0]].block, kRnaAux0, 0, kCfg[kF32Cfg[0]].tm>;
-   if (algo == MB_ABA) return thread_kernel_f32<MB_ABA, kCfg[kF32Cfg[1]].block, kAbaAux0, kAbaRec0, kCfg[kF32Cfg[1]].tm>;
-   return thread_kernel_f32<MB_CRBA, kCfg[kF32Cfg[2]].block, kCrbAux0, 0, 0>;
+   if (algo == MB_RNEA) return thread_kernel_f32<MB_RNEA, kCfg[kF32Cfg[0]].block, aux_of(MB_RNEA, 0), 0, kCfg[kF32Cfg[0]].tm>;
+   if (algo == MB_ABA) return thread_kernel_f32<MB_ABA, kCfg[kF32Cfg[1]].block, aux_of(MB_ABA, 0), kAbaRec0, kCfg[kF32Cfg[1]].tm>;
+   return thread_kernel_f32<MB_CRBA, kCfg[kF32Cfg[2]].block, aux_of(MB_CRBA, 0), 0, 0>;
 }
 #endif
 } // namespace mb

@@ -16,6 +16,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <string>
 #include <type_traits>
 
 #include "thread_kernels.cuh"
@@ -72,9 +73,9 @@ int forced_cfg(int algo)
 {
    const char *e = getenv("MECANO_B200_CFG");
    if (!e) return -1;
-   const char *key = algo == MB_RNEA ? "rnea=" : (algo == MB_ABA ? "aba=" : (algo == MB_CRBA ? "crba=" : (algo == MB_REGRESSOR ? "reg=" : (algo == MB_GRAVITY_GRADIENT ? "gg=" : (algo == MB_RNEA_DERIVATIVES ? "rd=" : "cor=")))));
-   const char *p = strstr(e, key);
-   return p ? atoi(p + strlen(key)) : -1;
+   const std::string key = std::string(mb_algo(algo).cfg_key) + "=";
+   const char *p = strstr(e, key.c_str());
+   return p ? atoi(p + key.size()) : -1;
 }
 } // namespace
 
@@ -134,22 +135,13 @@ cudaError_t plan_thread_kernel(int algo, const MbProgram &P, bool fext, LaunchPl
          nblk = 1; // cannot happen (smem_bytes), but a TMEM block must be alone on its SM
       // register spills cost more than the extra warps bring: a configuration whose kernel spills beyond its declared
       // work area only competes if nothing else fits
-      const int auxn = aux_of(algo, kCfg[cfg].cls);
-      // (the Coriolis kernel keeps two 46-double accumulators and three force columns live: a few hundred bytes of spills are its
-      // normal state at 255 registers; so are some 670 bytes for the inverse-dynamics derivatives, four accumulators of 58 doubles
-      // and four force columns)
-      const bool spills = (long)fa.localSizeBytes > 8l * auxn + (algo == MB_CORIOLIS ? 512 : (algo == MB_RNEA_DERIVATIVES ? 768 : 128));
+      const bool spills = (long)fa.localSizeBytes > 8l * aux_of(algo, kCfg[cfg].cls) + mb_algo(algo).spill_bytes;
       // warps that do not split evenly over the four sub-partitions lose more than they bring (ABA 320 threads: 3.44 ms,
       // 256 threads: 2.23 ms; profiles/r01i_cfg_sweep.jsonl): such block sizes only compete if nothing else fits
       const bool uneven = ((nblk * b) % 128) != 0 && nblk * b > 128;
       const int score = (spills || uneven) && forced < 0 ? 1 + (uneven ? 1 : 0) : nblk * b;
-      // prefer more resident states; on ties the first configuration in the table wins -- except for the two store-bound
-      // mass-matrix kernels, where more, smaller blocks win: hardware block scheduling evens out their store bursts (Coriolis,
-      // H37: 2 x 128 threads 5.89 ms, 1 x 256 6.54 ms, profiles/r02h_cor_sweep.jsonl; CRBA, 4 x 128 against 2 x 256 threads:
-      // 7 / 15 / 25 / 32 / 51 bodies -2.9 / -8.4 / -0.8 / -1.4 / -4.3 %, profiles/r03g_crba_block_sweep.jsonl); the
-      // regressor, the gravity gradient and the inverse-dynamics derivatives, store-bound the same way, follow them
-      const bool small_blocks = algo == MB_CORIOLIS || algo == MB_CRBA || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES;
-      if (nblk > 0 && (score > best_threads || (small_blocks && score == best_threads && b < plan.block)))
+      // prefer more resident states; on ties the first configuration in the table wins, or the smaller block (MbAlgoInfo::small_blocks)
+      if (nblk > 0 && (score > best_threads || (mb_algo(algo).small_blocks && score == best_threads && b < plan.block)))
       {
          best_threads = score;
          plan.block = b;
@@ -172,7 +164,7 @@ cudaError_t plan_thread_kernel(int algo, const MbProgram &P, bool fext, LaunchPl
    plan.local_bytes = (int)attr.localSizeBytes;
    plan.static_smem = (int)attr.sharedSizeBytes;
    // the fp32 variant exists for the configuration the planner picks for humanoid-sized trees
-   plan.fp32_ok = algo <= MB_CRBA && plan.size_class == kF32Cfg[algo] && !m3;
+   plan.fp32_ok = !mb_algo(algo).thread_only && plan.size_class == kF32Cfg[algo] && !m3;
    if (plan.fp32_ok)
    {
       cudaFuncAttributes fa32;
@@ -215,8 +207,8 @@ cudaError_t launch_thread_kernel(int algo, const MbProgram &P, const KernelArgs 
    const bool persistent = grid < (unsigned)ntiles;
    static const bool draw = [] { const char *e = getenv("MECANO_B200_DRAW"); return !e || atoi(e) != 0; }();
    // the warps of a persistent grid draw their states from a counter that the kernel itself re-arms (gpu_ctx.cuh: thread_block_run)
-   // (RNEA / ABA only: the mass-matrix kernels are launched one block per tile, and their stores carry no guard for clamped lanes)
-   if (!(persistent && draw) || smem_stack_only(algo))
+   // (wide-stack kernels only: the mass-matrix kernels are launched one block per tile, and their stores carry no guard for clamped lanes)
+   if (!(persistent && draw) || !mb_algo(algo).wide_stack)
       b.work_counter = nullptr;
    fn<<<grid, plan.block, plan.smem, stream>>>(P, b);
    return cudaGetLastError();

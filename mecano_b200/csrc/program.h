@@ -249,16 +249,60 @@ static inline int mb_sub_ndof(int sub) { return sub == MB_SUB_SIX ? 6 : 3; }
 enum MbAlgo { MB_RNEA = 0, MB_ABA = 1, MB_CRBA = 2, MB_CORIOLIS = 3, MB_REGRESSOR = 4, MB_GRAVITY_GRADIENT = 5, MB_RNEA_DERIVATIVES = 6 };
 #define MB_NUM_ALGOS 7
 
+// What the flattener, the planner, the launcher and the C ABI need to know about a thread-per-state algorithm (mb_algo).
+struct MbAlgoInfo
+{
+   const char *cfg_key; // its key in MECANO_B200_CFG (kernels.cu: forced_cfg)
+   int aux;             // branch save area per nested branching body (doubles, local memory; thread_kernels.cuh: aux_of)
+   bool wide_stack;     // the stack is split into a wide area, which may live in tensor memory, and a narrow one (MbOp2); without
+                        // it the whole stack is in shared memory and the TMEM configurations are never planned
+   bool thread_only;    // the generic thread-per-state kernel is its only form (no warp, team, tree-specialised or fp32 kernel);
+                        // when it does not fit, only its own entry point fails, not the handle
+   int ring_rows;       // double2 rows per stage of the prefetch ring (gpu_ctx.cuh)
+   int spill_bytes;     // local memory beyond the work area that the planner accepts before it counts the kernel as spilling
+   bool small_blocks;   // planner tie-break: more, smaller blocks win, as hardware block scheduling evens out the store bursts
+                        // of the store-bound matrix kernels (Coriolis, H37: 2 x 128 threads 5.89 ms, 1 x 256 6.54 ms,
+                        // profiles/r02h_cor_sweep.jsonl; CRBA, 4 x 128 against 2 x 256 threads: 7 / 15 / 25 / 32 / 51 bodies
+                        // -2.9 / -8.4 / -0.8 / -1.4 / -4.3 %, profiles/r03g_crba_block_sweep.jsonl)
+   int io_nq, io_nv, io_nv2, io_nbnv; // kernel_info bytes per state / 8: per configuration row, DoF, nv x nv and nb x nv entry
+                                      // (SURVEY.md 8(d); a call with external wrenches reads 48 n_bodies bytes more)
+};
+#if defined(__CUDACC__)
+__host__ __device__
+#endif
+static constexpr MbAlgoInfo mb_algo(int algo)
+{
+   switch (algo)
+   {
+      // aux: twist + spatial acceleration of a branching body; ring: q, qd, qdd
+      case MB_RNEA: return {"rnea", 12, true, false, 3, 128, false, 1, 3, 0, 0};
+      // aux: articulated inertia (6 + 9 + 6) + bias wrench (6), reused for (v, a) in pass three; ring: q | tau, qd (an op never
+      // needs q and tau together)
+      case MB_ABA: return {"aba", 27, true, false, 2, 128, false, 1, 3, 0, 0};
+      // aux: composite inertia (6 + 3 + 1); ring: q
+      case MB_CRBA: return {"crba", 10, false, false, 1, 128, true, 1, 0, 1, 0};
+      // aux: composite inertia (10) + composite factorized inertia (4 x 9); spills: with two 46-double accumulators and three
+      // force columns live, a few hundred bytes are its normal state at 255 registers
+      case MB_CORIOLIS: return {"cor", 46, false, true, 1, 512, true, 1, 1, 2, 0};
+      case MB_REGRESSOR: return {"reg", 12, false, true, 1, 128, true, 1, 2, 0, 10}; // aux: twist + spatial acceleration
+      case MB_GRAVITY_GRADIENT: return {"gg", 16, false, true, 1, 128, true, 1, 1, 1, 0}; // aux: composite inertia (10) + external wrench (6)
+      // aux: composite inertia (10), factorized inertia (4 x 9), momentum (6), RNEA force (6); spills: some 670 bytes, with four
+      // accumulators of 58 doubles and four force columns live
+      case MB_RNEA_DERIVATIVES: return {"rd", 58, false, true, 1, 768, true, 1, 3, 2, 0};
+   }
+   return {}; // not an algorithm
+}
+
 // Shared-memory stack slots (double2 per state) of a thread-per-state block.  With a tensor-memory stack (tm > 0 slots,
-// RNEA / ABA) the wide area lives in TMEM and only the narrow one in shared memory.  ABA overlays its pass-three ring
-// (4 stages x MB_ABA_RING_ROWS rows) on the stack area.
+// wide-stack algorithms) the wide area lives in TMEM and only the narrow one in shared memory.  ABA overlays its pass-three
+// ring (4 stages x MB_ABA_RING_ROWS rows) on the stack area.
 #if defined(__CUDACC__)
 __host__ __device__
 #endif
 static inline int mb_smem_stack_slots(int algo, const MbProgram &P, int tm)
 {
    int s = P.stack2;
-   if (tm > 0 && algo != MB_CRBA && algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && algo != MB_RNEA_DERIVATIVES)
+   if (tm > 0 && mb_algo(algo).wide_stack)
       s = P.nstack2 + (P.wstack2 > tm ? P.wstack2 - tm : 0); // wide slots beyond the TMEM share spill over behind the narrow area
    if (algo == MB_ABA && s < 4 * MB_ABA_RING_ROWS)
       s = 4 * MB_ABA_RING_ROWS; // the pass-three ring (4 stages) is overlaid on the stack area
@@ -273,5 +317,5 @@ __host__ __device__
 #endif
 static inline bool mb_tm_fits(int algo, const MbProgram &P, int tm, int block)
 {
-   return tm == 0 || (algo != MB_CRBA && algo != MB_CORIOLIS && algo != MB_REGRESSOR && algo != MB_GRAVITY_GRADIENT && algo != MB_RNEA_DERIVATIVES && (P.wstack2 <= tm || block == MB_PARTIAL_TM_BLOCK));
+   return tm == 0 || (mb_algo(algo).wide_stack && (P.wstack2 <= tm || block == MB_PARTIAL_TM_BLOCK));
 }

@@ -72,13 +72,7 @@ __global__ void __launch_bounds__(BLOCK) thread_kernel_f32(const __grid_constant
 // compiled work-area classes (local memory per thread): {aux, rec}
 //   class 0: up to 4 nested branching bodies, 32 one-DoF-equivalent records (humanoids); blocks of 256 / 128
 //   class 1: up to 16 nested branching bodies, 128 bodies; blocks of 128 / 64 / 32 (deeper stacks)
-constexpr int kRnaAux0 = 12 * 4, kRnaAux1 = 12 * 16;
-constexpr int kAbaAux0 = 27 * 4, kAbaAux1 = 27 * 16;
-constexpr int kCrbAux0 = 10 * 4, kCrbAux1 = 10 * 16;
-constexpr int kCorAux0 = 46 * 4, kCorAux1 = 46 * 16;
-constexpr int kRegAux0 = 12 * 4, kRegAux1 = 12 * 16;
-constexpr int kGgAux0 = 16 * 4, kGgAux1 = 16 * 16;
-constexpr int kRdAux0 = 58 * 4, kRdAux1 = 58 * 16;
+__host__ __device__ constexpr int aux_of(int algo, int cls) { return mb_algo(algo).aux * (cls ? 16 : 4); }
 constexpr int kAbaRec0 = MB_ABA_REC * 33, kAbaRec1 = MB_ABA_REC * 128;
 // launch configurations: threads per block, work-area class, stack slots (double2) held in tensor memory
 struct Cfg
@@ -92,37 +86,25 @@ constexpr Cfg kCfg[kNumCfg] = {{512, 0, 32}, {384, 0, 42}, {320, 0, 42}, {256, 0
 
 typedef void (*KernelFn)(const MbProgram, const KernelArgs);
 
-// work area (doubles) of an algorithm's class 0 / 1
-__host__ __device__ constexpr int aux_of(int algo, int cls)
-{
-   return algo == MB_RNEA ? (cls ? kRnaAux1 : kRnaAux0)
-                          : (algo == MB_ABA ? (cls ? kAbaAux1 : kAbaAux0)
-                                            : (algo == MB_CRBA ? (cls ? kCrbAux1 : kCrbAux0)
-                                                               : (algo == MB_REGRESSOR ? (cls ? kRegAux1 : kRegAux0)
-                                                                                       : (algo == MB_GRAVITY_GRADIENT ? (cls ? kGgAux1 : kGgAux0)
-                                                                                                                      : (algo == MB_RNEA_DERIVATIVES ? (cls ? kRdAux1 : kRdAux0)
-                                                                                                                                                     : (cls ? kCorAux1 : kCorAux0))))));
-}
-// the kernels whose stack lives in shared memory only (no wide area): their TMEM configurations alias the shared-memory kernels
-__host__ __device__ constexpr bool smem_stack_only(int algo) { return algo == MB_CRBA || algo == MB_CORIOLIS || algo == MB_REGRESSOR || algo == MB_GRAVITY_GRADIENT || algo == MB_RNEA_DERIVATIVES; }
-
 template <int ALGO, bool FEXT, int SM, bool M3> KernelFn pick_cfg(int cfg)
 {
    constexpr int a0 = aux_of(ALGO, 0);
    constexpr int a1 = aux_of(ALGO, 1);
    constexpr int r0 = ALGO == MB_ABA ? kAbaRec0 : 0, r1 = ALGO == MB_ABA ? kAbaRec1 : 0;
+   constexpr bool wide = mb_algo(ALGO).wide_stack;
    switch (cfg)
    {
-      // CRBA has no wide stack area: its TMEM configurations are never planned (mb_tm_fits) and alias the shared-memory kernels
-#define MB_CFG_CASE(i) case i: return thread_kernel<ALGO, FEXT, SM, kCfg[i].block, kCfg[i].cls ? a1 : a0, kCfg[i].cls ? r1 : r0, smem_stack_only(ALGO) ? 0 : kCfg[i].tm, M3>;
+      // without a wide stack area the TMEM configurations are never planned (mb_tm_fits) and alias the shared-memory kernels
+#define MB_CFG_CASE(i) case i: return thread_kernel<ALGO, FEXT, SM, kCfg[i].block, kCfg[i].cls ? a1 : a0, kCfg[i].cls ? r1 : r0, wide ? kCfg[i].tm : 0, M3>;
       MB_CFG_CASE(0) MB_CFG_CASE(1) MB_CFG_CASE(2) MB_CFG_CASE(3) MB_CFG_CASE(4) MB_CFG_CASE(5) MB_CFG_CASE(6)
       MB_CFG_CASE(7) MB_CFG_CASE(8) MB_CFG_CASE(9) MB_CFG_CASE(10) MB_CFG_CASE(11) MB_CFG_CASE(12) MB_CFG_CASE(14)
 #undef MB_CFG_CASE
-      default: return thread_kernel<ALGO, FEXT, SM, kCfg[13].block, a1, r1, smem_stack_only(ALGO) ? 0 : kCfg[13].tm, M3>;
+      default: return thread_kernel<ALGO, FEXT, SM, kCfg[13].block, a1, r1, wide ? kCfg[13].tm : 0, M3>;
    }
 }
 
-// fp32 variant: the one configuration per algorithm that the planner picks for humanoid-sized trees (kCfg index, class 0)
+// fp32 variant: the one configuration per algorithm that the planner picks for humanoid-sized trees (kCfg index, class 0),
+// for the algorithms that are not thread-only (MbAlgoInfo)
 constexpr int kF32Cfg[3] = {0, 1, 8}; // RNEA 512 threads + TMEM, ABA 384 threads + TMEM, CRBA 128 threads
 KernelFn pick_f32(int algo);
 
