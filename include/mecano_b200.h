@@ -358,6 +358,29 @@ int mecano_b200_rnea_derivatives(mecano_b200_handle *h, int64_t n_states, int64_
                                  const double *fext, double *tau, double *dtau_dq, double *dtau_dqd, void *stream);
 
 /*
+ * Forward-dynamics derivatives: the joint accelerations qdd(q, qd, tau) of ABA, their first-order partials d qdd / dq and d qdd / dqd,
+ * and d qdd / d tau = M^-1 -- the A = [d qdd / dq, d qdd / dqd] and B = M^-1 of the dynamics xdot = f(x, u), u = tau, that iLQR / DDP,
+ * MPC and batched-simulation gradients consume.  For N states, with the handle's gravity:
+ *   qdd       [n_dofs][ld]            what mecano_b200_aba computes on the same q, qd, tau and fext, bit for bit
+ *   dqdd_dq   [n_dofs * n_dofs][ld]   entry (i, j) at [(i * n_dofs + j) * ld + s], entry-major like the mass matrix
+ *   dqdd_dqd  [n_dofs * n_dofs][ld]   the same layout
+ *   minv      [n_dofs * n_dofs][ld]   the same layout
+ * Every entry of the three matrices is written.  Unlike M, M^-1 has no structural zeros in general: only the entries between
+ * branches that hang separately off the fixed root are zero (0.0), in minv and in both partials.  The conventions are those of
+ * mecano_b200_rnea_derivatives: column j of dqdd_dq is the derivative along the step mecano_b200_integrate takes with qd = e_j, so a
+ * floating base's columns are perturbations in its own frame; qd, tau and fext are held, and fext (nullable, the convention of
+ * mecano_b200_rnea) is body-fixed.  Since ID(q, qd, FD(q, qd, tau)) = tau,
+ *   dqdd_dq = -M^-1 dtau_dq(q, qd, qdd),   dqdd_dqd = -M^-1 dtau_dqd(q, qd, qdd),   minv = M^-1,
+ * and this is how they are computed: mecano_b200_aba, mecano_b200_rnea_derivatives at its qdd, mecano_b200_crba, then one kernel that
+ * factors M = L^T D L along the kinematic tree (no fill-in) and solves in place -- four launches on `stream`, no workspace.
+ * Refusals: a handle set to fp32 (MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY), a joint in ACCELERATION_SOURCE mode
+ * (MECANO_B200_ERR_INVALID_ARGUMENT), with fext a wrench_index rank >= n_bodies (MECANO_B200_ERR_SHAPE), and a tree the
+ * inverse-dynamics derivatives kernel does not fit (MECANO_B200_ERR_TOO_LARGE).  Mecano has no counterpart of this call.
+ */
+int mecano_b200_aba_derivatives(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd, const double *tau,
+                                const double *fext, double *qdd, double *dqdd_dq, double *dqdd_dqd, double *minv, void *stream);
+
+/*
  * Host-pointer entry points (what a JNI / Panama binding calls with DMatrixRMaj.data): inputs are
  * staged host -> device in chunks, the kernels run, results are copied back; the call returns when
  * the outputs are complete.  Pinned (page-locked) host memory makes the copies asynchronous and
@@ -422,6 +445,8 @@ int mecano_b200_gravity_gradient_host(mecano_b200_handle *h, int64_t n_states, i
                                       double *gradient);
 int mecano_b200_rnea_derivatives_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd, const double *qdd,
                                       const double *fext, double *tau, double *dtau_dq, double *dtau_dqd);
+int mecano_b200_aba_derivatives_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd, const double *tau,
+                                     const double *fext, double *qdd, double *dqdd_dq, double *dqdd_dqd, double *minv);
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, double *mass_matrix, double *cmm,
                                      double *com, int frame);
 int mecano_b200_centroidal_convective_term_host(mecano_b200_handle *h, int64_t n_states, int64_t ld, const double *q, const double *qd,

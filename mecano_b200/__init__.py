@@ -6,9 +6,10 @@ not been built: there is no CPU fallback.
 """
 from . import _capi  # noqa: F401  (raises ImportError if libmecano_b200.so is missing)
 from ._capi import MecanoB200Error  # noqa: F401
-from .calculators import (CompositeRigidBodyMassMatrixCalculator, ForwardDynamicsCalculator, InverseDynamicsCalculator,  # noqa: F401
-                          InverseDynamicsDerivativesCalculator, JointSourceMode, JointTorqueRegressorCalculator, MatrixDimensionException,
-                          MultiBodyDynamicsStep, MultiBodyGravityGradientCalculator, MultiBodySystemStateIntegrator)
+from .calculators import (CompositeRigidBodyMassMatrixCalculator, ForwardDynamicsCalculator,  # noqa: F401
+                          ForwardDynamicsDerivativesCalculator, InverseDynamicsCalculator, InverseDynamicsDerivativesCalculator,
+                          JointSourceMode, JointTorqueRegressorCalculator, MatrixDimensionException, MultiBodyDynamicsStep,
+                          MultiBodyGravityGradientCalculator, MultiBodySystemStateIntegrator)
 from .engine import Engine, MultiDeviceEngine, measure_fp64_peak, measure_fp64_sustained, measure_hbm_peak  # noqa: F401
 from .multibody import (FixedJoint, JointMatrixIndexProvider, MultiBodySystem, MultiBodySystemRandomTools, PlanarJoint, PrismaticJoint,  # noqa: F401
                         RevoluteJoint, RigidBody, RigidBodyTransform, ScrewTheoryException, SixDoFJoint, SphericalJoint)

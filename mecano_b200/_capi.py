@@ -79,6 +79,7 @@ EXPORTS = [
     "mecano_b200_joint_torque_regressor", "mecano_b200_joint_torque_regressor_host",
     "mecano_b200_gravity_gradient", "mecano_b200_gravity_gradient_host",
     "mecano_b200_rnea_derivatives", "mecano_b200_rnea_derivatives_host",
+    "mecano_b200_aba_derivatives", "mecano_b200_aba_derivatives_host",
 ]
 
 lib.mecano_b200_create.argtypes = [ctypes.POINTER(TreeDesc), ctypes.c_int, ctypes.POINTER(c_vp)]
@@ -115,6 +116,8 @@ lib.mecano_b200_gravity_gradient.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_v
 lib.mecano_b200_gravity_gradient_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp]
 lib.mecano_b200_rnea_derivatives.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
 lib.mecano_b200_rnea_derivatives_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
+lib.mecano_b200_aba_derivatives.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
+lib.mecano_b200_aba_derivatives_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]
 lib.mecano_b200_crba.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_u32, c_vp]
 lib.mecano_b200_rnea_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_u32]
 lib.mecano_b200_aba_host.argtypes = [c_vp, c_i64, c_i64, c_vp, c_vp, c_vp, c_vp, c_vp, c_u32]

@@ -6,6 +6,7 @@
     JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, see the class)
     MultiBodyGravityGradientCalculator        gravity torques and their configuration gradient (project definition, see the class)
     InverseDynamicsDerivativesCalculator      d tau / dq and d tau / dqd of inverse dynamics (project definition, see the class)
+    ForwardDynamicsDerivativesCalculator      d qdd / dq, d qdd / dqd and M^-1 of forward dynamics (project definition, see the class)
 
 Same names, argument meaning and error behaviour as the reference; the batching changes are that the joint state
 is passed explicitly as [rows, N] matrices (Mecano reads it from the joint objects) and that results come back as
@@ -726,6 +727,58 @@ class InverseDynamicsDerivativesCalculator(_BatchedCalculator):
 
     def getTauVelocityGradientMatrix(self):
         return self._dqd
+
+
+class ForwardDynamicsDerivativesCalculator(_BatchedCalculator):
+    """The first-order partials of forward dynamics for N states: qdd(q, qd, tau) of ForwardDynamicsCalculator together with
+    d qdd / dq, d qdd / dqd and d qdd / d tau = M^-1 (mecano_b200_aba_derivatives in include/mecano_b200.h: the conventions of
+    InverseDynamicsDerivativesCalculator -- column j of d qdd / dq is the derivative along the step the state integrator takes with
+    qd = e_j, so a floating base's columns are perturbations in its own frame; qd, tau and the body-fixed external wrenches are
+    held).  These are A = [d qdd / dq, d qdd / dqd] and B = M^-1 of xdot = f(x, u), u = tau.  Mecano has no counterpart: the
+    definition is this project's.
+
+    getJointAccelerationMatrix() is [nDoFs, N] and bit for bit what ForwardDynamicsCalculator computes; the three matrices are
+    [nDoFs * nDoFs, N], entry (i, j) of state s at [i * nDoFs + j, s].  Systems with fixed or ignored joints run on their welded
+    tables; external wrenches on such systems are not supported (the locked-joint reduction changes M^-1).  Every joint is an
+    EFFORT_SOURCE.  One device only.  kernelInfo() / setGridLimit() concern the inverse-dynamics derivatives kernel, the
+    heaviest of the four launches."""
+    _ALGO = _capi.ALGO_RNEA_DERIVATIVES
+
+    def __init__(self, input, device=0):
+        super().__init__(input, device)
+        self._qdd = self._dq = self._dqd = self._minv = None
+
+    def compute(self, q, qd, tau):
+        """compute(q, qd, tau) for N states; returns getAccelerationConfigurationGradientMatrix() ([nDoFs * nDoFs, N])."""
+        if isinstance(self._device, (list, tuple)):
+            raise NotImplementedError("the forward-dynamics derivatives run on one device")
+        nv, nq = self._input.getNumberOfDoFs(), self._input.getConfigurationMatrixSize()
+        n = q.shape[1] if q.ndim == 2 else -1
+        self._check("q", q, nq, n)
+        self._check("qd", qd, nv, n)
+        self._check("tau", tau, nv, n)
+        if self._fext is not None:
+            self._check("externalWrenches", self._fext, 6 * self._input.getNumberOfJoints(), n)
+            if self._input.hasWeldedBodies():
+                raise NotImplementedError("forward-dynamics derivatives with external wrenches on a system with fixed or ignored joints")
+        self._qdd = self._empty_like(q, nv, n)
+        self._dq = self._empty_like(q, nv * nv, n)
+        self._dqd = self._empty_like(q, nv * nv, n)
+        self._minv = self._empty_like(q, nv * nv, n)
+        self._engine.aba_derivatives(q, qd, tau, self._qdd, self._dq, self._dqd, self._minv, fext=self._fext)
+        return self._dq
+
+    def getJointAccelerationMatrix(self):
+        return self._qdd
+
+    def getAccelerationConfigurationGradientMatrix(self):
+        return self._dq
+
+    def getAccelerationVelocityGradientMatrix(self):
+        return self._dqd
+
+    def getInverseMassMatrix(self):
+        return self._minv
 
 
 class MultiBodyDynamicsStep:

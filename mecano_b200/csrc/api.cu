@@ -17,6 +17,7 @@
 #include "flatten.h"
 #include "jit.h"
 #include "kernels.h"
+#include "ltdl_solve.cuh"
 #include "specialize.h"
 
 #define MB_STAGGER_NS_DEFAULT 0
@@ -691,6 +692,56 @@ int enqueue_integrate(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, d
    MB_CUDA(h, mb::launch_integrate_kernel(J, a, h->sm_count, st));
    return MECANO_B200_OK;
 }
+
+// The refusals of the forward-dynamics derivatives, shared by their two entry points: those of ABA and of the inverse-dynamics
+// derivatives, whose kernels they reuse.
+int aba_derivatives_check(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
+                          const double *qdd, const double *dq, const double *dqd, const double *minv)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc) return rc;
+   if (h->fp32)
+      return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the forward-dynamics derivatives are computed in fp64 only (mecano_b200_set_precision)");
+   if (h->n_accel_source > 0)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the forward-dynamics derivatives need every joint in EFFORT_SOURCE mode (mecano_b200_set_joint_source_modes)");
+   if (h->plan[MB_RNEA_DERIVATIVES].block == 0)
+      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the inverse-dynamics derivatives kernel (branch nesting / depth too large)");
+   if (n > 0 && (!q || !qd || !tau || !qdd || !dq || !dqd || !minv))
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (fext)
+   {
+      const MbProgram &P = h->tree.prog[MB_RNEA_DERIVATIVES];
+      for (int i = 0; i < P.nb; i++)
+         if (P.body[i].ext_index >= P.nb)
+            return fail(h, MECANO_B200_ERR_SHAPE, "forward-dynamics derivatives: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
+   }
+   return MECANO_B200_OK;
+}
+
+// The four launches of mecano_b200_aba_derivatives on checked arguments, in stream order: ABA (qdd), the inverse-dynamics derivatives
+// at that qdd (into dq and dqd, their joint efforts into the first rows of minv, which nobody reads), CRBA (M into minv) and the
+// L^T D L solve (ltdl_solve.cuh), which turns minv into M^-1 and dq, dqd into -M^-1 dq, -M^-1 dqd in place.  opt: ws_slot and
+// variant_n only, so that qdd is what mecano_b200_aba computes.
+int enqueue_aba_derivatives(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
+                            double *qdd, double *dq, double *dqd, double *minv, cudaStream_t st, const RunOpts &opt)
+{
+   int rc = run(h, MB_ABA, n, ld, q, qd, tau, fext, qdd, 0u, st, opt);
+   if (rc) return rc;
+   RunOpts rd = opt;
+   rd.cor = dqd;
+   rd.root_wrench = minv;
+   if ((rc = run(h, MB_RNEA_DERIVATIVES, n, ld, q, qd, qdd, fext, dq, 0u, st, rd))) return rc;
+   if ((rc = run(h, MB_CRBA, n, ld, q, nullptr, nullptr, nullptr, minv, MECANO_B200_CRBA_ENTRY_MAJOR, st, opt))) return rc;
+   mb::LtdlTree t;
+   t.nv = h->tree.nv;
+   std::copy(h->tree.ltdl_dof.begin(), h->tree.ltdl_dof.end(), t.dof);
+   std::copy(h->tree.ltdl_parent.begin(), h->tree.ltdl_parent.end(), t.lam);
+   mb::LtdlArgs a;
+   a.minv = minv; a.dq = dq; a.dqd = dqd;
+   a.n = n; a.ld = ld;
+   MB_CUDA(h, mb::launch_ltdl_solve(t, a, st));
+   return MECANO_B200_OK;
+}
 } // namespace
 
 extern "C" {
@@ -1229,6 +1280,29 @@ int mecano_b200_rnea_derivatives_host(mecano_b200_handle *h, int64_t n, int64_t 
       opt.cor = c.out[2];
       return run(c.h, MB_RNEA_DERIVATIVES, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[1], 0u, c.stream, opt);
    }, {{tau, nv}, {dq, nv * nv}, {dqd, nv * nv}}});
+   return run_host(h, j);
+}
+
+int mecano_b200_aba_derivatives(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
+                                double *qdd, double *dq, double *dqd, double *minv, void *stream)
+{
+   const int rc = aba_derivatives_check(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv);
+   if (rc || n == 0) return rc;
+   MB_ON_DEVICE(h);
+   return enqueue_aba_derivatives(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv, (cudaStream_t)stream, RunOpts());
+}
+
+int mecano_b200_aba_derivatives_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau,
+                                     const double *fext, double *qdd, double *dq, double *dqd, double *minv)
+{
+   const int rc = aba_derivatives_check(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv);
+   if (rc || n == 0) return rc;
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   HostJob j{n, ld, {{q, nq}, {qd, nv}, {tau, nv}, {fext, 6 * (size_t)h->tree.nb}}};
+   // one step: the three matrices pass from launch to launch in the slot's device rows and are copied back once, after the solve
+   j.steps.push_back({[](const Chunk &c) {
+      return enqueue_aba_derivatives(c.h, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[0], c.out[1], c.out[2], c.out[3], c.stream, c.opt);
+   }, {{qdd, nv}, {dq, nv * nv}, {dqd, nv * nv}, {minv, nv * nv}}});
    return run_host(h, j);
 }
 

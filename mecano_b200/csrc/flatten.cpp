@@ -658,6 +658,16 @@ int flatten_tree(const mecano_b200_tree_desc *d, FlatTree &out, std::string &err
                return MECANO_B200_ERR_INVALID_ARGUMENT;
             }
          }
+      // DoF order of the L^T D L factor: bodies in pre-order, a joint's DoFs as a chain, so every DoF parent comes first
+      std::vector<int> last_dof(nb, -1);
+      for (int i = 0; i < nb; i++)
+         for (int r = 0; r < P.body[i].ndof; r++)
+         {
+            const int k = (int)out.ltdl_dof.size();
+            out.ltdl_parent.push_back((int16_t)(r > 0 ? k - 1 : (P.body[i].parent >= 0 ? last_dof[P.body[i].parent] : -1)));
+            out.ltdl_dof.push_back((int16_t)(P.body[i].dof_off + r));
+            last_dof[i] = k;
+         }
    }
    // ---- structural zeros of the joint-torque regressor: in the block of body i, the DoF rows of the joints that are not on the
    //      path from the root to i (flatten.h); only for wrench_index ranks that fit the 10 nb columns (api.cu refuses the others)

@@ -24,6 +24,9 @@ struct FlatTree
    // packed mass-matrix layout (MECANO_B200_CRBA_PACKED): packed row p holds M[packed_row[p]][packed_col[p]] (= the mirrored
    // entry); one row per unique entry that is not structurally zero, column by column, path from the root first
    std::vector<int32_t> packed_row, packed_col;
+   // the DoF tree of the forward-dynamics derivatives' L^T D L factor (ltdl_solve.cuh): DoF k in internal pre-order (a multi-DoF
+   // joint as a chain of its DoFs) is row ltdl_dof[k] of the matrices; its DoF parent ltdl_parent[k] < k, -1 at a root joint
+   std::vector<int16_t> ltdl_dof, ltdl_parent;
    // joint-torque regressor (MB_REGRESSOR): the structurally zero rows of each body's block, as the entry of the row's first
    // column (row * 10 nb + 10 w); a row's ten columns are zero together.  Empty if a wrench_index rank is >= nb.
    std::vector<uint32_t> regressor_zero_rows;

@@ -6,6 +6,7 @@
 //   JointTorqueRegressorCalculator            the inertial-parameter regressor of inverse dynamics (project definition, below)
 //   MultiBodyGravityGradientCalculator        gravity torques and their configuration gradient (project definition, below)
 //   InverseDynamicsDerivativesCalculator      d tau / dq and d tau / dqd of inverse dynamics (project definition, below)
+//   ForwardDynamicsDerivativesCalculator      d qdd / dq, d qdd / dqd and M^-1 of forward dynamics (project definition, below)
 //
 // Same names, argument meaning and error behaviour (exceptions) as the reference, with two batching changes:
 //   * compute(...) takes the joint state explicitly as nRows x N row-major matrices (what a Java
@@ -402,6 +403,40 @@ class InverseDynamicsDerivativesCalculator : public BatchedCalculatorBase
          check(mecano_b200_rnea_derivatives(handle_, n, q.ld, q.data, qd.data, qdd.data, fext_.data, tauOut.data, dqOut.data, dqdOut.data, stream_));
       else
          check(mecano_b200_rnea_derivatives_host(handle_, n, q.ld, q.data, qd.data, qdd.data, fext_.data, tauOut.data, dqOut.data, dqdOut.data));
+   }
+};
+
+// ForwardDynamicsDerivativesCalculator: the joint accelerations qdd(q, qd, tau) and their partials d qdd / dq, d qdd / dqd and
+// d qdd / d tau = M^-1 (mecano_b200_aba_derivatives: layout, floating-base and external-wrench conventions).  Systems with fixed /
+// ignored joints run on their welded tables; with external wrenches the call refuses them (their wrench ranks count the welded
+// bodies).
+class ForwardDynamicsDerivativesCalculator : public BatchedCalculatorBase
+{
+ public:
+   explicit ForwardDynamicsDerivativesCalculator(const MultiBodySystem &input, int device = 0) : BatchedCalculatorBase(input, device) {}
+   // compute(q, qd, tau) + getJointAccelerationMatrix() (nDoFs x N) + getAccelerationConfigurationGradientMatrix() /
+   // getAccelerationVelocityGradientMatrix() / getInverseMassMatrix() ((nDoFs * nDoFs) x N each, entry (i, j) at row i * nDoFs + j)
+   void compute(const MatrixView &q, const MatrixView &qd, const MatrixView &tau, const MatrixView &qddOut, const MatrixView &dqOut,
+                const MatrixView &dqdOut, const MatrixView &minvOut, Memory where = Memory::Device)
+   {
+      const int64_t n = q.cols, nv = input_.getNumberOfDoFs(), nq = input_.getConfigurationMatrixSize();
+      checkShape(q, nq, n, "q");
+      checkShape(qd, nv, n, "qd");
+      checkShape(tau, nv, n, "tau");
+      checkShape(qddOut, nv, n, "qdd");
+      checkShape(dqOut, nv * nv, n, "accelerationConfigurationGradient");
+      checkShape(dqdOut, nv * nv, n, "accelerationVelocityGradient");
+      checkShape(minvOut, nv * nv, n, "inverseMassMatrix");
+      if (fext_.data) checkShape(fext_, 6 * (int64_t)tables_.parent.size(), n, "externalWrenches");
+      if (qd.ld != q.ld || tau.ld != q.ld || qddOut.ld != q.ld || dqOut.ld != q.ld || dqdOut.ld != q.ld || minvOut.ld != q.ld ||
+          (fext_.data && fext_.ld != q.ld))
+         throw MatrixDimensionException("all matrices of one call must share the same leading dimension");
+      if (where == Memory::Device)
+         check(mecano_b200_aba_derivatives(handle_, n, q.ld, q.data, qd.data, tau.data, fext_.data, qddOut.data, dqOut.data, dqdOut.data, minvOut.data,
+                                           stream_));
+      else
+         check(mecano_b200_aba_derivatives_host(handle_, n, q.ld, q.data, qd.data, tau.data, fext_.data, qddOut.data, dqOut.data, dqdOut.data,
+                                                minvOut.data));
    }
 };
 } // namespace mecano

@@ -59,6 +59,15 @@ struct IntegrateArgs
 };
 cudaError_t launch_integrate_kernel(const IntegrateJoints &J, const IntegrateArgs &a, int sm_count, cudaStream_t stream);
 
+// forward-dynamics derivatives, last step (ltdl_solve.cu): per state, M in minv -> M^-1, d tau / dx in dq, dqd -> -M^-1 d tau / dx
+struct LtdlTree;
+struct LtdlArgs
+{
+   double *minv, *dq, *dqd; // [nv * nv][ld] entry-major each
+   long long n, ld;
+};
+cudaError_t launch_ltdl_solve(const LtdlTree &t, const LtdlArgs &a, cudaStream_t stream);
+
 // centroidal by-products, last step (centroidal.cu)
 struct CentroidalArgs
 {

@@ -264,6 +264,27 @@ class Engine:
             check(lib.mecano_b200_rnea_derivatives(self._h, n, ld, pq, pv, pa, pf, pt, pdq, pdv, self._stream()), self._h)
         return dq
 
+    def aba_derivatives(self, q, qd, tau, qdd, dq, dqd, minv, fext=None):
+        """qdd [nv, n], dq, dqd and minv [nv * nv, n] entry-major (mecano_b200_aba_derivatives), fext [6 * nb, n] or None; torch CUDA
+        tensors or numpy arrays (host path)."""
+        n = q.shape[1]
+        host = isinstance(q, np.ndarray)
+        f = _host_ptr_ld if host else self._dp
+        pq, l0 = f(q, self.nq, n)
+        pv, l1 = f(qd, self.nv, n)
+        pt, l2 = f(tau, self.nv, n)
+        pf, l3 = f(fext, 6 * self.nb, n)
+        pa, l4 = f(qdd, self.nv, n)
+        pdq, l5 = f(dq, self.nv * self.nv, n)
+        pdv, l6 = f(dqd, self.nv * self.nv, n)
+        pmi, l7 = f(minv, self.nv * self.nv, n)
+        ld = _same_ld([l0, l1, l2, l3, l4, l5, l6, l7])
+        if host:
+            check(lib.mecano_b200_aba_derivatives_host(self._h, n, ld, pq, pv, pt, pf, pa, pdq, pdv, pmi), self._h)
+        else:
+            check(lib.mecano_b200_aba_derivatives(self._h, n, ld, pq, pv, pt, pf, pa, pdq, pdv, pmi, self._stream()), self._h)
+        return dq
+
     def crba_centroidal(self, q, M, cmm, com, frame=_capi.FRAME_WORLD):
         """M [nv*nv, n] entry-major, cmm [6*nv, n], com [4, n]; torch CUDA tensors or numpy arrays (host path)."""
         n = q.shape[1]
@@ -520,7 +541,7 @@ class MultiDeviceEngine:
         raise NotImplementedError("this entry point is served per device: build the calculator on one device")
 
     aba_sources_host = coriolis = crba_centroidal = centroidal_convective_term = center_of_mass = integrate_host = set_joint_source_modes = _single_device_only
-    joint_torque_regressor = gravity_gradient = rnea_derivatives = _single_device_only
+    joint_torque_regressor = gravity_gradient = rnea_derivatives = aba_derivatives = _single_device_only
 
 
 def measure_fp64_peak(device=0):
