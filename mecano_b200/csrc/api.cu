@@ -375,48 +375,55 @@ cudaError_t copy_rows(double *dst, size_t dpitch, const double *src, size_t spit
    return cudaMemcpy2DAsync(dst, dpitch * sizeof(double), src, spitch * sizeof(double), w * sizeof(double), rows, kind, s);
 }
 
-// ------------------------------------------------------------------------------------------------ host-pointer pipeline
-// One host-pointer call on one handle ("lane"), declared as host matrices (entry-major, leading dimension ld) and the steps that
-// run on every chunk of states.  The pipeline stages each chunk in one slot: the inputs are uploaded, then each step is launched
-// and its outputs are copied back.  Pointers are already offset to the lane's first state.
+// ------------------------------------------------------------------------------------------------ jobs
+// One call on one handle ("lane"), declared as matrices (entry-major, leading dimension ld) and the steps that run on them.  On
+// device pointers (run_device) the job runs as one chunk of all n states on the caller's matrices.  On host pointers the pipeline
+// stages each chunk in one slot: the inputs are uploaded, then each step is launched and its outputs are copied back; pointers are
+// already offset to the lane's first state.
+// Fixed capacities, so that a device call does not allocate: at most 5 inputs (aba_job, step_job), 3 steps (step_job) and 4
+// outputs per step (aba_derivatives_job).  A value-initialised tail entry is absent; an empty launch ends the steps.
+#define MB_JOB_INPUTS 5
+#define MB_JOB_STEPS 3
+#define MB_STEP_OUTPUTS 4
 enum CopyBack
 {
    COPY_ROWS,        // entry-major rows
    COPY_STATES,      // state-major: `rows` contiguous doubles per state
    COPY_NONZERO_RUNS // entry-major, the rows of h->nonzero_runs only (CRBA ZEROS_PRESENT: the host matrix already holds the zeros)
 };
-struct HostIn
+struct JobIn
 {
    const double *host; // NULL: absent (no device rows)
    size_t rows;
 };
-struct HostOut
+struct JobOut
 {
    double *host; // NULL: device-only scratch
    size_t rows;  // 0: absent
    CopyBack how = COPY_ROWS;
    int in = -1; // >= 0: written in place into the device rows of that input
 };
-// what a step's launch sees: the chunk's device rows (leading dimension ld = the chunk; NULL for an absent matrix) of every input
-// and of the step's outputs, the chunk width w and the slot's stream and options (ws_slot, variant_n)
+// what a step's launch sees: the device rows (NULL for an absent matrix) of every input and of the step's outputs, the width w,
+// their leading dimension ld (the chunk in the pipeline) and the stream and options (ws_slot, variant_n)
 struct Chunk
 {
    mecano_b200_handle *h;
-   std::vector<double *> in, out;
+   const double *in[MB_JOB_INPUTS];
+   double *out[MB_STEP_OUTPUTS];
    int64_t w = 0, ld = 0;
    cudaStream_t stream = nullptr;
    RunOpts opt;
 };
-struct HostStep
+struct JobStep
 {
-   std::function<int(const Chunk &)> launch;
-   std::vector<HostOut> out;
+   std::function<int(const Chunk &)> launch; // captures a flag word, a frame, dt or a bool at most: stored inline, no allocation
+   JobOut out[MB_STEP_OUTPUTS];
 };
-struct HostJob
+struct Job
 {
    int64_t n = 0, ld = 0;
-   std::vector<HostIn> in;
-   std::vector<HostStep> steps;
+   JobIn in[MB_JOB_INPUTS];
+   JobStep steps[MB_JOB_STEPS];
    int64_t variant_n = 0; // size of the whole call (all lanes)
    // staging per slot (r06ze: 229 ms per dense 2^20-state step against 239 ms with 128 MB, 231 ms with 512 MB)
    double budget_mb = 256.0;
@@ -426,16 +433,16 @@ struct HostJob
    int slot = 0;
 };
 
-// chunk size and staging buffers (arguments are checked by the entry points).  n_slots slots per handle, each with its own stream:
+// chunk size and staging buffers (arguments are checked by the job builders).  n_slots slots per handle, each with its own stream:
 // H2D of chunk k+1 overlaps the kernels and the D2H of chunk k.
-int host_begin(mecano_b200_handle *h, HostJob &j)
+int host_begin(mecano_b200_handle *h, Job &j)
 {
    if (j.n == 0) return MECANO_B200_OK;
    size_t rows = 0; // device rows per state of one slot
-   for (const HostIn &i : j.in)
+   for (const JobIn &i : j.in)
       rows += i.host ? i.rows : 0;
-   for (const HostStep &s : j.steps)
-      for (const HostOut &o : s.out)
+   for (const JobStep &s : j.steps)
+      for (const JobOut &o : s.out)
          rows += o.in < 0 ? o.rows : 0;
    // chunk: the job's budget of rows per slot (MECANO_B200_HOST_CHUNK_MB overrides every job's), multiple of 256, at least 256 states
    // (no more: a wide job -- the regressor, a dense mass matrix of nv > 90 -- would otherwise make every slot far larger than the budget)
@@ -451,7 +458,7 @@ int host_begin(mecano_b200_handle *h, HostJob &j)
 }
 
 // issues the next chunk of the job (H2D, then each step's kernels and D2H, on the slot's stream); asynchronous with pinned host memory
-int host_issue_chunk(mecano_b200_handle *h, HostJob &j)
+int host_issue_chunk(mecano_b200_handle *h, Job &j)
 {
    if (j.s0 >= j.n) return MECANO_B200_OK;
    MB_ON_DEVICE(h);
@@ -464,29 +471,32 @@ int host_issue_chunk(mecano_b200_handle *h, HostJob &j)
    j.slot = (slot + 1) % h->n_slots;
    // a slot is reused every n_slots chunks: stream order already serialises it
    double *p = h->stage[slot];
+   double *in[MB_JOB_INPUTS] = {}; // the inputs' rows, also written by in-place outputs
    Chunk c{h, {}, {}, (int64_t)w, (int64_t)chunk, st};
    c.opt.ws_slot = 1 + slot;
    c.opt.variant_n = j.variant_n > 0 ? j.variant_n : j.n;
-   for (const HostIn &i : j.in)
+   for (int k = 0; k < MB_JOB_INPUTS; k++)
    {
-      c.in.push_back(i.host ? p : nullptr);
+      const JobIn &i = j.in[k];
       if (!i.host) continue;
+      c.in[k] = in[k] = p;
       MB_CUDA(h, copy_rows(p, chunk, i.host + s0, ld, w, i.rows, cudaMemcpyHostToDevice, st));
       p += i.rows * chunk;
    }
-   for (const HostStep &s : j.steps)
+   for (const JobStep &s : j.steps)
    {
-      c.out.clear();
-      for (const HostOut &o : s.out)
+      if (!s.launch) break;
+      for (int k = 0; k < MB_STEP_OUTPUTS; k++)
       {
-         c.out.push_back(o.in >= 0 ? c.in[(size_t)o.in] : (o.rows ? p : nullptr));
+         const JobOut &o = s.out[k];
+         c.out[k] = o.in >= 0 ? in[o.in] : (o.rows ? p : nullptr);
          if (o.in < 0) p += o.rows * chunk;
       }
       const int rc = s.launch(c);
       if (rc) return rc;
-      for (size_t k = 0; k < s.out.size(); k++)
+      for (int k = 0; k < MB_STEP_OUTPUTS; k++)
       {
-         const HostOut &o = s.out[k];
+         const JobOut &o = s.out[k];
          const double *d = c.out[k];
          if (!o.host || !o.rows) continue;
          if (o.how == COPY_STATES)
@@ -513,7 +523,7 @@ int host_finish(mecano_b200_handle *h)
 
 // Runs one job per lane: the chunks of all lanes are issued round-robin from the calling thread (everything is asynchronous
 // with pinned host memory), then every lane is synchronised once.  lanes.size() == 1 is the single-device host call.
-int run_host_lanes(const std::vector<mecano_b200_handle *> &lanes, std::vector<HostJob> &jobs, int *failed_lane)
+int run_host_lanes(const std::vector<mecano_b200_handle *> &lanes, std::vector<Job> &jobs, int *failed_lane)
 {
    int rc = MECANO_B200_OK;
    size_t started = 0;
@@ -550,54 +560,116 @@ int run_host_lanes(const std::vector<mecano_b200_handle *> &lanes, std::vector<H
    return rc;
 }
 
-int run_host(mecano_b200_handle *h, const HostJob &job)
+int run_host(mecano_b200_handle *h, const Job &job)
 {
    std::vector<mecano_b200_handle *> lanes(1, h);
-   std::vector<HostJob> jobs(1, job);
+   std::vector<Job> jobs(1, job);
    int failed = 0;
    return run_host_lanes(lanes, jobs, &failed);
 }
 
-// The jobs of the RNEA / ABA / CRBA host calls, single- and multi-device: argument checks (an empty batch gives an empty job), then
-// the job.
+// Runs a job on the caller's device pointers: one chunk of all n states, no staging, with the options of a device entry point
+// (ABA workspace slot 0, VARIANT_AUTO on n).  Every input and output is the caller's matrix, except device-only scratch, which lives
+// in h->d_scratch.  Like every device entry point it takes no lock.
+int run_device(mecano_b200_handle *h, const Job &j, void *stream)
+{
+   if (j.n == 0) return MECANO_B200_OK;
+   MB_ON_DEVICE(h);
+   const size_t ld = (size_t)j.ld;
+   size_t rows = 0; // scratch rows
+   for (const JobStep &s : j.steps)
+      for (const JobOut &o : s.out)
+         rows += o.host ? 0 : o.rows;
+   if (h->scratch_doubles < rows * ld)
+   {
+      if (h->d_scratch)
+      {
+         MB_CUDA(h, cudaDeviceSynchronize());
+         MB_CUDA(h, cudaFree(h->d_scratch));
+         h->d_scratch = nullptr;
+         h->scratch_doubles = 0;
+      }
+      MB_CUDA(h, cudaMalloc(&h->d_scratch, rows * ld * sizeof(double)));
+      h->scratch_doubles = rows * ld;
+   }
+   Chunk c{h, {}, {}, j.n, j.ld, (cudaStream_t)stream};
+   for (int k = 0; k < MB_JOB_INPUTS; k++)
+      c.in[k] = j.in[k].host;
+   double *p = h->d_scratch;
+   for (const JobStep &s : j.steps)
+   {
+      if (!s.launch) break;
+      for (int k = 0; k < MB_STEP_OUTPUTS; k++)
+      {
+         const JobOut &o = s.out[k];
+         c.out[k] = !o.rows ? nullptr : o.host ? o.host : p;
+         if (!o.host) p += o.rows * ld;
+      }
+      const int rc = s.launch(c);
+      if (rc) return rc;
+   }
+   return MECANO_B200_OK;
+}
+
+// refusals shared by several calls
+bool wrench_ranks_below_nb(const MbProgram &P)
+{
+   for (int i = 0; i < P.nb; i++)
+      if (P.body[i].ext_index >= P.nb) return false;
+   return true;
+}
+
+// a by-product kernel that did not fit the tree at mecano_b200_create (plan block 0)
+int refuse_unfit(mecano_b200_handle *h, const char *kernel)
+{
+   return fail(h, MECANO_B200_ERR_TOO_LARGE, std::string("tree exceeds the per-state work areas of the ") + kernel + " kernel (branch nesting / depth too large)");
+}
+
+// subject: "<result> is" / "<results> are"
+int refuse_fp32(mecano_b200_handle *h, const char *subject)
+{
+   return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, std::string("the ") + subject + " computed in fp64 only (mecano_b200_set_precision)");
+}
+
+// The job of each call, shared by its device and host entry points (and by the multi-device calls): argument checks in the order
+// the entry points report them (an empty batch gives an empty job), then the job.
 int rnea_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext, double *tau,
-             double *body_acc, double *joint_wrench, uint32_t flags, HostJob &j)
+             double *body_acc, double *joint_wrench, uint32_t flags, Job &j)
 {
    int rc = check_batch(h, n, ld);
    if (rc || n == 0) return rc;
    if (!q || !qd || !qdd || !tau) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
    const size_t nq = h->tree.nq, nv = h->tree.nv, nw = 6 * (size_t)h->tree.nb;
-   j = HostJob{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}, {fext, nw}}};
-   j.steps.push_back({[flags](const Chunk &c) {
+   j = Job{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}, {fext, nw}}};
+   j.steps[0] = {[flags](const Chunk &c) {
       RunOpts opt = c.opt;
       opt.body_acc = c.out[1];
       opt.joint_wrench = c.out[2];
       return run(c.h, MB_RNEA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[0], flags, c.stream, opt);
-   }, {{tau, nv}, {body_acc, body_acc ? nw : 0}, {joint_wrench, joint_wrench ? nw : 0}}});
+   }, {{tau, nv}, {body_acc, body_acc ? nw : 0}, {joint_wrench, joint_wrench ? nw : 0}}};
    return MECANO_B200_OK;
 }
 
-// qdd_in / tau_out given: mecano_b200_aba_sources_host
+// sources: mecano_b200_aba_sources[_host] (qdd_in, tau_out; no flags)
 int aba_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *qdd_in,
-            const double *fext, double *qdd, double *tau_out, uint32_t flags, HostJob &j)
+            const double *fext, double *qdd, double *tau_out, uint32_t flags, bool sources, Job &j)
 {
    int rc = check_batch(h, n, ld);
    if (rc || n == 0) return rc;
    if (!q || !qd || !tau || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
    const size_t nq = h->tree.nq, nv = h->tree.nv;
-   const bool sources = qdd_in || tau_out;
-   j = HostJob{n, ld, {{q, nq}, {qd, nv}, {tau, nv}, {fext, 6 * (size_t)h->tree.nb}, {qdd_in, nv}}};
-   j.steps.push_back({[flags, sources](const Chunk &c) {
+   j = Job{n, ld, {{q, nq}, {qd, nv}, {tau, nv}, {fext, 6 * (size_t)h->tree.nb}, {qdd_in, nv}}};
+   j.steps[0] = {[flags, sources](const Chunk &c) {
       if (sources) return run_aba_sources(c.h, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[4], c.in[3], c.out[0], c.out[1], c.stream, c.opt);
       return run(c.h, MB_ABA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[0], flags, c.stream, c.opt);
-   }, {{qdd, nv}, {tau_out, tau_out ? nv : 0}}});
+   }, {{qdd, nv}, {tau_out, tau_out ? nv : 0}}};
    return MECANO_B200_OK;
 }
 
 // mecano_b200_step_host: inputs q, qd, qdd_in, tau_in, fext; steps RNEA -> tau_out, ABA -> qdd_out, CRBA -> M, each one present
 // when its buffers are (M alone: mecano_b200_crba_host)
 int step_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd_in, const double *tau_in,
-             const double *fext, double *tau_out, double *qdd_out, double *M, uint32_t layout, HostJob &j)
+             const double *fext, double *tau_out, double *qdd_out, double *M, uint32_t layout, Job &j)
 {
    int rc = check_batch(h, n, ld);
    if (rc || n == 0) return rc;
@@ -613,133 +685,236 @@ int step_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, cons
    if (layout & MECANO_B200_CRBA_STATE_MAJOR)
       layout &= ~MECANO_B200_CRBA_ZEROS_PRESENT;
    const size_t nq = h->tree.nq, nv = h->tree.nv;
-   j = HostJob{n, ld, {{q, nq}, {rnea || aba ? qd : nullptr, nv}, {qdd_in, nv}, {tau_in, nv}, {fext, 6 * (size_t)h->tree.nb}}};
+   j = Job{n, ld, {{q, nq}, {rnea || aba ? qd : nullptr, nv}, {qdd_in, nv}, {tau_in, nv}, {fext, 6 * (size_t)h->tree.nb}}};
+   int s = 0;
    if (rnea)
-      j.steps.push_back({[](const Chunk &c) { return run(c.h, MB_RNEA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[4], c.out[0], 0u, c.stream, c.opt); },
-                         {{tau_out, nv}}});
+      j.steps[s++] = {[](const Chunk &c) { return run(c.h, MB_RNEA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[4], c.out[0], 0u, c.stream, c.opt); },
+                      {{tau_out, nv}}};
    if (aba)
-      j.steps.push_back({[](const Chunk &c) { return run(c.h, MB_ABA, c.w, c.ld, c.in[0], c.in[1], c.in[3], c.in[4], c.out[0], 0u, c.stream, c.opt); },
-                         {{qdd_out, nv}}});
+      j.steps[s++] = {[](const Chunk &c) { return run(c.h, MB_ABA, c.w, c.ld, c.in[0], c.in[1], c.in[3], c.in[4], c.out[0], 0u, c.stream, c.opt); },
+                      {{qdd_out, nv}}};
    if (M)
    {
       const CopyBack how = (layout & MECANO_B200_CRBA_STATE_MAJOR) ? COPY_STATES : (layout & MECANO_B200_CRBA_ZEROS_PRESENT) ? COPY_NONZERO_RUNS : COPY_ROWS;
-      j.steps.push_back({[layout](const Chunk &c) { return run(c.h, MB_CRBA, c.w, c.ld, c.in[0], nullptr, nullptr, nullptr, c.out[0], layout, c.stream, c.opt); },
-                         {{M, (layout & MECANO_B200_CRBA_PACKED) ? h->tree.packed_row.size() : nv * nv, how}}});
+      j.steps[s++] = {[layout](const Chunk &c) { return run(c.h, MB_CRBA, c.w, c.ld, c.in[0], nullptr, nullptr, nullptr, c.out[0], layout, c.stream, c.opt); },
+                      {{M, (layout & MECANO_B200_CRBA_PACKED) ? h->tree.packed_row.size() : nv * nv, how}}};
    }
    return MECANO_B200_OK;
 }
 
-// The kernels of mecano_b200_crba_centroidal (M, cmm given) and of mecano_b200_center_of_mass (M = cmm = NULL) on checked arguments.
-// The latter is the by-product CRBA kernel launched without a matrix: it keeps the composite-inertia recursion and drops the unit
-// momenta, their ancestor walks and every matrix store (crba.cuh: com_only) -- the same arithmetic, hence the same bits, as the com
-// rows of the former.
-int enqueue_centroidal(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame,
-                       cudaStream_t st, RunOpts opt)
+// mecano_b200_crba_centroidal, and with com_only (M = cmm = NULL) mecano_b200_center_of_mass.  The latter is the by-product CRBA
+// kernel launched without a matrix: it keeps the composite-inertia recursion and drops the unit momenta, their ancestor walks and
+// every matrix store (crba.cuh: com_only) -- the same arithmetic, hence the same bits, as the com rows of the former.
+int centroidal_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame, bool com_only,
+                   Job &j)
 {
-   // the kernel sums (mass * CoM, mass) over the children of the root body into the com rows
-   MB_CUDA(h, cudaMemset2DAsync(com, (size_t)ld * sizeof(double), 0, (size_t)n * sizeof(double), 4, st));
-   opt.cmm = cmm;
-   opt.com = com;
-   const int rc = run(h, MB_CRBA, n, ld, q, nullptr, nullptr, nullptr, M, MECANO_B200_CRBA_ENTRY_MAJOR, st, opt);
-   if (rc) return rc;
-   mb::CentroidalArgs ca;
-   ca.cols = cmm; ca.com = com; ca.n = n; ca.ld = ld; ca.ncols = cmm ? h->tree.nv : 0;
-   ca.normalize_com = 1;
-   ca.shift = frame == MECANO_B200_FRAME_CENTER_OF_MASS;
-   MB_CUDA(h, mb::launch_centroidal_finish(ca, st));
-   return MECANO_B200_OK;
-}
-
-// The kernels of mecano_b200_centroidal_convective_term on checked arguments; tau: nv rows for the joint efforts nobody reads.
-int enqueue_convective_term(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *com, double *out,
-                            double *tau, int frame, cudaStream_t st, RunOpts opt)
-{
-   // :811-839: the net wrench of every body under zero joint accelerations and no gravity, summed in the centroidal frame = the
-   // wrench at the root of inverse dynamics run that way
-   MB_CUDA(h, cudaMemset2DAsync(out, (size_t)ld * sizeof(double), 0, (size_t)n * sizeof(double), 6, st));
-   opt.root_wrench = out;
-   opt.zero_gravity = true;
-   const int rc = run(h, MB_RNEA, n, ld, q, qd, qd, nullptr, tau, MECANO_B200_RNEA_NO_ACCELERATIONS, st, opt);
-   if (rc) return rc;
-   if (frame == MECANO_B200_FRAME_CENTER_OF_MASS)
-   {
+   int rc = check_batch(h, n, ld);
+   if (rc || n == 0) return rc;
+   if (!q || (!com_only && (!M || !cmm)) || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
+   const size_t nv = h->tree.nv;
+   j = Job{n, ld, {{q, (size_t)h->tree.nq}}};
+   j.steps[0] = {[frame](const Chunk &c) {
+      double *const cmm = c.out[1], *const com = c.out[2];
+      // the kernel sums (mass * CoM, mass) over the children of the root body into the com rows
+      MB_CUDA(c.h, cudaMemset2DAsync(com, (size_t)c.ld * sizeof(double), 0, (size_t)c.w * sizeof(double), 4, c.stream));
+      RunOpts opt = c.opt;
+      opt.cmm = cmm;
+      opt.com = com;
+      const int rc = run(c.h, MB_CRBA, c.w, c.ld, c.in[0], nullptr, nullptr, nullptr, c.out[0], MECANO_B200_CRBA_ENTRY_MAJOR, c.stream, opt);
+      if (rc) return rc;
       mb::CentroidalArgs ca;
-      ca.cols = out; ca.com = const_cast<double *>(com); ca.n = n; ca.ld = ld; ca.ncols = 1;
-      ca.normalize_com = 0;
-      ca.shift = 1;
-      MB_CUDA(h, mb::launch_centroidal_finish(ca, st));
-   }
+      ca.cols = cmm; ca.com = com; ca.n = c.w; ca.ld = c.ld; ca.ncols = cmm ? c.h->tree.nv : 0;
+      ca.normalize_com = 1;
+      ca.shift = frame == MECANO_B200_FRAME_CENTER_OF_MASS;
+      MB_CUDA(c.h, mb::launch_centroidal_finish(ca, c.stream));
+      return MECANO_B200_OK;
+   }, {{M, com_only ? 0 : nv * nv}, {cmm, com_only ? 0 : 6 * nv}, {com, 4}}};
    return MECANO_B200_OK;
 }
 
-// The kernel of mecano_b200_integrate on checked arguments.
-int enqueue_integrate(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, double *q, double *qd, double *qdd, cudaStream_t st)
+// mecano_b200_centroidal_convective_term; the joint efforts nobody reads are device-only scratch
+int convective_term_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *com, double *out, int frame,
+                        Job &j)
 {
-   mb::IntegrateJoints J;
-   const MbProgram &P = h->tree.prog[MB_RNEA];
-   J.nb = P.nb;
-   for (int i = 0; i < P.nb; i++)
-   {
-      J.cfg[i] = (uint16_t)P.body[i].cfg_off;
-      J.dof[i] = (uint16_t)P.body[i].dof_off;
-      J.type[i] = (uint8_t)P.body[i].jtype;
-      J.sub[i] = (uint8_t)P.body[i].sub;
-   }
-   mb::IntegrateArgs a;
-   a.q = q; a.qd = qd; a.qdd = qdd;
-   a.n = n; a.ld = ld;
-   a.dt = dt;
-   MB_CUDA(h, mb::launch_integrate_kernel(J, a, h->sm_count, st));
+   int rc = check_batch(h, n, ld);
+   if (rc || n == 0) return rc;
+   if (!q || !qd || !out) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
+   if (frame == MECANO_B200_FRAME_CENTER_OF_MASS && !com)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the centre-of-mass frame needs the com rows of mecano_b200_crba_centroidal");
+   const size_t nv = h->tree.nv;
+   j = Job{n, ld, {{q, (size_t)h->tree.nq}, {qd, nv}, {com, 4}}};
+   j.steps[0] = {[frame](const Chunk &c) {
+      // :811-839: the net wrench of every body under zero joint accelerations and no gravity, summed in the centroidal frame = the
+      // wrench at the root of inverse dynamics run that way
+      MB_CUDA(c.h, cudaMemset2DAsync(c.out[0], (size_t)c.ld * sizeof(double), 0, (size_t)c.w * sizeof(double), 6, c.stream));
+      RunOpts opt = c.opt;
+      opt.root_wrench = c.out[0];
+      opt.zero_gravity = true;
+      const int rc = run(c.h, MB_RNEA, c.w, c.ld, c.in[0], c.in[1], c.in[1], nullptr, c.out[1], MECANO_B200_RNEA_NO_ACCELERATIONS, c.stream, opt);
+      if (rc) return rc;
+      if (frame == MECANO_B200_FRAME_CENTER_OF_MASS)
+      {
+         mb::CentroidalArgs ca;
+         ca.cols = c.out[0]; ca.com = const_cast<double *>(c.in[2]); ca.n = c.w; ca.ld = c.ld; ca.ncols = 1; // (com is read only: normalize_com = 0)
+         ca.normalize_com = 0;
+         ca.shift = 1;
+         MB_CUDA(c.h, mb::launch_centroidal_finish(ca, c.stream));
+      }
+      return MECANO_B200_OK;
+   }, {{out, 6}, {nullptr, nv}}};
    return MECANO_B200_OK;
 }
 
-// The refusals of the forward-dynamics derivatives, shared by their two entry points: those of ABA and of the inverse-dynamics
-// derivatives, whose kernels they reuse.
-int aba_derivatives_check(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
-                          const double *qdd, const double *dq, const double *dqd, const double *minv)
+int coriolis_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, double *M, double *C, Job &j)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc || n == 0) return rc;
+   if (!q || !qd || !M || !C) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (h->plan[MB_CORIOLIS].block == 0) return refuse_unfit(h, "Coriolis-matrix");
+   const size_t nv = h->tree.nv;
+   j = Job{n, ld, {{q, (size_t)h->tree.nq}, {qd, nv}}};
+   j.steps[0] = {[](const Chunk &c) {
+      RunOpts opt = c.opt;
+      opt.cor = c.out[1];
+      return run(c.h, MB_CORIOLIS, c.w, c.ld, c.in[0], c.in[1], c.in[1], nullptr, c.out[0], 0u, c.stream, opt);
+   }, {{M, nv * nv}, {C, nv * nv}}};
+   return MECANO_B200_OK;
+}
+
+int regressor_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, double *Y, Job &j)
 {
    int rc = check_batch(h, n, ld);
    if (rc) return rc;
-   if (h->fp32)
-      return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the forward-dynamics derivatives are computed in fp64 only (mecano_b200_set_precision)");
-   if (h->n_accel_source > 0)
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the forward-dynamics derivatives need every joint in EFFORT_SOURCE mode (mecano_b200_set_joint_source_modes)");
-   if (h->plan[MB_RNEA_DERIVATIVES].block == 0)
-      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the inverse-dynamics derivatives kernel (branch nesting / depth too large)");
-   if (n > 0 && (!q || !qd || !tau || !qdd || !dq || !dqd || !minv))
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (fext)
-   {
-      const MbProgram &P = h->tree.prog[MB_RNEA_DERIVATIVES];
-      for (int i = 0; i < P.nb; i++)
-         if (P.body[i].ext_index >= P.nb)
-            return fail(h, MECANO_B200_ERR_SHAPE, "forward-dynamics derivatives: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
-   }
+   if (h->fp32) return refuse_fp32(h, "joint-torque regressor is");
+   if (!wrench_ranks_below_nb(h->tree.prog[MB_REGRESSOR]))
+      return fail(h, MECANO_B200_ERR_SHAPE, "joint-torque regressor: wrench_index ranks must be below n_bodies (one ten-column block per body)");
+   if (h->plan[MB_REGRESSOR].block == 0) return refuse_unfit(h, "joint-torque regressor");
+   if (n == 0) return MECANO_B200_OK;
+   if (!q || !qd || !qdd || !Y) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   const size_t nv = h->tree.nv;
+   j = Job{n, ld, {{q, (size_t)h->tree.nq}, {qd, nv}, {qdd, nv}}};
+   j.steps[0] = {[](const Chunk &c) { return run(c.h, MB_REGRESSOR, c.w, c.ld, c.in[0], c.in[1], c.in[2], nullptr, c.out[0], 0u, c.stream, c.opt); },
+                 {{Y, nv * 10 * (size_t)h->tree.nb}}};
    return MECANO_B200_OK;
 }
 
-// The four launches of mecano_b200_aba_derivatives on checked arguments, in stream order: ABA (qdd), the inverse-dynamics derivatives
-// at that qdd (into dq and dqd, their joint efforts into the first rows of minv, which nobody reads), CRBA (M into minv) and the
-// L^T D L solve (ltdl_solve.cuh), which turns minv into M^-1 and dq, dqd into -M^-1 dq, -M^-1 dqd in place.  opt: ws_slot and
-// variant_n only, so that qdd is what mecano_b200_aba computes.
-int enqueue_aba_derivatives(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
-                            double *qdd, double *dq, double *dqd, double *minv, cudaStream_t st, const RunOpts &opt)
+int gravity_gradient_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *fext, double *tau, double *G, Job &j)
 {
-   int rc = run(h, MB_ABA, n, ld, q, qd, tau, fext, qdd, 0u, st, opt);
+   int rc = check_batch(h, n, ld);
    if (rc) return rc;
-   RunOpts rd = opt;
-   rd.cor = dqd;
-   rd.root_wrench = minv;
-   if ((rc = run(h, MB_RNEA_DERIVATIVES, n, ld, q, qd, qdd, fext, dq, 0u, st, rd))) return rc;
-   if ((rc = run(h, MB_CRBA, n, ld, q, nullptr, nullptr, nullptr, minv, MECANO_B200_CRBA_ENTRY_MAJOR, st, opt))) return rc;
-   mb::LtdlTree t;
-   t.nv = h->tree.nv;
-   std::copy(h->tree.ltdl_dof.begin(), h->tree.ltdl_dof.end(), t.dof);
-   std::copy(h->tree.ltdl_parent.begin(), h->tree.ltdl_parent.end(), t.lam);
-   mb::LtdlArgs a;
-   a.minv = minv; a.dq = dq; a.dqd = dqd;
-   a.n = n; a.ld = ld;
-   MB_CUDA(h, mb::launch_ltdl_solve(t, a, st));
+   if (h->fp32) return refuse_fp32(h, "gravity gradient is");
+   if (h->plan[MB_GRAVITY_GRADIENT].block == 0) return refuse_unfit(h, "gravity-gradient");
+   if (n > 0 && (!q || !tau || !G)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (fext && !wrench_ranks_below_nb(h->tree.prog[MB_GRAVITY_GRADIENT]))
+      return fail(h, MECANO_B200_ERR_SHAPE, "gravity gradient: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
+   if (n == 0) return MECANO_B200_OK;
+   const size_t nv = h->tree.nv;
+   j = Job{n, ld, {{q, (size_t)h->tree.nq}, {fext, 6 * (size_t)h->tree.nb}}};
+   j.steps[0] = {[](const Chunk &c) {
+      RunOpts opt = c.opt;
+      opt.cor = c.out[0]; // (kernel_args.h: the joint efforts travel in `cor`, G in `out`)
+      return run(c.h, MB_GRAVITY_GRADIENT, c.w, c.ld, c.in[0], nullptr, nullptr, c.in[1], c.out[1], 0u, c.stream, opt);
+   }, {{tau, nv}, {G, nv * nv}}};
+   return MECANO_B200_OK;
+}
+
+int rnea_derivatives_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
+                         double *tau, double *dq, double *dqd, Job &j)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc) return rc;
+   if (h->fp32) return refuse_fp32(h, "inverse-dynamics derivatives are");
+   if (h->plan[MB_RNEA_DERIVATIVES].block == 0) return refuse_unfit(h, "inverse-dynamics derivatives");
+   if (n > 0 && (!q || !qd || !qdd || !tau || !dq || !dqd)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (fext && !wrench_ranks_below_nb(h->tree.prog[MB_RNEA_DERIVATIVES]))
+      return fail(h, MECANO_B200_ERR_SHAPE, "inverse-dynamics derivatives: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
+   if (n == 0) return MECANO_B200_OK;
+   const size_t nv = h->tree.nv;
+   j = Job{n, ld, {{q, (size_t)h->tree.nq}, {qd, nv}, {qdd, nv}, {fext, 6 * (size_t)h->tree.nb}}};
+   j.steps[0] = {[](const Chunk &c) {
+      RunOpts opt = c.opt;
+      opt.root_wrench = c.out[0]; // (kernel_args.h: d tau / dq travels in `out`, d tau / dqd in `cor`,
+      opt.cor = c.out[2];         //  the joint efforts in `root_wrench`)
+      return run(c.h, MB_RNEA_DERIVATIVES, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[1], 0u, c.stream, opt);
+   }, {{tau, nv}, {dq, nv * nv}, {dqd, nv * nv}}};
+   return MECANO_B200_OK;
+}
+
+// mecano_b200_aba_derivatives: the refusals of ABA and of the inverse-dynamics derivatives, whose kernels it reuses, then one step of
+// four launches in stream order: ABA (qdd), the inverse-dynamics derivatives at that qdd (into dq and dqd, their joint efforts into
+// the first rows of minv, which nobody reads), CRBA (M into minv) and the L^T D L solve (ltdl_solve.cuh), which turns minv into M^-1
+// and dq, dqd into -M^-1 dq, -M^-1 dqd in place.  One step, so that in the pipeline the three matrices pass from launch to launch in
+// the slot's rows and are copied back once, after the solve; the options are the call's (ws_slot, variant_n), so that qdd is what
+// mecano_b200_aba computes.
+int aba_derivatives_job(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
+                        double *qdd, double *dq, double *dqd, double *minv, Job &j)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc) return rc;
+   if (h->fp32) return refuse_fp32(h, "forward-dynamics derivatives are");
+   if (h->n_accel_source > 0)
+      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the forward-dynamics derivatives need every joint in EFFORT_SOURCE mode (mecano_b200_set_joint_source_modes)");
+   if (h->plan[MB_RNEA_DERIVATIVES].block == 0) return refuse_unfit(h, "inverse-dynamics derivatives");
+   if (n > 0 && (!q || !qd || !tau || !qdd || !dq || !dqd || !minv)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (fext && !wrench_ranks_below_nb(h->tree.prog[MB_RNEA_DERIVATIVES]))
+      return fail(h, MECANO_B200_ERR_SHAPE, "forward-dynamics derivatives: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
+   if (n == 0) return MECANO_B200_OK;
+   const size_t nv = h->tree.nv;
+   j = Job{n, ld, {{q, (size_t)h->tree.nq}, {qd, nv}, {tau, nv}, {fext, 6 * (size_t)h->tree.nb}}};
+   j.steps[0] = {[](const Chunk &c) {
+      double *const qdd = c.out[0], *const dq = c.out[1], *const dqd = c.out[2], *const minv = c.out[3];
+      int rc = run(c.h, MB_ABA, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], qdd, 0u, c.stream, c.opt);
+      if (rc) return rc;
+      RunOpts rd = c.opt;
+      rd.cor = dqd;
+      rd.root_wrench = minv;
+      if ((rc = run(c.h, MB_RNEA_DERIVATIVES, c.w, c.ld, c.in[0], c.in[1], qdd, c.in[3], dq, 0u, c.stream, rd))) return rc;
+      if ((rc = run(c.h, MB_CRBA, c.w, c.ld, c.in[0], nullptr, nullptr, nullptr, minv, MECANO_B200_CRBA_ENTRY_MAJOR, c.stream, c.opt))) return rc;
+      mb::LtdlTree t;
+      t.nv = c.h->tree.nv;
+      std::copy(c.h->tree.ltdl_dof.begin(), c.h->tree.ltdl_dof.end(), t.dof);
+      std::copy(c.h->tree.ltdl_parent.begin(), c.h->tree.ltdl_parent.end(), t.lam);
+      mb::LtdlArgs a;
+      a.minv = minv; a.dq = dq; a.dqd = dqd;
+      a.n = c.w; a.ld = c.ld;
+      MB_CUDA(c.h, mb::launch_ltdl_solve(t, a, c.stream));
+      return MECANO_B200_OK;
+   }, {{qdd, nv}, {dq, nv * nv}, {dqd, nv * nv}, {minv, nv * nv}}};
+   return MECANO_B200_OK;
+}
+
+// mecano_b200_integrate: q, qd and qdd are updated in place, so the step writes them through its outputs
+int integrate_job(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, double *q, double *qd, double *qdd, Job &j)
+{
+   int rc = check_batch(h, n, ld);
+   if (rc || n == 0) return rc;
+   if (!q || !qd || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
+   if (!(dt == dt)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "dt is NaN");
+   const size_t nq = h->tree.nq, nv = h->tree.nv;
+   j = Job{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}}};
+   j.budget_mb = 64.0; // 2^20 H37 states on a B200 (1000 W), pinned: 22 ms per call against 24 ms with 256 MB per slot; pageable 148 against 153 ms
+   j.steps[0] = {[dt](const Chunk &c) {
+      mb::IntegrateJoints J;
+      const MbProgram &P = c.h->tree.prog[MB_RNEA];
+      J.nb = P.nb;
+      for (int i = 0; i < P.nb; i++)
+      {
+         J.cfg[i] = (uint16_t)P.body[i].cfg_off;
+         J.dof[i] = (uint16_t)P.body[i].dof_off;
+         J.type[i] = (uint8_t)P.body[i].jtype;
+         J.sub[i] = (uint8_t)P.body[i].sub;
+      }
+      mb::IntegrateArgs a;
+      a.q = c.out[0]; a.qd = c.out[1]; a.qdd = c.out[2];
+      a.n = c.w; a.ld = c.ld;
+      a.dt = dt;
+      MB_CUDA(c.h, mb::launch_integrate_kernel(J, a, c.h->sm_count, c.stream));
+      return MECANO_B200_OK;
+   }, {{q, nq, COPY_ROWS, 0}, {qd, nv, COPY_ROWS, 1}, {qdd, nv, COPY_ROWS, 2}}};
    return MECANO_B200_OK;
 }
 } // namespace
@@ -785,14 +960,8 @@ int mecano_b200_create(const mecano_b200_tree_desc *desc, int device, mecano_b20
    if (const char *es = getenv("MECANO_B200_HOST_SLOTS"))
       h->n_slots = std::min(MB_MAX_SLOTS, std::max(1, atoi(es)));
    auto bail = [&](cudaError_t ce, const char *what) {
-      std::string m = std::string(what) + ": " + cudaGetErrorString(ce);
-      if (h->d_consts) cudaFree(h->d_consts);
-      if (h->d_counters) cudaFree(h->d_counters);
-      if (h->d_zero) cudaFree(h->d_zero);
-      if (h->d_yzero) cudaFree(h->d_yzero);
-      if (h->d_prog) cudaFree(h->d_prog);
-      delete h;
-      return fail(nullptr, (int)ce, m);
+      mecano_b200_destroy(h);
+      return fail(nullptr, (int)ce, std::string(what) + ": " + cudaGetErrorString(ce));
    };
    DeviceGuard device_guard_(device);
    if ((e = device_guard_.err) != cudaSuccess) return bail(e, "cudaSetDevice");
@@ -838,11 +1007,7 @@ int mecano_b200_create(const mecano_b200_tree_desc *desc, int device, mecano_b20
       }
       if (!fits)
       {
-         cudaFree(h->d_consts);
-         if (h->d_counters) cudaFree(h->d_counters);
-         if (h->d_zero) cudaFree(h->d_zero);
-         if (h->d_yzero) cudaFree(h->d_yzero);
-         delete h;
+         mecano_b200_destroy(h);
          return fail(nullptr, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the compiled per-state work areas (branch nesting / depth too large)");
       }
    }
@@ -1001,37 +1166,25 @@ int mecano_b200_n_bodies(const mecano_b200_handle *h) { return h ? h->tree.nb : 
 int mecano_b200_rnea(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
                      double *tau, uint32_t flags, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK; /* empty batch: nothing to do, pointers may be NULL */
-   if (!q || !qd || !qdd || !tau) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   MB_ON_DEVICE(h);
-   return run(h, MB_RNEA, n, ld, q, qd, qdd, fext, tau, flags, (cudaStream_t)stream);
+   Job j;
+   const int rc = rnea_job(h, n, ld, q, qd, qdd, fext, tau, nullptr, nullptr, flags, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_rnea_full(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
                           double *tau, double *body_acc, double *joint_wrench, uint32_t flags, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !qdd || !tau) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   MB_ON_DEVICE(h);
-   RunOpts opt;
-   opt.body_acc = body_acc;
-   opt.joint_wrench = joint_wrench;
-   return run(h, MB_RNEA, n, ld, q, qd, qdd, fext, tau, flags, (cudaStream_t)stream, opt);
+   Job j;
+   const int rc = rnea_job(h, n, ld, q, qd, qdd, fext, tau, body_acc, joint_wrench, flags, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_aba(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
                     double *qdd, uint32_t flags, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !tau || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   MB_ON_DEVICE(h);
-   return run(h, MB_ABA, n, ld, q, qd, tau, fext, qdd, flags, (cudaStream_t)stream);
+   Job j;
+   const int rc = aba_job(h, n, ld, q, qd, tau, nullptr, fext, qdd, nullptr, flags, false, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_set_joint_source_modes(mecano_b200_handle *h, const int32_t *accel_source)
@@ -1045,313 +1198,145 @@ int mecano_b200_set_joint_source_modes(mecano_b200_handle *h, const int32_t *acc
 int mecano_b200_aba_sources(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *qdd_in,
                             const double *fext, double *qdd, double *tau_out, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !tau || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   MB_ON_DEVICE(h);
-   return run_aba_sources(h, n, ld, q, qd, tau, qdd_in, fext, qdd, tau_out, (cudaStream_t)stream, RunOpts());
+   Job j;
+   const int rc = aba_job(h, n, ld, q, qd, tau, qdd_in, fext, qdd, tau_out, 0u, true, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_aba_sources_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau,
                                  const double *qdd_in, const double *fext, double *qdd, double *tau_out)
 {
+   // ahead of the shape checks, also on an empty batch (the device entry point refuses a missing qdd_in when it launches)
    if (h && h->n_accel_source > 0 && !qdd_in)
       return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer (qdd_in) with joints in ACCELERATION_SOURCE mode");
-   HostJob j;
-   const int rc = aba_job(h, n, ld, q, qd, tau, qdd_in, fext, qdd, tau_out, 0u, j);
+   Job j;
+   const int rc = aba_job(h, n, ld, q, qd, tau, qdd_in, fext, qdd, tau_out, 0u, true, j);
    return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_crba_centroidal(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame,
                                 void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !M || !cmm || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
-   MB_ON_DEVICE(h);
-   return enqueue_centroidal(h, n, ld, q, M, cmm, com, frame, (cudaStream_t)stream, RunOpts());
+   Job j;
+   const int rc = centroidal_job(h, n, ld, q, M, cmm, com, frame, false, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 // The centre of mass alone (CenterOfMassCalculator.getCenterOfMass() / getTotalMass(), CenterOfMassCalculator.java:70-124; what
 // CenterOfMassReferenceFrame.updateTransformToParent(), CenterOfMassReferenceFrame.java:45-50, asks for).
 int mecano_b200_center_of_mass(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *com, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   MB_ON_DEVICE(h);
-   return enqueue_centroidal(h, n, ld, q, nullptr, nullptr, com, MECANO_B200_FRAME_WORLD, (cudaStream_t)stream, RunOpts());
+   Job j;
+   const int rc = centroidal_job(h, n, ld, q, nullptr, nullptr, com, MECANO_B200_FRAME_WORLD, true, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_centroidal_convective_term(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *com,
                                            double *out, int frame, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !out) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
-   if (frame == MECANO_B200_FRAME_CENTER_OF_MASS && !com)
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the centre-of-mass frame needs the com rows of mecano_b200_crba_centroidal");
-   MB_ON_DEVICE(h);
-   const size_t need = (size_t)h->tree.nv * (size_t)ld;
-   if (h->scratch_doubles < need)
-   {
-      if (h->d_scratch)
-      {
-         MB_CUDA(h, cudaDeviceSynchronize());
-         MB_CUDA(h, cudaFree(h->d_scratch));
-         h->d_scratch = nullptr;
-         h->scratch_doubles = 0;
-      }
-      MB_CUDA(h, cudaMalloc(&h->d_scratch, need * sizeof(double)));
-      h->scratch_doubles = need;
-   }
-   return enqueue_convective_term(h, n, ld, q, qd, com, out, h->d_scratch, frame, (cudaStream_t)stream, RunOpts());
+   Job j;
+   const int rc = convective_term_job(h, n, ld, q, qd, com, out, frame, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_coriolis(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, double *M, double *C, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !M || !C) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (h->plan[MB_CORIOLIS].block == 0)
-      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the Coriolis-matrix kernel (branch nesting / depth too large)");
-   MB_ON_DEVICE(h);
-   RunOpts opt;
-   opt.cor = C;
-   return run(h, MB_CORIOLIS, n, ld, q, qd, qd, nullptr, M, 0u, (cudaStream_t)stream, opt);
+   Job j;
+   const int rc = coriolis_job(h, n, ld, q, qd, M, C, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_coriolis_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, double *M, double *C)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !M || !C) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (h->plan[MB_CORIOLIS].block == 0)
-      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the Coriolis-matrix kernel (branch nesting / depth too large)");
-   const size_t nq = h->tree.nq, nv = h->tree.nv;
-   HostJob j{n, ld, {{q, nq}, {qd, nv}}};
-   j.steps.push_back({[](const Chunk &c) {
-      RunOpts opt = c.opt;
-      opt.cor = c.out[1];
-      return run(c.h, MB_CORIOLIS, c.w, c.ld, c.in[0], c.in[1], c.in[1], nullptr, c.out[0], 0u, c.stream, opt);
-   }, {{M, nv * nv}, {C, nv * nv}}});
-   return run_host(h, j);
-}
-
-// the regressor's refusals shared by its two entry points (after check_batch)
-int regressor_check(mecano_b200_handle *h)
-{
-   if (h->fp32)
-      return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the joint-torque regressor is computed in fp64 only (mecano_b200_set_precision)");
-   const MbProgram &P = h->tree.prog[MB_REGRESSOR];
-   for (int i = 0; i < P.nb; i++)
-      if (P.body[i].ext_index >= P.nb)
-         return fail(h, MECANO_B200_ERR_SHAPE, "joint-torque regressor: wrench_index ranks must be below n_bodies (one ten-column block per body)");
-   if (h->plan[MB_REGRESSOR].block == 0)
-      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the joint-torque regressor kernel (branch nesting / depth too large)");
-   return MECANO_B200_OK;
+   Job j;
+   const int rc = coriolis_job(h, n, ld, q, qd, M, C, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_joint_torque_regressor(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, double *Y,
                                        void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if ((rc = regressor_check(h))) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !qdd || !Y) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   MB_ON_DEVICE(h);
-   return run(h, MB_REGRESSOR, n, ld, q, qd, qdd, nullptr, Y, 0u, (cudaStream_t)stream);
+   Job j;
+   const int rc = regressor_job(h, n, ld, q, qd, qdd, Y, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_joint_torque_regressor_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, double *Y)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if ((rc = regressor_check(h))) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !qdd || !Y) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   const size_t nq = h->tree.nq, nv = h->tree.nv;
-   HostJob j{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}}};
-   j.steps.push_back({[](const Chunk &c) { return run(c.h, MB_REGRESSOR, c.w, c.ld, c.in[0], c.in[1], c.in[2], nullptr, c.out[0], 0u, c.stream, c.opt); },
-                      {{Y, nv * 10 * (size_t)h->tree.nb}}});
-   return run_host(h, j);
-}
-
-// the gravity gradient's refusals shared by its two entry points
-int gravity_gradient_check(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *fext, const double *tau, const double *G)
-{
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (h->fp32)
-      return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the gravity gradient is computed in fp64 only (mecano_b200_set_precision)");
-   if (h->plan[MB_GRAVITY_GRADIENT].block == 0)
-      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the gravity-gradient kernel (branch nesting / depth too large)");
-   if (n > 0 && (!q || !tau || !G))
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (fext)
-   {
-      const MbProgram &P = h->tree.prog[MB_GRAVITY_GRADIENT];
-      for (int i = 0; i < P.nb; i++)
-         if (P.body[i].ext_index >= P.nb)
-            return fail(h, MECANO_B200_ERR_SHAPE, "gravity gradient: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
-   }
-   return MECANO_B200_OK;
+   Job j;
+   const int rc = regressor_job(h, n, ld, q, qd, qdd, Y, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_gravity_gradient(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *fext, double *tau, double *G, void *stream)
 {
-   const int rc = gravity_gradient_check(h, n, ld, q, fext, tau, G);
-   if (rc || n == 0) return rc;
-   MB_ON_DEVICE(h);
-   RunOpts opt;
-   opt.cor = tau; // (kernel_args.h: the joint efforts travel in `cor`, G in `out`)
-   return run(h, MB_GRAVITY_GRADIENT, n, ld, q, nullptr, nullptr, fext, G, 0u, (cudaStream_t)stream, opt);
+   Job j;
+   const int rc = gravity_gradient_job(h, n, ld, q, fext, tau, G, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_gravity_gradient_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *fext, double *tau, double *G)
 {
-   const int rc = gravity_gradient_check(h, n, ld, q, fext, tau, G);
-   if (rc || n == 0) return rc;
-   const size_t nq = h->tree.nq, nv = h->tree.nv;
-   HostJob j{n, ld, {{q, nq}, {fext, 6 * (size_t)h->tree.nb}}};
-   j.steps.push_back({[](const Chunk &c) {
-      RunOpts opt = c.opt;
-      opt.cor = c.out[0];
-      return run(c.h, MB_GRAVITY_GRADIENT, c.w, c.ld, c.in[0], nullptr, nullptr, c.in[1], c.out[1], 0u, c.stream, opt);
-   }, {{tau, nv}, {G, nv * nv}}});
-   return run_host(h, j);
-}
-
-// the refusals of the inverse-dynamics derivatives, shared by their two entry points
-int rnea_derivatives_check(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
-                           const double *tau, const double *dq, const double *dqd)
-{
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (h->fp32)
-      return fail(h, MECANO_B200_ERR_UNSUPPORTED_TOPOLOGY, "the inverse-dynamics derivatives are computed in fp64 only (mecano_b200_set_precision)");
-   if (h->plan[MB_RNEA_DERIVATIVES].block == 0)
-      return fail(h, MECANO_B200_ERR_TOO_LARGE, "tree exceeds the per-state work areas of the inverse-dynamics derivatives kernel (branch nesting / depth too large)");
-   if (n > 0 && (!q || !qd || !qdd || !tau || !dq || !dqd))
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (fext)
-   {
-      const MbProgram &P = h->tree.prog[MB_RNEA_DERIVATIVES];
-      for (int i = 0; i < P.nb; i++)
-         if (P.body[i].ext_index >= P.nb)
-            return fail(h, MECANO_B200_ERR_SHAPE, "inverse-dynamics derivatives: with external wrenches the wrench_index ranks must be below n_bodies (fext has 6 n_bodies rows)");
-   }
-   return MECANO_B200_OK;
+   Job j;
+   const int rc = gravity_gradient_job(h, n, ld, q, fext, tau, G, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_rnea_derivatives(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
                                  double *tau, double *dq, double *dqd, void *stream)
 {
-   const int rc = rnea_derivatives_check(h, n, ld, q, qd, qdd, fext, tau, dq, dqd);
-   if (rc || n == 0) return rc;
-   MB_ON_DEVICE(h);
-   RunOpts opt;
-   opt.cor = dqd;          // (kernel_args.h: d tau / dq travels in `out`, d tau / dqd in `cor`,
-   opt.root_wrench = tau;  //  the joint efforts in `root_wrench`)
-   return run(h, MB_RNEA_DERIVATIVES, n, ld, q, qd, qdd, fext, dq, 0u, (cudaStream_t)stream, opt);
+   Job j;
+   const int rc = rnea_derivatives_job(h, n, ld, q, qd, qdd, fext, tau, dq, dqd, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_rnea_derivatives_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd,
                                       const double *fext, double *tau, double *dq, double *dqd)
 {
-   const int rc = rnea_derivatives_check(h, n, ld, q, qd, qdd, fext, tau, dq, dqd);
-   if (rc || n == 0) return rc;
-   const size_t nq = h->tree.nq, nv = h->tree.nv;
-   HostJob j{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}, {fext, 6 * (size_t)h->tree.nb}}};
-   j.steps.push_back({[](const Chunk &c) {
-      RunOpts opt = c.opt;
-      opt.root_wrench = c.out[0];
-      opt.cor = c.out[2];
-      return run(c.h, MB_RNEA_DERIVATIVES, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[1], 0u, c.stream, opt);
-   }, {{tau, nv}, {dq, nv * nv}, {dqd, nv * nv}}});
-   return run_host(h, j);
+   Job j;
+   const int rc = rnea_derivatives_job(h, n, ld, q, qd, qdd, fext, tau, dq, dqd, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_aba_derivatives(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
                                 double *qdd, double *dq, double *dqd, double *minv, void *stream)
 {
-   const int rc = aba_derivatives_check(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv);
-   if (rc || n == 0) return rc;
-   MB_ON_DEVICE(h);
-   return enqueue_aba_derivatives(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv, (cudaStream_t)stream, RunOpts());
+   Job j;
+   const int rc = aba_derivatives_job(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_aba_derivatives_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau,
                                      const double *fext, double *qdd, double *dq, double *dqd, double *minv)
 {
-   const int rc = aba_derivatives_check(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv);
-   if (rc || n == 0) return rc;
-   const size_t nq = h->tree.nq, nv = h->tree.nv;
-   HostJob j{n, ld, {{q, nq}, {qd, nv}, {tau, nv}, {fext, 6 * (size_t)h->tree.nb}}};
-   // one step: the three matrices pass from launch to launch in the slot's device rows and are copied back once, after the solve
-   j.steps.push_back({[](const Chunk &c) {
-      return enqueue_aba_derivatives(c.h, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.in[3], c.out[0], c.out[1], c.out[2], c.out[3], c.stream, c.opt);
-   }, {{qdd, nv}, {dq, nv * nv}, {dqd, nv * nv}, {minv, nv * nv}}});
-   return run_host(h, j);
+   Job j;
+   const int rc = aba_derivatives_job(h, n, ld, q, qd, tau, fext, qdd, dq, dqd, minv, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_crba_centroidal_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, double *cmm, double *com, int frame)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !M || !cmm || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
-   const size_t nv = h->tree.nv;
-   HostJob j{n, ld, {{q, (size_t)h->tree.nq}}};
-   j.steps.push_back({[frame](const Chunk &c) { return enqueue_centroidal(c.h, c.w, c.ld, c.in[0], c.out[0], c.out[1], c.out[2], frame, c.stream, c.opt); },
-                      {{M, nv * nv}, {cmm, 6 * nv}, {com, 4}}});
-   return run_host(h, j);
+   Job j;
+   const int rc = centroidal_job(h, n, ld, q, M, cmm, com, frame, false, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_centroidal_convective_term_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *com,
                                                 double *out, int frame)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !out) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (frame != MECANO_B200_FRAME_WORLD && frame != MECANO_B200_FRAME_CENTER_OF_MASS)
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "unknown centroidal momentum frame");
-   if (frame == MECANO_B200_FRAME_CENTER_OF_MASS && !com)
-      return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "the centre-of-mass frame needs the com rows of mecano_b200_crba_centroidal");
-   const size_t nv = h->tree.nv;
-   HostJob j{n, ld, {{q, (size_t)h->tree.nq}, {qd, nv}, {com, 4}}};
-   // the joint efforts nobody reads live in the slot
-   j.steps.push_back({[frame](const Chunk &c) { return enqueue_convective_term(c.h, c.w, c.ld, c.in[0], c.in[1], c.in[2], c.out[0], c.out[1], frame, c.stream, c.opt); },
-                      {{out, 6}, {nullptr, nv}}});
-   return run_host(h, j);
+   Job j;
+   const int rc = convective_term_job(h, n, ld, q, qd, com, out, frame, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_center_of_mass_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *com)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !com) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   HostJob j{n, ld, {{q, (size_t)h->tree.nq}}};
-   j.steps.push_back({[](const Chunk &c) { return enqueue_centroidal(c.h, c.w, c.ld, c.in[0], nullptr, nullptr, c.out[0], MECANO_B200_FRAME_WORLD, c.stream, c.opt); },
-                      {{com, 4}}});
-   return run_host(h, j);
+   Job j;
+   const int rc = centroidal_job(h, n, ld, q, nullptr, nullptr, com, MECANO_B200_FRAME_WORLD, true, j);
+   return rc ? rc : run_host(h, j);
 }
 
+// Not step_job: a caller's own buffer keeps ZEROS_PRESENT in every layout, and the kernel refuses what the layout does not combine with.
 int mecano_b200_crba(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, uint32_t layout, void *stream)
 {
    int rc = check_batch(h, n, ld);
@@ -1371,7 +1356,7 @@ int mecano_b200_rnea_host(mecano_b200_handle *h, int64_t n, int64_t ld, const do
 int mecano_b200_rnea_full_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd,
                                const double *fext, double *tau, double *body_acc, double *joint_wrench, uint32_t flags)
 {
-   HostJob j;
+   Job j;
    const int rc = rnea_job(h, n, ld, q, qd, qdd, fext, tau, body_acc, joint_wrench, flags, j);
    return rc ? rc : run_host(h, j);
 }
@@ -1379,35 +1364,23 @@ int mecano_b200_rnea_full_host(mecano_b200_handle *h, int64_t n, int64_t ld, con
 int mecano_b200_aba_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau,
                          const double *fext, double *qdd, uint32_t flags)
 {
-   HostJob j;
-   const int rc = aba_job(h, n, ld, q, qd, tau, nullptr, fext, qdd, nullptr, flags, j);
+   Job j;
+   const int rc = aba_job(h, n, ld, q, qd, tau, nullptr, fext, qdd, nullptr, flags, false, j);
    return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_integrate(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, double *q, double *qd, double *qdd, void *stream)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (!(dt == dt)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "dt is NaN");
-   MB_ON_DEVICE(h);
-   return enqueue_integrate(h, n, ld, dt, q, qd, qdd, (cudaStream_t)stream);
+   Job j;
+   const int rc = integrate_job(h, n, ld, dt, q, qd, qdd, j);
+   return rc ? rc : run_device(h, j, stream);
 }
 
 int mecano_b200_integrate_host(mecano_b200_handle *h, int64_t n, int64_t ld, double dt, double *q, double *qd, double *qdd)
 {
-   int rc = check_batch(h, n, ld);
-   if (rc) return rc;
-   if (n == 0) return MECANO_B200_OK;
-   if (!q || !qd || !qdd) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "NULL buffer");
-   if (!(dt == dt)) return fail(h, MECANO_B200_ERR_INVALID_ARGUMENT, "dt is NaN");
-   const size_t nq = h->tree.nq, nv = h->tree.nv;
-   HostJob j{n, ld, {{q, nq}, {qd, nv}, {qdd, nv}}};
-   j.budget_mb = 64.0; // 2^20 H37 states on a B200 (1000 W), pinned: 22 ms per call against 24 ms with 256 MB per slot; pageable 148 against 153 ms
-   j.steps.push_back({[dt](const Chunk &c) { return enqueue_integrate(c.h, c.w, c.ld, dt, c.in[0], c.in[1], c.in[2], c.stream); },
-                      {{q, nq, COPY_ROWS, 0}, {qd, nv, COPY_ROWS, 1}, {qdd, nv, COPY_ROWS, 2}}});
-   return run_host(h, j);
+   Job j;
+   const int rc = integrate_job(h, n, ld, dt, q, qd, qdd, j);
+   return rc ? rc : run_host(h, j);
 }
 
 int mecano_b200_crba_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, double *M, uint32_t layout)
@@ -1428,7 +1401,7 @@ int mecano_b200_crba_packed_index(const mecano_b200_handle *h, int32_t *row, int
 int mecano_b200_step_host(mecano_b200_handle *h, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd_in, const double *tau_in,
                           const double *fext, double *tau_out, double *qdd_out, double *M, uint32_t layout)
 {
-   HostJob j;
+   Job j;
    const int rc = step_job(h, n, ld, q, qd, qdd_in, tau_in, fext, tau_out, qdd_out, M, layout, j);
    return rc ? rc : run_host(h, j);
 }
@@ -1605,22 +1578,22 @@ int multi_run(mecano_b200_multi *m, int64_t n, int64_t ld, const Build &build)
       m->error = "n_states must be >= 0 and ld >= n_states";
       return MECANO_B200_ERR_SHAPE;
    }
-   HostJob whole;
+   Job whole;
    int rc = build(m->lanes[0], whole);
    if (rc) return multi_fail(m, rc, 0);
    const int L = (int)m->lanes.size();
-   std::vector<HostJob> jobs((size_t)L, whole);
+   std::vector<Job> jobs((size_t)L, whole);
    for (int i = 0; i < L; i++)
    {
       int64_t s0 = 0, cnt = 0;
       multi_slice(n, L, i, &s0, &cnt);
-      HostJob &j = jobs[(size_t)i];
+      Job &j = jobs[(size_t)i];
       j.n = cnt;
       j.variant_n = n;
-      for (HostIn &in : j.in)
+      for (JobIn &in : j.in)
          if (in.host) in.host += s0;
-      for (HostStep &st : j.steps)
-         for (HostOut &o : st.out)
+      for (JobStep &st : j.steps)
+         for (JobOut &o : st.out)
             if (o.host) o.host += o.how == COPY_STATES ? (size_t)s0 * o.rows : (size_t)s0;
    }
    int failed = 0;
@@ -1681,13 +1654,13 @@ int mecano_b200_multi_set_gravity(mecano_b200_multi *m, double gx, double gy, do
 int mecano_b200_multi_rnea_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd, const double *fext,
                                 double *tau, uint32_t flags)
 {
-   return multi_run(m, n, ld, [&](mecano_b200_handle *h, HostJob &j) { return rnea_job(h, n, ld, q, qd, qdd, fext, tau, nullptr, nullptr, flags, j); });
+   return multi_run(m, n, ld, [&](mecano_b200_handle *h, Job &j) { return rnea_job(h, n, ld, q, qd, qdd, fext, tau, nullptr, nullptr, flags, j); });
 }
 
 int mecano_b200_multi_aba_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, const double *qd, const double *tau, const double *fext,
                                double *qdd, uint32_t flags)
 {
-   return multi_run(m, n, ld, [&](mecano_b200_handle *h, HostJob &j) { return aba_job(h, n, ld, q, qd, tau, nullptr, fext, qdd, nullptr, flags, j); });
+   return multi_run(m, n, ld, [&](mecano_b200_handle *h, Job &j) { return aba_job(h, n, ld, q, qd, tau, nullptr, fext, qdd, nullptr, flags, false, j); });
 }
 
 int mecano_b200_multi_crba_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, double *M, uint32_t layout)
@@ -1698,7 +1671,7 @@ int mecano_b200_multi_crba_host(mecano_b200_multi *m, int64_t n, int64_t ld, con
 int mecano_b200_multi_step_host(mecano_b200_multi *m, int64_t n, int64_t ld, const double *q, const double *qd, const double *qdd_in, const double *tau_in,
                                 const double *fext, double *tau_out, double *qdd_out, double *M, uint32_t layout)
 {
-   return multi_run(m, n, ld, [&](mecano_b200_handle *h, HostJob &j) {
+   return multi_run(m, n, ld, [&](mecano_b200_handle *h, Job &j) {
       return step_job(h, n, ld, q, qd, qdd_in, tau_in, fext, tau_out, qdd_out, M, layout, j);
    });
 }
